@@ -17,6 +17,7 @@ Workload
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference ...                     # the reference's algorithm on host cores (oracle)
+  python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed, as .npy
 """
 import argparse
 import glob
@@ -32,6 +33,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the checkout may be read-only and is left as it is: no bytecode caches next to the sources
+sys.dont_write_bytecode = True
 
 # stdout carries exactly ONE JSON line: library chatter written to fd 1 (e.g. NCCL's version banner) is sent
 # to stderr for the whole run and the result goes to the saved descriptor
@@ -121,6 +124,25 @@ def solve_info(L, s):
     return {"kernel": name.value.decode(), "alg_flops": float(vals[0]), "exec_flops": float(vals[1]),
             "dense_flops": float(vals[2]), "bw": int(vals[3]), "ctas": int(vals[4]), "chain_steps": float(vals[5]),
             "band_clear": bool(vals[6]), "alg_bytes": float(vals[7])}
+
+
+DUMP_BYTES = 64_000_000   # --dump-outputs: all files together, .npy headers included
+
+
+def dump_outputs(out_dir, s, res):
+    """What ba_solve hands its caller after the last timed step, as float64 .npy files, so that two builds can be
+    compared output for output: poses.npy (N_total x 12, world-to-camera R row-major | t) and points.npy (M_total x 3),
+    both in the engine's internal units as ba_get_poses / ba_get_points return them, and cost.npy (initial, final cost
+    of the timed solve).  Points beyond the size budget are a seeded sample of rows, the same rows for the same
+    arguments."""
+    T, X = s.get_internal()
+    cost = np.array([res.initial_cost, res.final_cost], dtype=np.float64)
+    rows = (DUMP_BYTES - 3 * 4096 - T.nbytes - cost.nbytes) // (3 * 8)
+    if len(X) > rows:
+        X = X[np.sort(np.random.default_rng(0).choice(len(X), rows, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("poses", T), ("points", X), ("cost", cost)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def ncu_traffic_table():
@@ -385,12 +407,11 @@ def run_reference(args, rank, world):
         return
     workload = args.workload or ("c3" if world == 1 else "c4")
     sc, sample = cpu_sample(make_scene(workload, 0, args.scale), workload)
-    iters = max(1, min(args.steps, args.cpu_iters))
     warm = 1 if args.warmup > 0 else 0
     if warm:
         cpu_iterations(sc, 1, True)
-    dt, n = cpu_iterations(sc, iters, True)
-    dt_p, n_p = cpu_iterations(sc, iters, False)
+    dt, n = cpu_iterations(sc, args.steps, True)
+    dt_p, n_p = cpu_iterations(sc, args.steps, False)
     value = sc.n_obs * n / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": n,
@@ -430,14 +451,20 @@ def main():
     ap.add_argument("--e2e-max-iters", type=int, default=300,
                     help="iteration cap of the end-to-end solve (SURVEY 8d: thresholds 1e-6f, max 300 iterations)")
     ap.add_argument("--quick", action="store_true", help="profiling run: no clock-settling loop, phases, e2e or CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the poses, points and cost of the last timed step to DIR/<name>.npy (--impl b200; on "
+                         "several GPUs rank 0 writes, with its share of the landmarks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
-    args.steps = max(1, args.steps)
     args.warmup = max(3, args.warmup)
     workload = args.workload or ("c3" if world == 1 else "c4")
 
@@ -547,6 +574,8 @@ def main():
         ms, res = timed_steps(s, args.steps, args.warmup, settle=not args.quick)
         launches = int(res.kernel_launches)
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, s, res)
         nobs_all = torch.tensor([sz["n_obs"]], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(nobs_all)

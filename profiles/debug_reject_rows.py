@@ -1,5 +1,6 @@
-import sys, numpy as np
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
 import oracle
 from bundle_adjustment_solver_b200 import scenes
 from bundle_adjustment_solver_b200.solver import Summary

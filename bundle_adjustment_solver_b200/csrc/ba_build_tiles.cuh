@@ -5,7 +5,7 @@
 // work:
 //   * the tile chunks are cut into batches of 8 landmarks (K = 24 operand rows); the flat list of batches is split
 //     evenly over one persistent CTA per SM, so the producer/consumer pipeline never drains between chunks
-//     (a chunk that straddles two CTAs is simply flushed twice -- the flush is additive);
+//     (a chunk that straddles two CTAs is flushed into two staging segments);
 //   * a landmark is owned by 4 adjacent lanes of one warp; lane `sub` linearises incidences sub, sub+4, ... of the
 //     landmark, the 9 C/b partials are combined with an xor-butterfly (bitwise identical on the 4 lanes, so each
 //     lane inverts the damped C redundantly and forms E = B C^-1 for its own incidences): no CTA barrier, no
@@ -17,9 +17,9 @@
 //     the next batch's landmark data only after the observation loop (live across it, it would be spilled, and a
 //     spill waits for the load);
 //   * the four DMMA warps consume the buffers round-robin (2 x 2 super-tiles: every fragment read feeds two DMMAs,
-//     accumulators in registers across all batches of a chunk, FP64 reds when the chunk changes) and hand them back: full[g] / empty[g] named barriers,
-//     nothing else; a producer clears the few window slots its landmark does not cover instead of anybody
-//     clearing whole buffers.
+//     accumulators in registers across all batches of a chunk, flushed into a staging window when the chunk changes)
+//     and hand them back: full[g] / empty[g] named barriers, nothing else; a producer clears the few window slots its
+//     landmark does not cover instead of anybody clearing whole buffers.
 #pragma once
 
 constexpr int kT2LB = 8;                  // landmarks per batch (one producer warp, 4 lanes per landmark)
@@ -62,8 +62,7 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
                const int2 *__restrict__ inc_b /*slot (-1: fixed pose), camera slots of obs 0 | obs 1 << 8*/,
                const double2 *__restrict__ obs_uv, const int *__restrict__ obs_camflags, Params prm,
                const double *__restrict__ cams, double thres_huber, double *__restrict__ Bsoa, size_t Pp,
-               double *__restrict__ ptblk, size_t Mp, double *__restrict__ Saug, int ld,
-               const int *__restrict__ cta_seg_ptr /*first staging segment of every CTA; nullptr: flush with FP64 reds into S*/,
+               double *__restrict__ ptblk, size_t Mp, const int *__restrict__ cta_seg_ptr /*first staging segment of every CTA*/,
                const long long *__restrict__ seg_off, double *__restrict__ stage, const LmState *__restrict__ st) {
   if (st->done) return;
   extern __shared__ double tsm[];
@@ -313,41 +312,14 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
     int sdesc[kT2SPW];               // I | J << 8 | diagonal << 16 of the warp's super-tiles; mycnt of them are live
     int aofs[kT2SPW], bofs[kT2SPW];  // 16 I, 16 J
     double acc[kT2SPW][4][2];
-    int mycnt = 0, cur_chunk = -1, nrows = 0, row0 = 0, nt = 0;
-    // flush: upper triangle of the chunk's window (row-major) and its rhs column.  Deterministic mode: every
-    // (CTA, chunk) SEGMENT of the batch list owns a private staging window, written with plain stores (every entry,
-    // zeros included, so nothing has to be cleared); k_tile_reduce then adds the windows into S in segment order and S
-    // is bit-reproducible.  Otherwise: one FP64 red per live entry straight into S.
-    int seg = cta_seg_ptr ? __ldg(cta_seg_ptr + blockIdx.x) - 1 : 0;
+    int mycnt = 0, cur_chunk = -1, nrows = 0, nt = 0;
+    // flush: upper triangle of the chunk's window (row-major) and its rhs column.  Every (CTA, chunk) SEGMENT of the
+    // batch list owns a private staging window, written with plain stores (every entry, zeros included, so nothing has
+    // to be cleared); k_tile_reduce then adds the windows into S in segment order and S is bit-reproducible.
+    int seg = __ldg(cta_seg_ptr + blockIdx.x) - 1;
     double *stg = stage;
     auto flush = [&]() {
-      if (cta_seg_ptr) {
-        const int ldc = nrows + 1;
-#pragma unroll
-        for (int i = 0; i < kT2SPW; ++i) {
-          if (i >= mycnt) continue;
-          const int I = sdesc[i] & 0xff, J = (sdesc[i] >> 8) & 0xff;
-#pragma unroll
-          for (int p = 0; p < 2; ++p)
-#pragma unroll
-            for (int q = 0; q < 2; ++q) {
-              const int tj = 2 * J + q;
-              const int lr = 8 * (2 * I + p) + fr;
-              if (lr >= nrows || tj > nt) continue;
-              double *srow = stg + (size_t)lr * ldc;
-              if (tj == nt) {
-                if (fc == 0) __stcg(srow + nrows, acc[i][2 * p + q][0]);
-              } else {
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                  const int lc = 8 * tj + fc + e;
-                  if (lc < nrows && lc >= lr) __stcg(srow + lc, acc[i][2 * p + q][e]);
-                }
-              }
-            }
-        }
-        return;
-      }
+      const int ldc = nrows + 1;
 #pragma unroll
       for (int i = 0; i < kT2SPW; ++i) {
         if (i >= mycnt) continue;
@@ -359,15 +331,14 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
             const int tj = 2 * J + q;
             const int lr = 8 * (2 * I + p) + fr;
             if (lr >= nrows || tj > nt) continue;
-            const size_t grow = (size_t)(row0 + lr) * ld;
+            double *srow = stg + (size_t)lr * ldc;
             if (tj == nt) {
-              if (fc == 0 && acc[i][2 * p + q][0] != 0.0) atomicAdd(&Saug[grow + (ld - 1)], acc[i][2 * p + q][0]);
+              if (fc == 0) __stcg(srow + nrows, acc[i][2 * p + q][0]);
             } else {
 #pragma unroll
               for (int e = 0; e < 2; ++e) {
                 const int lc = 8 * tj + fc + e;
-                const double v = acc[i][2 * p + q][e];
-                if (lc < nrows && lc >= lr && v != 0.0) atomicAdd(&Saug[grow + row0 + lc], v);
+                if (lc < nrows && lc >= lr) __stcg(srow + lc, acc[i][2 * p + q][e]);
               }
             }
           }
@@ -381,10 +352,9 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
       if (rec.z != cur_chunk) {
         if (cur_chunk >= 0) flush();
         cur_chunk = rec.z;
-        if (cta_seg_ptr) stg = stage + __ldg(seg_off + (++seg));
+        stg = stage + __ldg(seg_off + (++seg));
         const SchurChunk ch = chunks[cur_chunk];
         nrows = 6 * ch.width;
-        row0 = 6 * ch.jmin;
         nt = (nrows + 7) >> 3;
         const int nI = (nt + 1) >> 1, nJ = (nt + 2) >> 1;          // super-rows, super-columns (rhs included)
         const int nst = nI * nJ - nI * (nI - 1) / 2;
@@ -435,7 +405,7 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
 // Second stage of the deterministic flush: S(r, c) += sum over the staging segments whose window holds (r, c), in
 // segment order.  One CTA per scalar row; segments are sorted by their first pose, so the candidates of a row are a
 // contiguous range (pose_seg).
-// STORE form (store_bw >= 0; speculative pose side on a banded plan, ba_engine.cu enqueue_build): the row is WRITTEN
+// STORE form (store_bw >= 0; banded plans, ba_engine.cu enqueue_build): the row is WRITTEN
 // instead of added to -- band entries r .. r + store_bw and the rhs entry get (damped pose-side sums of the accepted
 // parameter buffer, Au) + (sum of the windows), everything else of the band gets the plain sum (zero where no window
 // reaches) -- so neither the clearing of S nor k_pose_diag is launched; the row's CTA also stores the row of A and the

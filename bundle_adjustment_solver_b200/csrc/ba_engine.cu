@@ -3,10 +3,11 @@
 // Device pipeline of one LM iteration (reference: core/full_bundle_adjustment_solver.cpp:709-1008); six launches on
 // one GPU for a sequential trajectory (C3 / C4), replayed as a CUDA graph:
 //   K2 pose side            : the sums A (21) / a (6) per pose come from the trial-cost pass of the previous iteration
-//                             (K7; speculative, Au[parameter buffer]); damped and stored at the start of the iteration
-//                             by the storing form of k_tile_reduce (banded plans) or k_pose_diag.  BA_B200_SPEC_LIN=0 and
-//                             ba_build_only: k_linearize_by_pose, per-observation Jacobians in pose order, per-chunk
-//                             partials, ordered per-pose sum in the pose's last chunk (:795-810, :833-844, :878-888)
+//                             (K7; speculative, Au[parameter buffer]; per-observation Jacobians in pose order, per-chunk
+//                             partials, ordered per-pose sum in the pose's last chunk, :795-810, :833-844, :878-888);
+//                             damped and stored at the start of the iteration by the storing form of k_tile_reduce
+//                             (banded plans) or k_pose_diag.  ba_solve's initial cost and ba_build_only run the same
+//                             pass at the accepted parameters first
 //   K1b+K3+K4 k_build_tiles : landmarks whose poses fit a 16-pose window (ba_build_tiles.cuh): linearisation, C, b,
 //      + k_tile_reduce        B (last-writer rule), damping + pivoted 3x3 LDLT inverse, E = B C^-1 and the Schur
 //                             products S -= E B^T as an FP64 tensor-core GEMM, fused (:716-831, :846-856, :858-888);
@@ -23,7 +24,7 @@
 //                             gradient-descent variant for FullBundleAdjustmentSolverRefactor::SolveByGradientDescent
 //   K7 k_cost_linearize_by_pose : trial cost in pose order + the pose-side sums at the trial parameters; the last CTA
 //                             sums the partials in order and takes the rho / accept / lambda / convergence decision
-//                             on the device (:930-1007).  k_cost_decide (point order) with BA_B200_SPEC_LIN=0
+//                             on the device (:930-1007)
 // Multi-GPU: landmarks sharded; the band of [S | rhs] is exchanged through peer memory (one-shot pushes + epoch flags,
 // summed in rank order; NCCL all-reduce as the fallback), the five LM scalars by k_exchange_decide.
 // There is no CPU fallback: every entry point that computes requires a CUDA device.
@@ -276,9 +277,9 @@ k_finish_points(int M_total, const uint8_t *__restrict__ point_fb /*free landmar
 }
 
 // ---------------------------------------------------------------------------
-// K2: linearise in pose order -> per-chunk partial A (upper 21) and a (6); the LAST chunk of a pose to finish (ticket
-// per pose) sums the pose's partials in chunk order and stores A, a, the S diagonal block and the rhs (a pose without
-// observations keeps its zeros: A / a are cleared at finalisation, S every iteration).
+// K2: the pose side.  The pose-order pass of the trial cost (k_cost_linearize_by_pose, K7) leaves per-chunk partial
+// A (upper 21) and a (6); the LAST chunk of a pose to finish (ticket per pose) sums the pose's partials in chunk order
+// into Au (a pose without observations keeps its zeros).
 // ---------------------------------------------------------------------------
 // one warp per free pose.  pose_partial_sum: ordered sum of the pose's chunk partials (lane e < 21: packed upper element
 // e of A, lanes 21..26: a).  pose_diag_store: fill-lower, damping, A / a store, S diagonal block and rhs initialisation.
@@ -314,12 +315,6 @@ __device__ __forceinline__ void pose_diag_store(int j, int lane, double s, doubl
     Saug[(size_t)(6 * j + (lane - 21)) * ld + (ld - 1)] = s;  // rhs column
   }
 }
-__device__ __forceinline__ void finish_pose_warp(int j, int lane, const int *__restrict__ pose_chunk_ptr,
-                                                 const double *partials, double *__restrict__ A, double *__restrict__ a,
-                                                 double *__restrict__ Saug, int ld, const LmState *__restrict__ st) {
-  pose_diag_store(j, lane, pose_partial_sum(j, lane, pose_chunk_ptr, partials), A, a, Saug, ld, st);
-}
-
 // Speculative pose side (single launch with the trial cost, k_cost_linearize_by_pose below): the undamped sums of a
 // pose (27 values) live in Au[parameter buffer]; at the start of an iteration one warp per free pose damps the sums of
 // the ACCEPTED buffer with the current lambda and stores A, a, the S diagonal block and the rhs.
@@ -335,70 +330,6 @@ __global__ void k_pose_diag(int N, const double *__restrict__ Au0, const double 
   pose_diag_store(j, lane, s, A, a, Saug, ld, st);
 }
 
-
-__global__ void __launch_bounds__(kThreads, 2)
-k_linearize_by_pose(const ChunkA *__restrict__ chunks, const double2 *__restrict__ uvA,
-                    const int *__restrict__ pointA, const int *__restrict__ camA, const int *__restrict__ poseidA,
-                    Params prm, const double *__restrict__ cams, double thres_huber,
-                    double *__restrict__ partials /*[n_chunks][27]*/, const int *__restrict__ pose_chunk_ptr,
-                    unsigned *__restrict__ pose_ticket, double *__restrict__ A, double *__restrict__ a,
-                    double *__restrict__ Saug, int ld, const LmState *__restrict__ st) {
-  if (st->done) return;
-  __shared__ double sm[kWarps][27];
-  __shared__ int is_last;
-  const ChunkA ch = chunks[blockIdx.x];
-  const double *poses = prm.poses[st->cur];
-  const double *points = prm.points[st->cur];
-  double T[12];
-  {
-    const double *Tp = poses + (size_t)poseidA[ch.obs_start] * 12;
-#pragma unroll
-    for (int i = 0; i < 12; ++i) T[i] = __ldg(Tp + i);
-  }
-  double acc[27];
-#pragma unroll
-  for (int i = 0; i < 27; ++i) acc[i] = 0.0;
-  for (int t = threadIdx.x; t < ch.obs_count; t += kThreads) {
-    const int k = ch.obs_start + t;
-    const double2 uv = uvA[k];
-    const int pt = pointA[k];
-    const double *cam = cams + (camA[k] & kCamMask) * kCamStride;
-    double X[3] = {__ldg(points + (size_t)pt * 3), __ldg(points + (size_t)pt * 3 + 1),
-                   __ldg(points + (size_t)pt * 3 + 2)};
-    Proj p;
-    project(T, X, cam, uv.x, uv.y, p);
-    const double w = huber_weight(p.r0, p.r1, thres_huber);
-    const double wr0 = w * p.r0, wr1 = w * p.r1;
-    double G[6], Q[12];
-    jac_G(p, cam, G);
-    jac_Q(G, p.Xb, Q);
-    // A_j(upper) += (w Q)^T Q (:519-556,807) ; a_j -= Q^T (w r) (:809)
-    int e = 0;
-#pragma unroll
-    for (int r = 0; r < 6; ++r) {
-      const double wa0 = w * Q[r], wa1 = w * Q[6 + r];
-#pragma unroll
-      for (int c = r; c < 6; ++c) acc[e++] += wa0 * Q[c] + wa1 * Q[6 + c];
-    }
-#pragma unroll
-    for (int r = 0; r < 6; ++r) acc[21 + r] -= Q[r] * wr0 + Q[6 + r] * wr1;
-  }
-  block_sum<27, kWarps>(acc, sm);
-  if (threadIdx.x == 0) {
-    double *o = partials + (size_t)blockIdx.x * 27;
-#pragma unroll
-    for (int i = 0; i < 27; ++i) __stcg(o + i, acc[i]);
-    __threadfence();
-    const unsigned n_ck = (unsigned)(pose_chunk_ptr[ch.j_opt + 1] - pose_chunk_ptr[ch.j_opt]);
-    is_last = atomicAdd(pose_ticket + ch.j_opt, 1u) == n_ck - 1;
-    if (is_last) pose_ticket[ch.j_opt] = 0;
-  }
-  __syncthreads();
-  if (is_last && threadIdx.x < 32) {
-    __threadfence();
-    finish_pose_warp(ch.j_opt, threadIdx.x, pose_chunk_ptr, partials, A, a, Saug, ld, st);
-  }
-}
 
 // ---------------------------------------------------------------------------
 // K4: Schur complement  S -= sum_i E_ji B_ki^T (j<=k), rhs_j -= E_ji b_i, E_ji = B_ji Cinv_i  (:858-888).
@@ -687,52 +618,6 @@ k_backsub_points_update_poses(int point_blocks, int M_total, const int *__restri
     update_poses_body(blockIdx.x - point_blocks, N_total, pose_opt, x, A, a, prm, prw, pose_partials, st);
 }
 
-// EvaluateCurrentCost (:381-433): sum over observations of ||r||_2 ; which = 0 current, 1 trial.
-__device__ __forceinline__ double cost_block_sum(long long n_obs, const double2 *__restrict__ obs_uv,
-                                                 const int *__restrict__ obs_pose, const int *__restrict__ obs_point,
-                                                 const int *__restrict__ obs_camflags, const Params &prm, int which,
-                                                 const double *__restrict__ cams, const LmState *__restrict__ st) {
-  __shared__ double sm[kWarps][1];
-  const int buf = st->cur ^ which;
-  const double *poses = prm.poses[buf];
-  const double *points = prm.points[buf];
-  double acc[1] = {0.0};
-  // grid-stride loop, software-pipelined: the index record of the next observation is requested before the pose /
-  // point gathers of the current one, so the two dependent round trips of consecutive iterations overlap
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  double2 uv = make_double2(0.0, 0.0);
-  int ps = 0, pt = 0, cf = 0;
-  if (k < n_obs) { uv = obs_uv[k]; ps = obs_pose[k]; pt = obs_point[k]; cf = obs_camflags[k]; }
-  while (k < n_obs) {
-    const long long kn = k + stride;
-    double2 uv_n = uv;
-    int ps_n = ps, pt_n = pt, cf_n = cf;
-    if (kn < n_obs) { uv_n = obs_uv[kn]; ps_n = obs_pose[kn]; pt_n = obs_point[kn]; cf_n = obs_camflags[kn]; }
-    const double *cam = cams + (cf & kCamMask) * kCamStride;
-    double T[12], X[3];
-    load_pose(poses + (size_t)ps * 12, T);
-    X[0] = __ldg(points + (size_t)pt * 3);
-    X[1] = __ldg(points + (size_t)pt * 3 + 1);
-    X[2] = __ldg(points + (size_t)pt * 3 + 2);
-    Proj p;
-    project(T, X, cam, uv.x, uv.y, p);
-    acc[0] += sqrt(p.r0 * p.r0 + p.r1 * p.r1);
-    uv = uv_n; ps = ps_n; pt = pt_n; cf = cf_n;
-    k = kn;
-  }
-  block_sum<1, kWarps>(acc, sm);
-  return acc[0];     // the CTA's sum, valid in thread 0
-}
-__global__ void __launch_bounds__(kThreads)
-k_cost(long long n_obs, const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
-       const int *__restrict__ obs_point, const int *__restrict__ obs_camflags, Params prm, int which,
-       const double *__restrict__ cams, double *__restrict__ partials, int ignore_done,
-       const LmState *__restrict__ st) {
-  if (!ignore_done && st->done) return;
-  const double v = cost_block_sum(n_obs, obs_uv, obs_pose, obs_point, obs_camflags, prm, which, cams, st);
-  if (threadIdx.x == 0) partials[blockIdx.x] = v;
-}
 
 // ---------------------------------------------------------------------------
 // K4 for by-point landmarks when the reduced system is SMALL (dense co-visibility such as the test_ba.cpp scene:
@@ -962,82 +847,22 @@ __global__ void k_decide(DecideArgs g, LmState *st, ba_iter_info *infos, int cap
   decide(g, st, infos, cap);
 }
 
-// single GPU: the ordered sums of k_reduce_scalars and the decision in one launch (no exchange in between)
-__global__ void __launch_bounds__(kThreads) k_reduce_decide(DecideArgs g, LmState *st, ba_iter_info *infos, int cap) {
-  if (st->done) return;
-  __shared__ double sm[kWarps][5];
-  double acc[5] = {0, 0, 0, 0, 0};
-  for (int i = threadIdx.x; i < g.n_cost; i += kThreads) acc[0] += g.cost_partials[i];
-  for (int i = threadIdx.x; i < g.n_point; i += kThreads) {
-    acc[1] += g.point_partials[2 * i];
-    acc[2] += g.point_partials[2 * i + 1];
-  }
-  for (int i = threadIdx.x; i < g.n_pose; i += kThreads) {
-    acc[3] += g.pose_partials[2 * i];
-    acc[4] += g.pose_partials[2 * i + 1];
-  }
-  block_sum<5, kWarps>(acc, sm);
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int i = 0; i < 5; ++i) g.scal[i] = acc[i];
-    decide(g, st, infos, cap);
-  }
-}
-
-// single GPU: the trial cost AND the decision in one launch -- the last CTA to finish (ticket counter) sums all the
-// partials in their fixed order and takes the trust-region decision (saves k_reduce_decide's launch and its 6 us)
-__global__ void __launch_bounds__(kThreads)
-k_cost_decide(long long n_obs, const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
-              const int *__restrict__ obs_point, const int *__restrict__ obs_camflags, Params prm,
-              const double *__restrict__ cams, double *__restrict__ partials, unsigned *__restrict__ ticket, DecideArgs g,
-              LmState *st, ba_iter_info *infos, int cap) {
-  if (st->done) return;
-  const double v = cost_block_sum(n_obs, obs_uv, obs_pose, obs_point, obs_camflags, prm, 1, cams, st);
-  __shared__ int is_last;
-  if (threadIdx.x == 0) {
-    __stcg(partials + blockIdx.x, v);
-    __threadfence();
-    is_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-  }
-  __syncthreads();
-  if (!is_last) return;
-  __threadfence();
-  __shared__ double sm2[kWarps][5];
-  double acc[5] = {0, 0, 0, 0, 0};
-  for (int i = threadIdx.x; i < g.n_cost; i += kThreads) acc[0] += __ldcg(g.cost_partials + i);
-  for (int i = threadIdx.x; i < g.n_point; i += kThreads) {
-    acc[1] += __ldcg(g.point_partials + 2 * i);
-    acc[2] += __ldcg(g.point_partials + 2 * i + 1);
-  }
-  for (int i = threadIdx.x; i < g.n_pose; i += kThreads) {
-    acc[3] += __ldcg(g.pose_partials + 2 * i);
-    acc[4] += __ldcg(g.pose_partials + 2 * i + 1);
-  }
-  block_sum<5, kWarps>(acc, sm2);
-  if (threadIdx.x == 0) {
-    *ticket = 0;
-#pragma unroll
-    for (int i = 0; i < 5; ++i) g.scal[i] = acc[i];
-    decide(g, st, infos, cap);
-  }
-}
-
-// Speculative pose side: the trial cost AND the pose-side linearisation at the trial parameters in ONE pass over the
-// observations in pose order.  When the step is accepted the trial parameters are the next iteration's linearisation
-// point, so its A / a sums are already there (Au[trial buffer]); when it is rejected the sums of the kept buffer are
-// still valid (RevertToReservedParameters re-linearises at the same point, :939-953) -- either way the next iteration
-// starts with k_pose_diag instead of a second pass over the observations (k_linearize_by_pose + the point-order cost
-// pass cost 57 us on C3, this pass costs as much as the linearisation alone).  Chunks of FIXED poses (j_opt < 0, at the
-// end of the list) contribute to the cost only.  Per pose the last chunk to finish sums the pose's partials in chunk
-// order (bit-reproducible, same sums as k_linearize_by_pose); with decide_here the last CTA of the grid sums all the
-// partials in their fixed order and takes the trust-region decision (as k_cost_decide).
+// K7, the trial cost AND the pose-side linearisation at the trial parameters in ONE pass over the observations in pose
+// order (speculative pose side).  When the step is accepted the trial parameters are the next iteration's
+// linearisation point, so its A / a sums are already there (Au[trial buffer]); when it is rejected the sums of the kept
+// buffer are still valid (RevertToReservedParameters re-linearises at the same point, :939-953) -- either way the next
+// iteration starts with k_pose_diag (or the storing k_tile_reduce) instead of a second pass over the observations.
+// which = 0 (ignore_done) evaluates the accepted parameters instead: the initial cost and the sums the first iteration
+// starts from.  Chunks of FIXED poses (j_opt < 0, at the end of the list) contribute to the cost only.  Per pose the
+// last chunk to finish sums the pose's partials in chunk order (bit-reproducible); with decide_here the last CTA of the
+// grid sums all the partials in their fixed order and takes the trust-region decision.
 #ifndef BA_K7_MINB
 #define BA_K7_MINB 2   // resident CTAs per SM the register allocation aims at (A/B builds: 3 -> 85 registers, spills)
 #endif
 __global__ void __launch_bounds__(kThreads, BA_K7_MINB)
 k_cost_linearize_by_pose(const ChunkA *__restrict__ chunks, const double2 *__restrict__ uvA,
                          const int *__restrict__ pointA, const int *__restrict__ camA, const int *__restrict__ poseidA,
-                         Params prm, int which, const double *__restrict__ cams, double thres_huber,
+                         int n_chunks, Params prm, int which, const double *__restrict__ cams, double thres_huber,
                          double *__restrict__ partials /*[free chunks][27]*/, double *__restrict__ cost_partials /*[grid]*/,
                          const int *__restrict__ pose_chunk_ptr, unsigned *__restrict__ pose_ticket,
                          double *__restrict__ Au0, double *__restrict__ Au1, unsigned *__restrict__ ticket,
@@ -1045,13 +870,14 @@ k_cost_linearize_by_pose(const ChunkA *__restrict__ chunks, const double2 *__res
   if (!ignore_done && st->done) return;
   __shared__ double sm[kWarps][28];
   __shared__ int is_last_pose, is_last;
-  const ChunkA ch = chunks[blockIdx.x];
+  // a problem without observations has no chunks: its grid is one CTA that contributes zeros and takes the decision
+  const ChunkA ch = (int)blockIdx.x < n_chunks ? chunks[blockIdx.x] : ChunkA{0, 0, -1, 0};
   const int buf = st->cur ^ which;
   const double *poses = prm.poses[buf];
   const double *points = prm.points[buf];
   const bool free_pose = ch.j_opt >= 0;
-  double T[12];
-  {
+  double T[12] = {};
+  if (ch.obs_count > 0) {
     const double *Tp = poses + (size_t)poseidA[ch.obs_start] * 12;
 #pragma unroll
     for (int i = 0; i < 12; ++i) T[i] = __ldg(Tp + i);
@@ -1817,17 +1643,16 @@ struct ba_solver {
   // blocks
   size_t Mp = 0, Pp = 0;
   DevBuf<double> d_ptblk, d_Bsoa, d_A, d_a, d_partialsA, d_Saug, d_Scopy, d_x, d_z, d_linv, d_Btx, d_y;
-  DevBuf<double> d_cost_partials, d_point_partials, d_pose_partials, d_scal;
+  DevBuf<double> d_point_partials, d_pose_partials, d_scal;
   DevBuf<LmState> d_state;
-  DevBuf<unsigned> d_ticket;     // k_cost_decide: CTAs that have finished
-  DevBuf<unsigned> d_pose_ticket;   // k_linearize_by_pose: chunks of every pose that have finished
+  DevBuf<unsigned> d_ticket;        // k_cost_linearize_by_pose: CTAs that have finished
+  DevBuf<unsigned> d_pose_ticket;   // k_cost_linearize_by_pose: chunks of every pose that have finished
   DevBuf<double> d_Au[2];           // speculative pose side: undamped A (21) / a (6) sums per free pose and parameter buffer
   DevBuf<double> d_cost_partialsA;  // cost partials of k_cost_linearize_by_pose, one per pose-order chunk
   int n_chunksA_all = 0;            // free-pose chunks (the first n_chunksA) + fixed-pose chunks
-  bool spec_now = false, graph_spec = false;   // speculative pose side: this ba_solve / the captured graph
   bool rs_now = false, graph_rs = false;       // storing form of k_tile_reduce allowed (BA_B200_REDUCE_STORES)
   DevBuf<ba_iter_info> d_infos;
-  int cost_grid = 0, point_grid = 0, pose_grid = 0;
+  int point_grid = 0, pose_grid = 0;
   LmState *h_state = nullptr;  // pinned
   double *h_scal = nullptr;    // pinned
 
@@ -1902,7 +1727,7 @@ static void free_device(ba_solver *s) {
   s->d_nd_flags.release(); s->d_nd_helpers.release(); s->d_nd_L.release(); s->d_nd_U.release();
   s->d_ptblk.release(); s->d_Bsoa.release();
   s->d_A.release(); s->d_a.release(); s->d_partialsA.release(); s->d_Saug.release(); s->d_Scopy.release();
-  s->d_x.release(); s->d_z.release(); s->d_linv.release(); s->d_Btx.release(); s->d_y.release(); s->d_cost_partials.release();
+  s->d_x.release(); s->d_z.release(); s->d_linv.release(); s->d_Btx.release(); s->d_y.release();
   s->d_point_partials.release(); s->d_pose_partials.release(); s->d_scal.release(); s->d_state.release(); s->d_ticket.release(); s->d_pose_ticket.release();
   s->d_Au[0].release(); s->d_Au[1].release(); s->d_cost_partialsA.release();
   s->d_infos.release();
@@ -2628,8 +2453,8 @@ int ba_finalize(ba_solver *s) {
     for (auto &c : chunksA) cnt[c.j_opt]++;
     pose_chunk_ptr[0] = 0;
     for (int j = 0; j < s->N; ++j) pose_chunk_ptr[j + 1] = pose_chunk_ptr[j] + cnt[j];
-    // observations of FIXED poses, behind the free ones (chunks with j_opt = -1): only the speculative pass
-    // (k_cost_linearize_by_pose) walks them, for the cost; k_linearize_by_pose launches the first n_chunksA chunks
+    // observations of FIXED poses, behind the free ones (chunks with j_opt = -1): k_cost_linearize_by_pose walks them
+    // for the cost only, so the first n_chunksA chunks are the ones with pose-side partials (d_partialsA)
     s->n_chunksA = (int)chunksA.size();
     long long f_at = nA;
     std::vector<long long> f_begin(Nt, -1);
@@ -2699,8 +2524,6 @@ int ba_finalize(ba_solver *s) {
   CUDA_TRY(s->d_inc_b.upload(inc_b, st));
   CUDA_TRY(s->d_tile_batches.upload(tile_batches, st));
   CUDA_TRY(s->d_cta_batch_ptr.upload(cta_batch_ptr, st));
-  // BA_B200_TILE_FLUSH=atomic: the earlier flush (one FP64 red per entry straight into S), for A/B runs
-  if (getenv("BA_B200_TILE_FLUSH") && std::string(getenv("BA_B200_TILE_FLUSH")) == "atomic") { cta_seg_ptr.clear(); stage_doubles = 0; }
   CUDA_TRY(s->d_cta_seg_ptr.upload(cta_seg_ptr, st));
   CUDA_TRY(s->d_seg_off.upload(seg_off, st));
   CUDA_TRY(s->d_seg_win.upload(seg_win, st));
@@ -2755,10 +2578,8 @@ int ba_finalize(ba_solver *s) {
   CUDA_TRY(cudaMemsetAsync(s->d_Btx.p, 0, s->d_Btx.n * sizeof(double), st));
   CUDA_TRY(cudaMemsetAsync(s->d_A.p, 0, s->d_A.n * sizeof(double), st));
   CUDA_TRY(cudaMemsetAsync(s->d_a.p, 0, s->d_a.n * sizeof(double), st));
-  s->cost_grid = (int)std::min<long long>(148 * 8, std::max<long long>(1, (n + kThreads - 1) / kThreads));
   s->point_grid = std::max(1, (Mt + kThreads - 1) / kThreads);
   s->pose_grid = std::max(1, (Nt + kThreads - 1) / kThreads);
-  CUDA_TRY(s->d_cost_partials.alloc(s->cost_grid));
   CUDA_TRY(s->d_point_partials.alloc(2 * (size_t)s->point_grid));
   CUDA_TRY(s->d_pose_partials.alloc(2 * (size_t)s->pose_grid));
   CUDA_TRY(s->d_scal.alloc(8));
@@ -2822,18 +2643,17 @@ namespace {
 
 struct Phase { enum { Lin = 0, Schur, Solve, Backsub, Update, End, Count }; };
 
-// BA_B200_SPEC_LIN=0: the trial cost in point order and a separate pose-side pass per iteration (k_cost_decide +
-// k_linearize_by_pose) instead of the speculative pose side (k_cost_linearize_by_pose + k_pose_diag)
-// (read at every ba_solve, so that one process can run both forms; the captured graph is keyed on it)
-static bool spec_lin(const ba_solver *s) {
-  const char *e = getenv("BA_B200_SPEC_LIN");
-  return !(e && atoi(e) == 0) && s->n_chunksA_all > 0;
+// BA_B200_REDUCE_STORES=0: clear of S + k_pose_diag + adding k_tile_reduce instead of the storing reduce on banded
+// plans (A/B runs; the two forms are bit-identical).  Read by every entry point that builds, so that one process can
+// run both forms; the captured graph is keyed on it.
+static void read_reduce_stores(ba_solver *s) {
+  const char *e = getenv("BA_B200_REDUCE_STORES");
+  s->rs_now = !(e && atoi(e) == 0);
 }
 
-static DecideArgs make_decide_args(ba_solver *s, const ba_options *opt, bool spec = false) {
+static DecideArgs make_decide_args(ba_solver *s, const ba_options *opt) {
   DecideArgs g;
-  g.cost_partials = s->d_cost_partials.p; g.n_cost = s->cost_grid;
-  if (spec) { g.cost_partials = s->d_cost_partialsA.p; g.n_cost = s->n_chunksA_all; }
+  g.cost_partials = s->d_cost_partialsA.p; g.n_cost = s->n_chunksA_all;
   g.point_partials = s->d_point_partials.p; g.n_point = s->point_grid;
   g.pose_partials = s->d_pose_partials.p; g.n_pose = s->pose_grid;
   g.scal = s->d_scal.p;
@@ -2863,7 +2683,7 @@ static int ensure_S_clean(ba_solver *s) {
 }
 
 // Enqueue the build (K1..K4) on the stream.  ev: optional events at phase boundaries.
-static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev, bool spec = false) {
+static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
   cudaStream_t st = s->stream;
   const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
   const double thres = (double)opt->threshold_huber_loss;
@@ -2872,12 +2692,11 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev, b
   if (ev) cudaEventRecord(ev[Phase::Lin], st);
   // BA_B200_BAND_CLEAR_MIN_MB: size of the dense buffer above which only the band is cleared (tests force 0)
   static const size_t band_clear_min = (size_t)(getenv("BA_B200_BAND_CLEAR_MIN_MB") ? atoi(getenv("BA_B200_BAND_CLEAR_MIN_MB")) : 64) << 20;
-  // Speculative pose side on a banded plan with the deterministic tile flush: k_tile_reduce WRITES every band entry
-  // and rhs entry of S (damped pose-side sums + windows) and the rows of A / a, so nothing is cleared here and
-  // k_pose_diag is not launched (BA_B200_REDUCE_STORES=0: clear + k_pose_diag + adding reduce)
-  const bool reduce_stores = spec && s->rs_now && s->N > 0 && s->n_schur_chunks > 0 &&
-                             s->d_cta_seg_ptr.n > 0 && s->chol.banded && s->S_clean_outside_band &&
-                             std::max(s->stage_span, s->chol.bw) + 2 <= 2 * 96;
+  // On a banded plan k_tile_reduce WRITES every band entry and rhs entry of S (damped pose-side sums + windows) and
+  // the rows of A / a, so nothing is cleared here and k_pose_diag is not launched (BA_B200_REDUCE_STORES=0: clear +
+  // k_pose_diag + adding reduce)
+  const bool reduce_stores = s->rs_now && s->N > 0 && s->n_schur_chunks > 0 && s->chol.banded &&
+                             s->S_clean_outside_band && std::max(s->stage_span, s->chol.bw) + 2 <= 2 * 96;
   if (reduce_stores) {
     // nothing to clear
   } else if (s->chol.banded && s->S_clean_outside_band && (size_t)ld * ld * sizeof(double) > band_clear_min) {
@@ -2894,19 +2713,10 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev, b
     k_zero_split<<<(s->n_split + 127) / 128, 128, 0, st>>>(s->d_split_points.p, s->n_split, s->d_ptblk.p, s->Mp, dst);
     s->launches++;
   }
-  // pose side first: the per-pose finish of k_linearize_by_pose STORES the damped diagonal blocks and the rhs,
-  // everything after it adds
-  if (spec) {
-    // the sums of the accepted buffer are there (the trial-cost pass of the previous iteration, or the initial pass)
-    if (s->N > 0 && !reduce_stores) {
-      k_pose_diag<<<(s->N + 3) / 4, 128, 0, st>>>(s->N, s->d_Au[0].p, s->d_Au[1].p, s->d_A.p, s->d_a.p, s->d_Saug.p, ld, dst);
-      s->launches++;
-    }
-  } else if (s->n_chunksA > 0) {
-    k_linearize_by_pose<<<s->n_chunksA, kThreads, 0, st>>>(s->d_chunksA.p, s->d_uvA.p, s->d_pointA.p,
-                                                           s->d_camA.p, s->d_poseidA.p, prm, s->d_cams.p, thres,
-                                                           s->d_partialsA.p, s->d_pose_chunk_ptr.p, s->d_pose_ticket.p,
-                                                           s->d_A.p, s->d_a.p, s->d_Saug.p, ld, dst);
+  // pose side first: k_pose_diag STORES the damped diagonal blocks and the rhs, everything after it adds.  The sums
+  // of the accepted buffer are there (the trial-cost pass of the previous iteration, or the initial pass)
+  if (s->N > 0 && !reduce_stores) {
+    k_pose_diag<<<(s->N + 3) / 4, 128, 0, st>>>(s->N, s->d_Au[0].p, s->d_Au[1].p, s->d_A.p, s->d_a.p, s->d_Saug.p, ld, dst);
     s->launches++;
   }
   // landmarks on the by-point path (poses do not fit a window, or not enough neighbours for a chunk)
@@ -2943,19 +2753,18 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev, b
     }
     const TileLaunch &tl = s->tile_launch;
     const size_t smem = (size_t)tl.G * tl.bufD * sizeof(double);
-    const int *stage_tab = s->d_cta_seg_ptr.n > 0 ? s->d_cta_seg_ptr.p : nullptr;
     if (opt->b_accumulate)
       k_build_tiles<true><<<tl.n_cta, kT2Threads, smem, st>>>(
           s->d_schur_chunks.p, s->d_tile_batches.p, s->d_cta_batch_ptr.p, tl, s->d_tpt_point.p, s->d_tpt_inc_start.p,
           s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p,
-          s->Pp, s->d_ptblk.p, s->Mp, s->d_Saug.p, ld, stage_tab, s->d_seg_off.p, s->d_stage.p, dst);
+          s->Pp, s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
     else
       k_build_tiles<false><<<tl.n_cta, kT2Threads, smem, st>>>(
           s->d_schur_chunks.p, s->d_tile_batches.p, s->d_cta_batch_ptr.p, tl, s->d_tpt_point.p, s->d_tpt_inc_start.p,
           s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p,
-          s->Pp, s->d_ptblk.p, s->Mp, s->d_Saug.p, ld, stage_tab, s->d_seg_off.p, s->d_stage.p, dst);
+          s->Pp, s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
     s->launches++;
-    if (stage_tab && s->N > 0) {
+    if (s->N > 0) {
       k_tile_reduce<<<6 * s->N, 96, 0, st>>>(6 * s->N, ld, s->stage_span, s->d_seg_win.p, s->d_pose_seg.p, s->d_stage.p,
                                              s->d_Saug.p, reduce_stores ? s->chol.bw : -1, s->d_Au[0].p, s->d_Au[1].p,
                                              s->d_A.p, s->d_a.p, dst);
@@ -3063,48 +2872,27 @@ static int enqueue_solve_backsub(ba_solver *s, const ba_options *opt, cudaEvent_
 static void launch_cost_linearize(ba_solver *s, const ba_options *opt, int which, int decide_here, int ignore_done,
                                   const DecideArgs &g) {
   const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
-  k_cost_linearize_by_pose<<<s->n_chunksA_all, kThreads, 0, s->stream>>>(
-      s->d_chunksA.p, s->d_uvA.p, s->d_pointA.p, s->d_camA.p, s->d_poseidA.p, prm, which, s->d_cams.p,
+  k_cost_linearize_by_pose<<<std::max(1, s->n_chunksA_all), kThreads, 0, s->stream>>>(
+      s->d_chunksA.p, s->d_uvA.p, s->d_pointA.p, s->d_camA.p, s->d_poseidA.p, s->n_chunksA_all, prm, which, s->d_cams.p,
       (double)opt->threshold_huber_loss, s->d_partialsA.p, s->d_cost_partialsA.p, s->d_pose_chunk_ptr.p,
       s->d_pose_ticket.p, s->d_Au[0].p, s->d_Au[1].p, s->d_ticket.p, decide_here, ignore_done, g, s->d_state.p,
       s->d_infos.p, (int)s->d_infos.n);
 }
 
-static int enqueue_update_decide(ba_solver *s, const ba_options *opt, cudaEvent_t *ev, bool spec = false) {
+static int enqueue_update_decide(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
   cudaStream_t st = s->stream;
-  const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
   LmState *dst = s->d_state.p;
   if (ev) cudaEventRecord(ev[Phase::Update], st);
   // the pose update (se3Exp, pose part of the model change) ran with the back-substitution of the landmarks
   // (k_backsub_points_update_poses; a forked graph branch for it cost more than the 9 us it hid)
-  DecideArgs g = make_decide_args(s, opt, spec);
-  if (spec) {
-    launch_cost_linearize(s, opt, 1, s->comm ? 0 : 1, 0, g);
-    s->launches++;
-    if (!s->comm) {
-      if (ev) cudaEventRecord(ev[Phase::End], st);
-      return BA_OK;
-    }
-  } else if (!s->comm) {
-    k_cost_decide<<<s->cost_grid, kThreads, 0, st>>>(s->n_obs, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                                     s->d_obs_camflags.p, prm, s->d_cams.p, s->d_cost_partials.p,
-                                                     s->d_ticket.p, g, dst, s->d_infos.p, (int)s->d_infos.n);
-    s->launches += 1;
-    if (ev) cudaEventRecord(ev[Phase::End], st);
-    return BA_OK;
-  }
-  if (!spec) {
-    k_cost<<<s->cost_grid, kThreads, 0, st>>>(s->n_obs, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                              s->d_obs_camflags.p, prm, 1, s->d_cams.p, s->d_cost_partials.p, 0, dst);
-    s->launches += 1;
-  }
-  if (!s->comm) {
-    k_reduce_decide<<<1, kThreads, 0, st>>>(g, dst, s->d_infos.p, (int)s->d_infos.n);
-    s->launches++;
-  } else if (s->shared && s->shared->peer_ok) {
+  DecideArgs g = make_decide_args(s, opt);
+  // single GPU: the trial-cost pass also takes the decision; several GPUs exchange the partial sums first
+  launch_cost_linearize(s, opt, 1, s->comm ? 0 : 1, 0, g);
+  s->launches++;
+  if (s->comm && s->shared && s->shared->peer_ok) {
     k_exchange_decide<<<1, kThreads, 0, st>>>(g, s->shared->table(), dst, s->d_infos.p, (int)s->d_infos.n);
     s->launches++;
-  } else {
+  } else if (s->comm) {
     k_reduce_scalars<<<1, kThreads, 0, st>>>(g, 0, dst);
     if (int rc = enqueue_allreduce_scal(s)) return rc;
     k_decide<<<1, 1, 0, st>>>(g, dst, s->d_infos.p, (int)s->d_infos.n);
@@ -3130,11 +2918,21 @@ static int check_nd_error(ba_solver *s) {
 }
 
 static int enqueue_iteration(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
-  const bool spec = s->spec_now;
-  if (int rc = enqueue_build(s, opt, ev, spec)) return rc;
+  if (int rc = enqueue_build(s, opt, ev)) return rc;
   if (int rc = enqueue_allreduce_S(s)) return rc;
   if (int rc = enqueue_solve_backsub(s, opt, ev)) return rc;
-  return enqueue_update_decide(s, opt, ev, spec);
+  return enqueue_update_decide(s, opt, ev);
+}
+
+// Cost of the accepted parameters (buffer cur) into scal[0], ordered over the pose-order chunks (and summed over the
+// ranks), together with their pose-side sums in Au[cur]: the initial cost of ba_solve and the sums its first
+// iteration starts from.  Ignores `done`.
+static int enqueue_current_cost(ba_solver *s, const ba_options *opt) {
+  DecideArgs g = make_decide_args(s, opt);
+  launch_cost_linearize(s, opt, 0, 0, 1, g);
+  k_reduce_scalars<<<1, kThreads, 0, s->stream>>>(g, 1, s->d_state.p);
+  s->launches += 2;
+  return enqueue_allreduce_scal(s);
 }
 
 }  // namespace
@@ -3145,15 +2943,11 @@ int ba_cost(ba_solver *s, double *cost) {
   if (!s || !cost) return BA_ERR_INVALID;
   if (int rc = ba_finalize(s)) return rc;
   CUDA_TRY(cudaSetDevice(s->device));
-  const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
-  k_cost<<<s->cost_grid, kThreads, 0, s->stream>>>(s->n_obs, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                                   s->d_obs_camflags.p, prm, 0, s->d_cams.p,
-                                                   s->d_cost_partials.p, 1, s->d_state.p);
+  // no options here, so no Huber threshold: the pose-side sums this leaves in Au[cur] are not meaningful.  Nothing
+  // reads them -- ba_solve and ba_build_only form Au[cur] again before they use it
   ba_options o{};
   o.max_num_iterations = 1;
-  DecideArgs g = make_decide_args(s, &o);
-  k_reduce_scalars<<<1, kThreads, 0, s->stream>>>(g, 1, s->d_state.p);
-  if (int rc = enqueue_allreduce_scal(s)) return rc;
+  if (int rc = enqueue_current_cost(s, &o)) return rc;
   CUDA_TRY(cudaMemcpyAsync(s->h_scal, s->d_scal.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
   CUDA_TRY(cudaStreamSynchronize(s->stream));
   *cost = s->h_scal[0];
@@ -3176,27 +2970,12 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
   s->launches = 0;
   CUDA_TRY(s->d_infos.alloc(std::max(1, max_it)));
   if (int rc = ensure_S_clean(s)) return rc;
-  // --- initial cost (:707) and state
-  {
-    const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
-    const bool spec = s->spec_now = spec_lin(s);
-    {
-      const char *e = getenv("BA_B200_REDUCE_STORES");
-      s->rs_now = !(e && atoi(e) == 0);
-    }
-    DecideArgs g = make_decide_args(s, &opt, spec);
-    if (spec)   // initial cost + the pose-side sums of the initial parameters (buffer cur)
-      launch_cost_linearize(s, &opt, 0, 0, 1, g);
-    else
-      k_cost<<<s->cost_grid, kThreads, 0, st>>>(s->n_obs, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                                s->d_obs_camflags.p, prm, 0, s->d_cams.p, s->d_cost_partials.p, 1,
-                                                s->d_state.p);
-    k_reduce_scalars<<<1, kThreads, 0, st>>>(g, 1, s->d_state.p);
-    if (int rc = enqueue_allreduce_scal(s)) return rc;
-    k_init_state<<<1, 1, 0, st>>>(s->d_state.p, s->d_scal.p, (double)opt.initial_lambda);
-    s->launches += 3;
-    CUDA_TRY(cudaMemcpyAsync(s->h_scal, s->d_scal.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
-  }
+  read_reduce_stores(s);
+  // --- initial cost (:707), the pose-side sums of the initial parameters, and the state
+  if (int rc = enqueue_current_cost(s, &opt)) return rc;
+  k_init_state<<<1, 1, 0, st>>>(s->d_state.p, s->d_scal.p, (double)opt.initial_lambda);
+  s->launches++;
+  CUDA_TRY(cudaMemcpyAsync(s->h_scal, s->d_scal.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
   struct EventPair {   // destroyed on every return path
     cudaEvent_t a = nullptr, b = nullptr;
     ~EventPair() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
@@ -3222,7 +3001,7 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
   if (use_graph && max_it > 0) {
     ba_options key = opt;
     key.check_every = 0;
-    if (!s->graph_exec || std::memcmp(&s->graph_opt, &key, sizeof(key)) != 0 || s->graph_spec != s->spec_now || s->graph_rs != s->rs_now) {
+    if (!s->graph_exec || std::memcmp(&s->graph_opt, &key, sizeof(key)) != 0 || s->graph_rs != s->rs_now) {
       destroy_graph(s);
       cudaGraph_t graph;
       const long long l0 = s->launches;
@@ -3236,7 +3015,6 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
       CUDA_TRY(cudaGraphInstantiate(&s->graph_exec, graph, 0));
       cudaGraphDestroy(graph);
       s->graph_opt = key;
-      s->graph_spec = s->spec_now;
       s->graph_rs = s->rs_now;
     }
   }
@@ -3327,6 +3105,10 @@ int ba_build_only(ba_solver *s, const ba_options *opt_in, double lambda, int do_
     CUDA_TRY(s->d_Scopy.alloc(ldc * ldc));
   }
   if (int rc = ensure_S_clean(s)) return rc;
+  read_reduce_stores(s);
+  // the pose-side sums at the accepted parameters (Au[cur]), then the build of an iteration
+  DecideArgs g = make_decide_args(s, &opt);
+  launch_cost_linearize(s, &opt, 0, /*decide_here*/0, /*ignore_done*/1, g);
   if (int rc = enqueue_build(s, &opt, nullptr)) return rc;
   if (int rc = enqueue_allreduce_S(s)) return rc;
   if (do_solve) {

@@ -20,6 +20,7 @@
 //     accumulators in registers across all batches of a chunk, flushed into a staging window when the chunk changes)
 //     and hand them back: full[g] / empty[g] named barriers, nothing else; a producer clears the few window slots its
 //     landmark does not cover instead of anybody clearing whole buffers.
+// B is never stored to global memory: k_backsub_tiles (end of this file) forms it again for the back-substitution.
 #pragma once
 
 constexpr int kT2LB = 8;                  // landmarks per batch (one producer warp, 4 lanes per landmark)
@@ -61,8 +62,8 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
                const int *__restrict__ tpt_inc_start, const int4 *__restrict__ inc_a /*obs_first, n_obs, pose, pair*/,
                const int2 *__restrict__ inc_b /*slot (-1: fixed pose), camera slots of obs 0 | obs 1 << 8*/,
                const double2 *__restrict__ obs_uv, const int *__restrict__ obs_camflags, Params prm,
-               const double *__restrict__ cams, double thres_huber, double *__restrict__ Bsoa, size_t Pp,
-               double *__restrict__ ptblk, size_t Mp, const int *__restrict__ cta_seg_ptr /*first staging segment of every CTA*/,
+               const double *__restrict__ cams, double thres_huber, double *__restrict__ ptblk, size_t Mp,
+               const int *__restrict__ cta_seg_ptr /*first staging segment of every CTA*/,
                const long long *__restrict__ seg_off, double *__restrict__ stage, const LmState *__restrict__ st) {
   if (st->done) return;
   extern __shared__ double tsm[];
@@ -177,14 +178,10 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
           const double2 uv = obs_uv[k];
           const int kk = k - ia.x;
           const int cid = (kk == 0) ? (cams01 & 0xff) : (kk == 1) ? (cams01 >> 8) : (obs_camflags[k] & kCamMask);
-          const double *cam = cams + cid * kCamStride;
-          Proj pr;
-          project(T, Xc, cam, uv.x, uv.y, pr);
-          const double w = huber_weight(pr.r0, pr.r1, thres_huber);
-          const double wr0 = w * pr.r0, wr1 = w * pr.r1;
-          double Gm[6], Rm[6];
-          jac_G(pr, cam, Gm);
-          jac_R(Gm, T, Rm);
+          ObsLin o;
+          linearize_obs(T, Xc, cams + cid * kCamStride, uv.x, uv.y, thres_huber, o);
+          const double w = o.w, wr0 = w * o.pr.r0, wr1 = w * o.pr.r1;
+          const double *Rm = o.Rm;
           cp[0] += w * (Rm[0] * Rm[0] + Rm[3] * Rm[3]);
           cp[1] += w * (Rm[0] * Rm[1] + Rm[3] * Rm[4]);
           cp[2] += w * (Rm[0] * Rm[2] + Rm[3] * Rm[5]);
@@ -194,14 +191,7 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
           cp[6] -= Rm[0] * wr0 + Rm[3] * wr1;
           cp[7] -= Rm[1] * wr0 + Rm[4] * wr1;
           cp[8] -= Rm[2] * wr0 + Rm[5] * wr1;
-          if (slot >= 0 && (ACCUM_B || k == ia.x + ia.y - 1)) {
-            double Q[12];
-            jac_Q(Gm, pr.Xb, Q);
-#pragma unroll
-            for (int r = 0; r < 6; ++r)
-#pragma unroll
-              for (int c = 0; c < 3; ++c) Bv[r * 3 + c] += w * (Q[r] * Rm[c] + Q[6 + r] * Rm[3 + c]);
-          }
+          if (slot >= 0 && (ACCUM_B || k == ia.x + ia.y - 1)) add_B(o, Bv);
         }
         }
         if (rd == 0 && fb - b0 >= G) bar_sync(8 + grp, bar_cnt);   // the consumers have read this buffer
@@ -211,10 +201,7 @@ k_build_tiles(const SchurChunk *__restrict__ chunks, const int4 *__restrict__ ba
 #pragma unroll
           for (int r = 0; r < 6; ++r)
 #pragma unroll
-            for (int c = 0; c < 3; ++c) {
-              Bbase[(3 * li + c) * ldB + 6 * slot + r] = Bv[r * 3 + c];
-              Bsoa[(size_t)(r * 3 + c) * Pp + ia.w] = Bv[r * 3 + c];
-            }
+            for (int c = 0; c < 3; ++c) Bbase[(3 * li + c) * ldB + 6 * slot + r] = Bv[r * 3 + c];
         }
       }
       if (rounds == 0 && fb - b0 >= G) bar_sync(8 + grp, bar_cnt);
@@ -499,5 +486,81 @@ __global__ void __launch_bounds__(96) k_tile_reduce(int n, int ld, int span /*la
     } else if (sum[u] != 0.0) {
       *dst += sum[u];
     }
+  }
+}
+
+// K6 for the tile landmarks: Btx[pt] = sum_j B_ji^T x_j.  k_build_tiles keeps B only in its shared-memory operands;
+// here B is formed again at the accepted parameters by the same linearize_obs / add_B (last observation of the
+// incidence, or all of them when ACCUM_B), which reads ~40 B per incidence instead of storing and reading back 144 B
+// per pair (C3: 72 MB written by the build + 76 MB read here, per iteration).  4 adjacent lanes per tile landmark, in
+// tile order, as in the producers of k_build_tiles: lane sub takes incidences sub, sub + 4, ...; the 4 partials are
+// combined with the xor butterfly (fixed order: bit-reproducible, no atomics) and stored, zeros for a landmark without
+// a free incidence.  The kernel is bound by its chain of dependent gathers (landmark -> incidences -> pose, pixel ->
+// x), so the landmarks are numbered directly rather than through the batch list, and the free-pose index of x comes
+// from pose_opt (same level as the pose) rather than from the chunk's window.
+// Registers: reference mode runs three CTAs per SM (80 registers, 56 B of spill stores) because that measured faster
+// than two CTAs without spills (108 registers); back-substitution phase on one B200 at 1000 W, C3 / C4 / C5: 29.7 /
+// 232 / 373 us against 29.7 / 268 / 412 us (profiles/r03_bench_*_backsub_2cta.json).  Corrected mode keeps two CTAs
+// (128 registers, 24 B of spill stores; at three it spills 364 B).
+template <bool ACCUM_B>
+__global__ void __launch_bounds__(256, ACCUM_B ? 2 : 3)
+k_backsub_tiles(int n_tpt, const int *__restrict__ tpt_point, const int *__restrict__ tpt_inc_start,
+                const int4 *__restrict__ inc_a, const int2 *__restrict__ inc_b, const double2 *__restrict__ obs_uv,
+                const int *__restrict__ obs_camflags, const int *__restrict__ pose_opt, Params prm,
+                const double *__restrict__ cams, double thres_huber, const double *__restrict__ x,
+                double *__restrict__ Btx /*[3][Mp]*/, size_t Mp, const LmState *__restrict__ st) {
+  if (st->done) return;
+  const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+  if ((gt & ~31) >= 4 * n_tpt) return;   // whole warps
+  const int ti = gt >> 2, sub = gt & 3;
+  const bool live = ti < n_tpt;
+  int pt = 0;
+  double v[3] = {0.0, 0.0, 0.0};
+  if (live) {
+    const int a = __ldg(tpt_inc_start + ti), b = __ldg(tpt_inc_start + ti + 1);
+    pt = __ldg(tpt_point + ti);
+    const double *poses = prm.poses[st->cur];
+    const double *points = prm.points[st->cur];
+    const double X[3] = {__ldg(points + (size_t)pt * 3), __ldg(points + (size_t)pt * 3 + 1),
+                         __ldg(points + (size_t)pt * 3 + 2)};
+    for (int ii = a + sub; ii < b; ii += 4) {
+      const int2 sc = __ldg(inc_b + ii);
+      const int4 ia = __ldg(inc_a + ii);
+      if (sc.x < 0) continue;   // fixed pose: no B block
+      const int j = __ldg(pose_opt + ia.z);   // = window start + sc.x
+      double T[12];
+      load_pose(poses + (size_t)ia.z * 12, T);
+      double Bv[18];
+#pragma unroll
+      for (int i = 0; i < 18; ++i) Bv[i] = 0.0;
+      for (int k = ACCUM_B ? ia.x : ia.x + ia.y - 1; k < ia.x + ia.y; ++k) {
+        const double2 uv = obs_uv[k];
+        const int kk = k - ia.x;   // camera: the producers' rule
+        const int cid = (kk == 0) ? (sc.y & 0xff) : (kk == 1) ? (sc.y >> 8) : (obs_camflags[k] & kCamMask);
+        ObsLin o;
+        linearize_obs(T, X, cams + cid * kCamStride, uv.x, uv.y, thres_huber, o);
+        add_B(o, Bv);
+      }
+      const double *xj = x + (size_t)6 * j;
+      double xv[6];
+#pragma unroll
+      for (int r = 0; r < 6; ++r) xv[r] = __ldg(xj + r);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        double s = 0.0;
+#pragma unroll
+        for (int r = 0; r < 6; ++r) s += Bv[r * 3 + c] * xv[r];
+        v[c] += s;
+      }
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    v[c] += __shfl_xor_sync(0xffffffffu, v[c], 1);
+    v[c] += __shfl_xor_sync(0xffffffffu, v[c], 2);
+  }
+  if (live && sub == 0) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) Btx[(size_t)c * Mp + pt] = v[c];
   }
 }

@@ -103,6 +103,31 @@ __device__ __forceinline__ void jac_R(const double *G, const double *__restrict_
       Rm[r * 3 + c] = G[r * 3] * T[c] + G[r * 3 + 1] * T[3 + c] + G[r * 3 + 2] * T[6 + c];
 }
 
+// One observation linearised for the landmark side: residual, Huber weight, G and Rm (full...cpp:733-814).
+struct ObsLin {
+  Proj pr;
+  double w;
+  double G[6], Rm[6];
+};
+__device__ __forceinline__ void linearize_obs(const double *__restrict__ T, const double *__restrict__ X,
+                                              const double *__restrict__ cam, double u, double v, double thres,
+                                              ObsLin &o) {
+  project(T, X, cam, u, v, o.pr);
+  o.w = huber_weight(o.pr.r0, o.pr.r1, thres);
+  jac_G(o.pr, cam, o.G);
+  jac_R(o.G, T, o.Rm);
+}
+// Bv (6x3 row-major) += w Q^T Rm, the observation's share of the pose-landmark block B_ji (:826).  Every kernel that
+// forms B calls this, so the Schur complement, the back-substitution and the debug dump see the same B.
+__device__ __forceinline__ void add_B(const ObsLin &o, double *Bv) {
+  double Q[12];
+  jac_Q(o.G, o.pr.Xb, Q);
+#pragma unroll
+  for (int r = 0; r < 6; ++r)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) Bv[r * 3 + c] += o.w * (Q[r] * o.Rm[c] + Q[6 + r] * o.Rm[3 + c]);
+}
+
 // se3Exp (full...cpp:1046-1082), xi = [v; w]; out = R row-major 9 | t 3
 __device__ __forceinline__ void se3_exp(const double *xi, double *out) {
   const double v0 = xi[0], v1 = xi[1], v2 = xi[2];

@@ -19,7 +19,9 @@
 //                             (k_nd_persistent, nested-dissection fronts over many CTAs, ba_cholesky_nd.cuh), cluster
 //                             (small dense, ba_cholesky_cluster.cuh), multi-kernel blocked DMMA (large dense,
 //                             ba_cholesky.cuh); the serial window kernel of ba_cholesky_banded.cuh is the fallback
-//   K6 k_backsub_pairs, k_backsub_points_update_poses : y = C^-1 b - C^-1 sum_j B^T x_j, model change, trial points
+//   K6 k_backsub_tiles / k_backsub_pairs, k_backsub_points_update_poses : y = C^-1 b - C^-1 sum_j B^T x_j (tile
+//                             landmarks: B formed again from their observations, ba_build_tiles.cuh; by-point landmarks:
+//                             the stored B), model change, trial points
 //                             (:910-917,:435-455) and, in the same launch, the se3Exp pose update (:922-927);
 //                             gradient-descent variant for FullBundleAdjustmentSolverRefactor::SolveByGradientDescent
 //   K7 k_cost_linearize_by_pose : trial cost in pose order + the pose-side sums at the trial parameters; the last CTA
@@ -210,6 +212,7 @@ k_linearize_by_point(const Chunk *__restrict__ chunks, const int2 *__restrict__ 
 // K1b: off-diagonal blocks.  One thread per (pose, point) pair: B_ji = w Q^T Rm of the pair's LAST inserted
 // observation (reference-exact, full...cpp:826) or the sum over the pair's observations (corrected mode).
 // Every lane does useful work and consecutive pairs write consecutive slots of the component-major Bsoa.
+// Launched over the by-point pairs, or over every pair (list = null) when the blocks are kept for ba_debug_dump.
 template <bool ACCUM_B>
 __global__ void __launch_bounds__(kThreads, ACCUM_B ? 2 : 3)
 k_pair_blocks(int n_list, const int *__restrict__ list /*pair indices, or null = identity*/,
@@ -236,18 +239,9 @@ k_pair_blocks(int n_list, const int *__restrict__ list /*pair indices, or null =
   X[2] = __ldg(points + (size_t)pt * 3 + 2);
   for (int k = ACCUM_B ? po.x : po.y; k <= po.y; ++k) {
     const double2 uv = obs_uv[k];
-    const double *cam = cams + (obs_camflags[k] & kCamMask) * kCamStride;
-    Proj pr;
-    project(T, X, cam, uv.x, uv.y, pr);
-    const double w = huber_weight(pr.r0, pr.r1, thres_huber);
-    double G[6], Rm[6], Q[12];
-    jac_G(pr, cam, G);
-    jac_R(G, T, Rm);
-    jac_Q(G, pr.Xb, Q);
-#pragma unroll
-    for (int r = 0; r < 6; ++r)
-#pragma unroll
-      for (int c = 0; c < 3; ++c) Bv[r * 3 + c] += w * (Q[r] * Rm[c] + Q[6 + r] * Rm[3 + c]);
+    ObsLin o;
+    linearize_obs(T, X, cams + (obs_camflags[k] & kCamMask) * kCamStride, uv.x, uv.y, thres_huber, o);
+    add_B(o, Bv);
   }
 #pragma unroll
   for (int i = 0; i < 18; ++i) Bsoa[(size_t)i * Pp + p] = Bv[i];
@@ -417,7 +411,7 @@ k_schur_pairs_list(int n_list, const int *__restrict__ list /*pair indices p1, o
 // ---------------------------------------------------------------------------
 // K6: back-substitution.
 // ---------------------------------------------------------------------------
-// per pair: w = B^T x_j ; segmented sum by point -> Btx[pt]
+// by-point landmarks (the tile landmarks: k_backsub_tiles), per pair: w = B^T x_j ; segmented sum by point -> Btx[pt]
 __global__ void __launch_bounds__(kThreads)
 k_backsub_pairs(const Chunk *__restrict__ chunks, const int *__restrict__ chunk_pair_count,
                 const int *__restrict__ pair_pose, const int *__restrict__ pair_point,
@@ -1595,26 +1589,24 @@ struct ba_solver {
   std::vector<int> h_pose_opt, h_point_opt, h_opt_pose, h_opt_point;
   std::vector<int> h_pair_pose, h_pair_point;  // j_opt, original point id
   std::vector<int> h_first_pose;               // per free pose: first co-visible free pose (envelope of S)
-  int n_chunks = 0, n_chunksA = 0, n_split = 0, n_split_pairs = 0;
+  int n_chunksA = 0, n_split = 0, n_split_pairs = 0;
 
   // device problem
   DevBuf<double> d_cams, d_poses[2], d_points[2];
   DevBuf<double2> d_obs_uv, d_uvA;
   DevBuf<int> d_obs_pose, d_obs_point, d_obs_camflags, d_obs_pair;
   DevBuf<int> d_pointA, d_camA, d_poseidA;
-  DevBuf<Chunk> d_chunks;
-  DevBuf<int2> d_chunk_pts, d_pair_obs;
-  DevBuf<ChunkPoint> d_cpts;
-  DevBuf<int> d_chunk_pair_count;
+  DevBuf<int2> d_pair_obs;
   DevBuf<ChunkA> d_chunksA;
   DevBuf<int> d_pose_chunk_ptr, d_pose_opt, d_pair_pose, d_pair_point, d_pair_end, d_point_has_pairs;
   DevBuf<uint8_t> d_point_free;
-  DevBuf<int> d_split_points, d_split_pairs;
+  DevBuf<int> d_split_points;
   DevBuf<SchurChunk> d_schur_chunks;
   DevBuf<int> d_tpt_point, d_tpt_inc_start, d_fallback_pairs;
   DevBuf<int2> d_fb_groups;   // pair range of every by-point landmark (dense-GEMM Schur path of small systems)
   int n_fb_groups = 0;
   DevBuf<int4> d_inc_a, d_tile_batches;
+  int n_tpt = 0;   // tile landmarks
   DevBuf<int2> d_inc_b;
   DevBuf<int> d_cta_batch_ptr;
   // deterministic tile flush: one staging window per (CTA, chunk) segment of the batch list
@@ -1628,6 +1620,7 @@ struct ba_solver {
   DevBuf<Chunk> d_chunks_fb;
   DevBuf<int2> d_chunk_pts_fb;
   DevBuf<ChunkPoint> d_cpts_fb;
+  DevBuf<int> d_chunk_pair_count_fb;
   DevBuf<uint8_t> d_point_fb;
   int n_chunks_fb = 0;
   int n_schur_chunks = 0, n_fallback_pairs = 0;
@@ -1716,12 +1709,12 @@ static void free_device(ba_solver *s) {
   for (int i = 0; i < 2; ++i) { s->d_poses[i].release(); s->d_points[i].release(); }
   s->d_obs_uv.release(); s->d_uvA.release(); s->d_obs_pose.release(); s->d_obs_point.release();
   s->d_obs_camflags.release(); s->d_obs_pair.release(); s->d_pointA.release(); s->d_camA.release();
-  s->d_poseidA.release(); s->d_chunks.release(); s->d_chunk_pts.release(); s->d_pair_obs.release(); s->d_cpts.release(); s->d_chunk_pair_count.release(); s->d_chunksA.release();
+  s->d_poseidA.release(); s->d_pair_obs.release(); s->d_chunksA.release();
   s->d_pose_chunk_ptr.release(); s->d_pose_opt.release(); s->d_pair_pose.release(); s->d_pair_point.release();
   s->d_pair_end.release(); s->d_point_has_pairs.release(); s->d_point_free.release();
-  s->d_split_points.release(); s->d_split_pairs.release(); s->d_schur_chunks.release();
+  s->d_split_points.release(); s->d_schur_chunks.release();
   s->d_tpt_point.release(); s->d_tpt_inc_start.release(); s->d_fallback_pairs.release(); s->d_fb_groups.release();
-  s->d_inc_a.release(); s->d_inc_b.release(); s->d_tile_batches.release(); s->d_cta_batch_ptr.release(); s->d_cta_seg_ptr.release(); s->d_seg_off.release(); s->d_seg_win.release(); s->d_pose_seg.release(); s->d_stage.release(); s->d_chunks_fb.release(); s->d_chunk_pts_fb.release(); s->d_cpts_fb.release(); s->d_point_fb.release();
+  s->d_inc_a.release(); s->d_inc_b.release(); s->d_tile_batches.release(); s->d_cta_batch_ptr.release(); s->d_cta_seg_ptr.release(); s->d_seg_off.release(); s->d_seg_win.release(); s->d_pose_seg.release(); s->d_stage.release(); s->d_chunks_fb.release(); s->d_chunk_pts_fb.release(); s->d_cpts_fb.release(); s->d_chunk_pair_count_fb.release(); s->d_point_fb.release();
   s->d_chol_rows.release(); s->d_chol_first.release(); s->d_chol_rows_ptr.release(); s->d_band.release();
   s->d_nd_nodes.release(); s->d_nd_level_nodes.release(); s->d_nd_cta_nodes.release(); s->d_nd_cta_ptr.release();
   s->d_nd_flags.release(); s->d_nd_helpers.release(); s->d_nd_L.release(); s->d_nd_U.release();
@@ -2295,15 +2288,15 @@ int ba_finalize(ba_solver *s) {
   s->n_schur_chunks = (int)schur_chunks.size();
   s->n_fallback_pairs = (int)fallback_pairs.size();
   lap("cholesky plan");
-  // --- chunks of whole points (<= kThreads observations); longer points are split.  Built twice: over all
-  //     landmarks (back-substitution, cost) and over the landmarks of the by-point path only (linearisation)
+  // --- chunks of whole points (<= kThreads observations) of the by-point path (linearisation, back-substitution);
+  //     longer points are split
   struct PointChunks {
     std::vector<Chunk> chunks;
     std::vector<int> chunk_pair_count, split_points, split_pairs;
     std::vector<int2> chunk_pts;
     std::vector<ChunkPoint> cpts;
   };
-  auto build_point_chunks = [&](bool skip_tile_points, long long q_begin, long long q_end) {
+  auto build_point_chunks = [&](long long q_begin, long long q_end) {
     PointChunks pc;
     long long q = q_begin;
     const long long n = q_end;     // this part's observations end here (shadows the total on purpose)
@@ -2329,7 +2322,7 @@ int ba_finalize(ba_solver *s) {
       long long e = q;
       while (e < n && o_point[e] == o_point[q]) ++e;
       const long long len = e - q;
-      if (skip_tile_points && is_tile_point[o_point[q]]) { flush(); q = e; continue; }
+      if (is_tile_point[o_point[q]]) { flush(); q = e; continue; }
       if (len > kThreads) {
         flush();
         if (s->h_point_opt[o_point[q]] >= 0) pc.split_points.push_back(o_point[q]);
@@ -2364,10 +2357,10 @@ int ba_finalize(ba_solver *s) {
     }
     return pc;
   };
-  // Both lists are serial scans; the landmark sequence is cut into kParts parts of about equal observation count
-  // (always kParts, whatever the number of host threads: the chunking, hence the summation order on the device, must
-  // not depend on the machine) that are scanned independently and concatenated
-  PointChunks pc_all, pc_fb;
+  // A serial scan; the landmark sequence is cut into kParts parts of about equal observation count (always kParts,
+  // whatever the number of host threads: the chunking, hence the summation order on the device, must not depend on
+  // the machine) that are scanned independently and concatenated
+  PointChunks pc_fb;
   {
     constexpr int kParts = 16;
     long long cut[kParts + 1];
@@ -2377,34 +2370,24 @@ int ba_finalize(ba_solver *s) {
       const int lm = (int)(std::lower_bound(pt_q0.begin(), pt_q0.end(), target) - pt_q0.begin());
       cut[p] = std::max(cut[p - 1], pt_q0[std::min(lm, Mt)]);
     }
-    std::vector<PointChunks> parts(2 * kParts);
-    parallel_ranges(2 * kParts, [&](long long lo_, long long hi_, int) {
-      for (long long j = lo_; j < hi_; ++j) parts[j] = build_point_chunks(j >= kParts, cut[j % kParts], cut[j % kParts + 1]);
+    std::vector<PointChunks> parts(kParts);
+    parallel_ranges(kParts, [&](long long lo_, long long hi_, int) {
+      for (long long j = lo_; j < hi_; ++j) parts[j] = build_point_chunks(cut[j], cut[j + 1]);
     }, 1);
-    auto merge = [&](PointChunks &dst, int first) {
-      for (int p = first; p < first + kParts; ++p) {
-        PointChunks &src = parts[p];
-        const int cp0 = (int)dst.cpts.size();
-        dst.chunks.insert(dst.chunks.end(), src.chunks.begin(), src.chunks.end());
-        dst.chunk_pair_count.insert(dst.chunk_pair_count.end(), src.chunk_pair_count.begin(), src.chunk_pair_count.end());
-        dst.split_points.insert(dst.split_points.end(), src.split_points.begin(), src.split_points.end());
-        dst.split_pairs.insert(dst.split_pairs.end(), src.split_pairs.begin(), src.split_pairs.end());
-        for (int2 cp : src.chunk_pts) dst.chunk_pts.push_back(make_int2(cp.x + cp0, cp.y));
-        dst.cpts.insert(dst.cpts.end(), src.cpts.begin(), src.cpts.end());
-      }
-    };
-    merge(pc_all, 0);
-    merge(pc_fb, kParts);
+    for (PointChunks &src : parts) {
+      PointChunks &dst = pc_fb;
+      const int cp0 = (int)dst.cpts.size();
+      dst.chunks.insert(dst.chunks.end(), src.chunks.begin(), src.chunks.end());
+      dst.chunk_pair_count.insert(dst.chunk_pair_count.end(), src.chunk_pair_count.begin(), src.chunk_pair_count.end());
+      dst.split_points.insert(dst.split_points.end(), src.split_points.begin(), src.split_points.end());
+      dst.split_pairs.insert(dst.split_pairs.end(), src.split_pairs.begin(), src.split_pairs.end());
+      for (int2 cp : src.chunk_pts) dst.chunk_pts.push_back(make_int2(cp.x + cp0, cp.y));
+      dst.cpts.insert(dst.cpts.end(), src.cpts.begin(), src.cpts.end());
+    }
   }
-  std::vector<Chunk> &chunks = pc_all.chunks;
-  std::vector<int> &chunk_pair_count = pc_all.chunk_pair_count;
-  std::vector<int> &split_points = pc_fb.split_points, &split_pairs = pc_all.split_pairs;
-  std::vector<int2> &chunk_pts = pc_all.chunk_pts;
-  std::vector<ChunkPoint> &cpts = pc_all.cpts;
-  s->n_chunks = (int)chunks.size();
   s->n_chunks_fb = (int)pc_fb.chunks.size();
-  s->n_split = (int)split_points.size();
-  s->n_split_pairs = (int)split_pairs.size();
+  s->n_split = (int)pc_fb.split_points.size();
+  s->n_split_pairs = (int)pc_fb.split_pairs.size();
   lap("point chunks");
   // --- pose-ordered arrays (free poses only) and their chunks
   // the pose-ordered copies of the observations (uvA, pointA, camA, poseidA) are gathered ON THE DEVICE from the
@@ -2501,10 +2484,6 @@ int ba_finalize(ba_solver *s) {
     CUDA_TRY(cudaGetLastError());
     d_perm.release();   // stream-ordered: freed after the gather
   }
-  CUDA_TRY(s->d_chunks.upload(chunks, st));
-  CUDA_TRY(s->d_chunk_pts.upload(chunk_pts, st));
-  CUDA_TRY(s->d_cpts.upload(cpts, st));
-  CUDA_TRY(s->d_chunk_pair_count.upload(chunk_pair_count, st));
   CUDA_TRY(s->d_chunksA.upload(chunksA, st));
   CUDA_TRY(s->d_pose_chunk_ptr.upload(pose_chunk_ptr, st));
   CUDA_TRY(s->d_pose_opt.upload(s->h_pose_opt, st));
@@ -2519,6 +2498,7 @@ int ba_finalize(ba_solver *s) {
   if (int rc = upload_cholesky_plan(s)) return rc;
   CUDA_TRY(s->d_schur_chunks.upload(schur_chunks, st));
   CUDA_TRY(s->d_tpt_point.upload(tpt_point, st));
+  s->n_tpt = (int)tpt_point.size();
   CUDA_TRY(s->d_tpt_inc_start.upload(tpt_inc_start, st));
   CUDA_TRY(s->d_inc_a.upload(inc_a, st));
   CUDA_TRY(s->d_inc_b.upload(inc_b, st));
@@ -2532,6 +2512,7 @@ int ba_finalize(ba_solver *s) {
   CUDA_TRY(s->d_chunks_fb.upload(pc_fb.chunks, st));
   CUDA_TRY(s->d_chunk_pts_fb.upload(pc_fb.chunk_pts, st));
   CUDA_TRY(s->d_cpts_fb.upload(pc_fb.cpts, st));
+  CUDA_TRY(s->d_chunk_pair_count_fb.upload(pc_fb.chunk_pair_count, st));
   {
     std::vector<uint8_t> point_fb(Mt);
     for (int i = 0; i < Mt; ++i) point_fb[i] = (!s->h_point_fixed[i] && !is_tile_point[i]) ? 1 : 0;
@@ -2551,8 +2532,7 @@ int ba_finalize(ba_solver *s) {
     s->n_fb_groups = (int)fb_groups.size();
     CUDA_TRY(s->d_fb_groups.upload(fb_groups, st));
   }
-  CUDA_TRY(s->d_split_points.upload(split_points, st));
-  CUDA_TRY(s->d_split_pairs.upload(split_pairs, st));
+  CUDA_TRY(s->d_split_points.upload(pc_fb.split_points, st));
   CUDA_TRY(cudaStreamSynchronize(st));
   lap("uploads");
   // --- block storage
@@ -2560,7 +2540,11 @@ int ba_finalize(ba_solver *s) {
   s->Pp = ((size_t)P + 31) / 32 * 32;
   const size_t nS = (size_t)6 * s->N + 1;
   CUDA_TRY(s->d_ptblk.alloc(std::max<size_t>(1, kPtBlk * s->Mp)));
-  CUDA_TRY(s->d_Bsoa.alloc(std::max<size_t>(1, 18 * s->Pp)));
+  // B blocks in global memory: by-point pairs, and every pair when they are kept for ba_debug_dump (the tile build
+  // keeps its blocks on chip, their back-substitution forms them again)
+  const bool keep_B = s->n_fallback_pairs > 0 || s->debug_keep;
+  if (keep_B) CUDA_TRY(s->d_Bsoa.alloc(std::max<size_t>(1, 18 * s->Pp)));
+  else s->d_Bsoa.release();
   CUDA_TRY(s->d_A.alloc(std::max<size_t>(1, (size_t)s->N * 36)));
   CUDA_TRY(s->d_a.alloc(std::max<size_t>(1, (size_t)s->N * 6)));
   CUDA_TRY(s->d_partialsA.alloc(std::max<size_t>(1, (size_t)s->n_chunksA * 27)));
@@ -2572,7 +2556,7 @@ int ba_finalize(ba_solver *s) {
   CUDA_TRY(s->d_Btx.alloc(std::max<size_t>(1, 3 * s->Mp)));
   CUDA_TRY(s->d_y.alloc(std::max<size_t>(1, (size_t)Mt * 3)));
   CUDA_TRY(cudaMemsetAsync(s->d_ptblk.p, 0, s->d_ptblk.n * sizeof(double), st));
-  CUDA_TRY(cudaMemsetAsync(s->d_Bsoa.p, 0, s->d_Bsoa.n * sizeof(double), st));
+  if (keep_B) CUDA_TRY(cudaMemsetAsync(s->d_Bsoa.p, 0, s->d_Bsoa.n * sizeof(double), st));
   CUDA_TRY(cudaMemsetAsync(s->d_x.p, 0, s->d_x.n * sizeof(double), st));
   CUDA_TRY(cudaMemsetAsync(s->d_y.p, 0, s->d_y.n * sizeof(double), st));
   CUDA_TRY(cudaMemsetAsync(s->d_Btx.p, 0, s->d_Btx.n * sizeof(double), st));
@@ -2727,16 +2711,19 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
                                                               s->d_ptblk.p, s->Mp, dst);
     s->launches++;
   }
-  if (s->n_fallback_pairs > 0) {
-    const int grid = (s->n_fallback_pairs + kThreads - 1) / kThreads;
+  // B of the by-point pairs; with debug_keep, of every pair (the tile build keeps its own on chip), for ba_debug_dump
+  const int n_blk = s->debug_keep ? (int)s->P : s->n_fallback_pairs;
+  if (n_blk > 0) {
+    const int grid = (n_blk + kThreads - 1) / kThreads;
+    const int *list = s->debug_keep ? nullptr : s->d_fallback_pairs.p;
     if (opt->b_accumulate)
-      k_pair_blocks<true><<<grid, kThreads, 0, st>>>(s->n_fallback_pairs, s->d_fallback_pairs.p, s->d_pair_obs.p,
-                                                     s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                                     s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p, s->Pp, dst);
+      k_pair_blocks<true><<<grid, kThreads, 0, st>>>(n_blk, list, s->d_pair_obs.p, s->d_obs_uv.p, s->d_obs_pose.p,
+                                                     s->d_obs_point.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres,
+                                                     s->d_Bsoa.p, s->Pp, dst);
     else
-      k_pair_blocks<false><<<grid, kThreads, 0, st>>>(s->n_fallback_pairs, s->d_fallback_pairs.p, s->d_pair_obs.p,
-                                                      s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p,
-                                                      s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p, s->Pp, dst);
+      k_pair_blocks<false><<<grid, kThreads, 0, st>>>(n_blk, list, s->d_pair_obs.p, s->d_obs_uv.p, s->d_obs_pose.p,
+                                                      s->d_obs_point.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres,
+                                                      s->d_Bsoa.p, s->Pp, dst);
     s->launches++;
   }
   if (s->n_chunks_fb > 0) {
@@ -2756,13 +2743,13 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
     if (opt->b_accumulate)
       k_build_tiles<true><<<tl.n_cta, kT2Threads, smem, st>>>(
           s->d_schur_chunks.p, s->d_tile_batches.p, s->d_cta_batch_ptr.p, tl, s->d_tpt_point.p, s->d_tpt_inc_start.p,
-          s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p,
-          s->Pp, s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
+          s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres,
+          s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
     else
       k_build_tiles<false><<<tl.n_cta, kT2Threads, smem, st>>>(
           s->d_schur_chunks.p, s->d_tile_batches.p, s->d_cta_batch_ptr.p, tl, s->d_tpt_point.p, s->d_tpt_inc_start.p,
-          s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres, s->d_Bsoa.p,
-          s->Pp, s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
+          s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p, s->d_obs_camflags.p, prm, s->d_cams.p, thres,
+          s->d_ptblk.p, s->Mp, s->d_cta_seg_ptr.p, s->d_seg_off.p, s->d_stage.p, dst);
     s->launches++;
     if (s->N > 0) {
       k_tile_reduce<<<6 * s->N, 96, 0, st>>>(6 * s->N, ld, s->stage_span, s->d_seg_win.p, s->d_pose_seg.p, s->d_stage.p,
@@ -2853,11 +2840,26 @@ static int enqueue_solve_backsub(ba_solver *s, const ba_options *opt, cudaEvent_
     cholesky_solve_enqueue(s->chol, s->d_Saug.p, s->d_x.p, s->d_z.p, s->d_linv.p, dst, st, &s->launches);
   }
   if (ev) cudaEventRecord(ev[Phase::Backsub], st);
+  // sum_j B^T x_j of every landmark with pairs: plain stores, except the pieces of a split by-point landmark (reds;
+  // tile landmarks are never split)
   if (!gd && s->n_split_pairs > 0) cudaMemsetAsync(s->d_Btx.p, 0, 3 * s->Mp * sizeof(double), st);
-  if (!gd && s->n_chunks > 0 && s->P > 0) {
-    k_backsub_pairs<<<s->n_chunks, kThreads, 0, st>>>(s->d_chunks.p, s->d_chunk_pair_count.p, s->d_pair_pose.p,
-                                                      s->d_pair_point.p, s->d_Bsoa.p, s->Pp, s->d_x.p,
-                                                      s->d_Btx.p, s->Mp, dst);
+  if (!gd && s->n_tpt > 0) {
+    const int grid = (4 * s->n_tpt + kThreads - 1) / kThreads;
+    const double thres = (double)opt->threshold_huber_loss;
+    if (opt->b_accumulate)
+      k_backsub_tiles<true><<<grid, kThreads, 0, st>>>(
+          s->n_tpt, s->d_tpt_point.p, s->d_tpt_inc_start.p, s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p,
+          s->d_obs_camflags.p, s->d_pose_opt.p, prm, s->d_cams.p, thres, s->d_x.p, s->d_Btx.p, s->Mp, dst);
+    else
+      k_backsub_tiles<false><<<grid, kThreads, 0, st>>>(
+          s->n_tpt, s->d_tpt_point.p, s->d_tpt_inc_start.p, s->d_inc_a.p, s->d_inc_b.p, s->d_obs_uv.p,
+          s->d_obs_camflags.p, s->d_pose_opt.p, prm, s->d_cams.p, thres, s->d_x.p, s->d_Btx.p, s->Mp, dst);
+    s->launches++;
+  }
+  if (!gd && s->n_fallback_pairs > 0) {
+    k_backsub_pairs<<<s->n_chunks_fb, kThreads, 0, st>>>(s->d_chunks_fb.p, s->d_chunk_pair_count_fb.p, s->d_pair_pose.p,
+                                                         s->d_pair_point.p, s->d_Bsoa.p, s->Pp, s->d_x.p,
+                                                         s->d_Btx.p, s->Mp, dst);
     s->launches++;
   }
   k_backsub_points_update_poses<<<s->point_grid + s->pose_grid, kThreads, 0, st>>>(
@@ -2988,9 +2990,10 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
   int it_launched = 0;
   int n_done = 0, converged = 0;
   const bool use_graph = opt.use_graph != 0 && !s->profile;   // NCCL collectives are captured with the kernels
-  if (s->debug_keep) {
+  if (s->debug_keep) {   // (debug switched on after ba_finalize: the B blocks may not be allocated yet)
     const size_t ld = (size_t)6 * s->N + 1;
     CUDA_TRY(s->d_Scopy.alloc(ld * ld));
+    CUDA_TRY(s->d_Bsoa.alloc(std::max<size_t>(1, 18 * s->Pp)));
   }
   if (s->comm && s->chol.banded && s->N > 0) {
     // exchange buffer of the band: allocated HERE, outside the capture (an allocation inside would become a graph
@@ -3103,6 +3106,7 @@ int ba_build_only(ba_solver *s, const ba_options *opt_in, double lambda, int do_
   if (s->debug_keep) {
     const size_t ldc = (size_t)6 * s->N + 1;
     CUDA_TRY(s->d_Scopy.alloc(ldc * ldc));
+    CUDA_TRY(s->d_Bsoa.alloc(std::max<size_t>(1, 18 * s->Pp)));
   }
   if (int rc = ensure_S_clean(s)) return rc;
   read_reduce_stores(s);
@@ -3187,7 +3191,8 @@ long long ba_debug_dump(ba_solver *s, int which, double *buf) {
       }
       return (long long)M * w;
     }
-    case 5:
+    case 5:   // every pair's B is stored only with debug_keep (the tile build keeps its blocks on chip)
+      if (P > 0 && (!s->debug_keep || s->d_Bsoa.n < 18 * s->Pp)) return BA_ERR_STATE;
       if (buf) {
         auto h = fetch(s->d_Bsoa.p, 18 * s->Pp);
         for (long long p = 0; p < P; ++p)

@@ -99,7 +99,7 @@ int ba_reset(ba_solver *s);                           /* Reset() (:44-70) */
 const char *ba_last_error(const ba_solver *s);
 int ba_set_stream(ba_solver *s, void *cuda_stream);   /* run on the caller's stream (e.g. torch's current stream) */
 int ba_set_profile(ba_solver *s, int enable);         /* per-phase CUDA events */
-int ba_set_debug(ba_solver *s, int keep_blocks);      /* keep a copy of S/rhs before factorisation for ba_debug_dump */
+int ba_set_debug(ba_solver *s, int keep_blocks);      /* keep S/rhs before factorisation and every pair's B for ba_debug_dump */
 
 /* ---- problem definition (host buffers; copied, never retained) --------- */
 /* AddCamera (full...cpp:72-85): ids are the user's camera indices; intr = fx,fy,cx,cy per camera
@@ -144,7 +144,8 @@ int ba_get_sizes(ba_solver *s, long long *out6); /* N_opt, M_opt, P(pairs), n_ob
  * which: 0 A (N*36, damped, row-major 6x6)  1 a (N*6)  2 C (M*9, damped)  3 b (M*3)  4 Cinv (M*9)
  *        5 B (P*18, row-major 6x3, pairs sorted by (point,pose))  6 S (n*n, symmetric, n=6N)
  *        7 rhs (n)  8 x (n)  9 y (M*3)  10 scalars {cost_prev,cost_new,model,rho,lambda}
- * buf == NULL returns the element count.  Free blocks are indexed by free index in id order. */
+ * buf == NULL returns the element count.  Free blocks are indexed by free index in id order.  S, rhs and B are
+ * kept only with ba_set_debug(s, 1): without it these return BA_ERR_STATE. */
 long long ba_debug_dump(ba_solver *s, int which, double *buf);
 int ba_debug_pairs(ba_solver *s, int *pair_pose_id, int *pair_point_id); /* original ids per pair */
 /* In-situ timing of parts of the reduced solve (bit 0 diag, 1 trsm, 2 syrk, 3 backward); timing only. */

@@ -10,7 +10,7 @@ import pytest
 
 from bundle_adjustment_solver_b200 import scenes
 from bundle_adjustment_solver_b200.solver import Summary
-from helpers import load_engine, options_pair
+from helpers import launched_kernels, load_engine, options_pair
 
 pytestmark = pytest.mark.gpu
 
@@ -30,15 +30,8 @@ def _mixed_scene():
 
 
 def _backsub_kernels(run):
-    """Names of the back-substitution kernels that run() launches (CUDA activities of torch.profiler)."""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        run()
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA}
-    return {k for k in ("k_backsub_tiles", "k_backsub_pairs") if any(k in n for n in names)}
+    """Names of the back-substitution kernels that run() launches."""
+    return launched_kernels(run, ("k_backsub_tiles", "k_backsub_pairs"))
 
 
 def _check_paths(sc, scene):

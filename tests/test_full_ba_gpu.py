@@ -7,25 +7,9 @@ import numpy as np
 import pytest
 
 from bundle_adjustment_solver_b200 import scenes
-from helpers import S_block_view, blockwise_rel_err, load_engine, load_oracle, options_pair
+from helpers import BLOCK_TOL, blockwise_rel_err, compare_blocks, load_engine, load_oracle, options_pair
 
 pytestmark = pytest.mark.gpu
-
-BLOCK_TOL = 1e-9
-
-
-def _compare_blocks(o, e, sizes, tol=BLOCK_TOL, check_S=True):
-    N = sizes["N"]
-    errs = {}
-    for name, blk in (("A", 36), ("a", 6), ("C", 9), ("b", 3), ("Cinv", 9), ("B", 18)):
-        errs[name] = blockwise_rel_err(e.dump(name), o.dump(name), blk)
-    if check_S:
-        errs["S"] = blockwise_rel_err(S_block_view(e.dump("S"), N), S_block_view(o.dump("S"), N), 36)
-        errs["rhs"] = blockwise_rel_err(e.dump("rhs"), o.dump("rhs"), 6)
-    bad = {k: v for k, v in errs.items() if not v <= tol}
-    assert not bad, f"block parity failed: {bad} (all: {errs})"
-    return errs
-
 
 @pytest.mark.parametrize("seed", [0, 1])
 @pytest.mark.parametrize("accum", [0, 1])
@@ -40,7 +24,7 @@ def test_blocks_match_oracle_c1(seed, accum, oracle_mod, engine_lib):
     assert e.sizes() == o.sizes()
     # same pair set, same order (sorted by point, pose)
     assert all(np.array_equal(x, y) for x, y in zip(e.pairs(), o.pairs()))
-    _compare_blocks(o, e, o.sizes())
+    compare_blocks(o, e, o.sizes())
     # reduced solve and back-substitution: x, y  (conditioning of S enters -> looser, stated)
     assert blockwise_rel_err(e.dump("x"), o.dump("x"), 6) < 1e-6
     assert blockwise_rel_err(e.dump("y"), o.dump("y"), 3) < 1e-6
@@ -213,7 +197,7 @@ def test_fixed_points_and_split_point(oracle_mod, engine_lib):
         oo, eo = options_pair(b_accumulate=accum)
         e.build_only(eo, 3.0, do_solve=True)
         assert e.sizes() == o.sizes()
-        _compare_blocks(o, e, o.sizes())
+        compare_blocks(o, e, o.sizes())
         assert blockwise_rel_err(e.dump("y"), o.dump("y"), 3) < 1e-6
     # and a short solve agrees
     oo, eo = options_pair(max_num_iterations=6)
@@ -341,7 +325,7 @@ def test_c3_scaled_blocks_and_iterations(oracle_mod, engine_lib):
     e.set_debug(True)
     oo, eo = options_pair()
     e.build_only(eo, 100.0, do_solve=True)
-    _compare_blocks(o, e, o.sizes())
+    compare_blocks(o, e, o.sizes())
     assert blockwise_rel_err(e.dump("x"), o.dump("x"), 6) < 1e-6
     oo, eo = options_pair(max_num_iterations=3)
     o = load_oracle(sc)
@@ -435,7 +419,7 @@ def test_tile_build_with_fixed_poses_points_and_wide_tracks(oracle_mod, engine_l
         oo, eo = options_pair(b_accumulate=accum)
         e.build_only(eo, 100.0, do_solve=True)
         assert e.sizes() == o.sizes()
-        _compare_blocks(o, e, o.sizes())
+        compare_blocks(o, e, o.sizes())
         assert blockwise_rel_err(e.dump("y"), o.dump("y"), 3) < 1e-6
 
 
@@ -548,7 +532,7 @@ def test_c4_c5_full_size_blocks_match_oracle(workload, oracle_mod, engine_lib):
     sz = o.sizes()
     assert e.sizes() == sz and sz["n_obs"] > 4_500_000
     assert all(np.array_equal(x, y) for x, y in zip(e.pairs(), o.pairs()))
-    _compare_blocks(o, e, sz, check_S=False)
+    compare_blocks(o, e, sz, check_S=False)
     assert blockwise_rel_err(e.dump("rhs"), o.dump("rhs"), 6) <= BLOCK_TOL
     assert _S_blockwise_rel_err_chunked(e.dump("S"), o.dump("S"), sz["N"]) <= BLOCK_TOL
 

@@ -391,6 +391,16 @@ __global__ void __launch_bounds__(256) k_backward_block(const double *__restrict
   }
 }
 
+// The reduced solve a plan runs.  Each path falls back to the next one when its launch fails (a partitioned solve
+// whose cooperative launch is refused runs its per-level launches instead).
+enum class SolvePath {
+  NdPersistent,   // partitioned banded, one persistent launch (ba_cholesky_nd.cuh)
+  NdLevels,       // partitioned banded, one launch per tree level
+  Banded,         // serial window kernel (ba_cholesky_banded.cuh)
+  Cluster,        // blocked Cholesky in one thread-block-cluster launch (ba_cholesky_cluster.cuh)
+  Dense,          // blocked multi-kernel Cholesky (below)
+};
+
 // Tile-level row envelope (skyline) of S: Cholesky creates no fill left of a row's first non-zero, so
 // tiles (r, c) with c < first_tile[r] stay zero and are skipped by TRSM / SYRK / the backward sweep.
 // For a dense S (every pose co-visible with every other) first_tile is all zeros and nothing is skipped.
@@ -411,21 +421,21 @@ struct CholeskyPlan {
   bool banded = false;    // banded reduced system: serial window kernel (ba_cholesky_banded.cuh) or the partition below
   NdPlan nd;              // partitioned banded solve (ba_cholesky_nd.cuh); nd.valid: preferred over the serial kernel
   NdDevice nd_dev;
+  SolvePath path = SolvePath::Dense;   // chosen once the partition's device resources are known
 };
 
-inline void cholesky_make_plan(CholeskyPlan &pl, int n, const std::vector<int> &first_pose /*per free pose: first co-visible pose*/) {
+// chol_mode: -1 auto (banded > cluster > multi-kernel), 0 forces the multi-kernel path, 1 the cluster path where the
+// plan allows it.  force_depth / force_chunk (-1: chosen by the planner) force the partition's tree depth and chunk
+// size in poses.
+inline void cholesky_make_plan(CholeskyPlan &pl, int n, const std::vector<int> &first_pose /*per free pose: first co-visible pose*/,
+                               int chol_mode, int force_depth, int force_chunk) {
   pl.n = n;
   pl.bw = 0;
   for (size_t j = 0; j < first_pose.size(); ++j) pl.bw = std::max(pl.bw, 6 * ((int)j - first_pose[j]) + 5);
   pl.bw = std::min(pl.bw, std::max(0, n - 1));
-  pl.banded = cholesky_banded_supported(n, pl.bw) && n > kBandMaxW;
+  pl.banded = cholesky_banded_supported(n, pl.bw) && n > kBandMaxW && chol_mode != 0 && chol_mode != 1;
   pl.nd = NdPlan();
-  if (pl.banded && n % 6 == 0) {
-    // BA_B200_ND_DEPTH / BA_B200_ND_CHUNK: force the tree depth / the chunk size in poses (tests)
-    const int fd = getenv("BA_B200_ND_DEPTH") ? atoi(getenv("BA_B200_ND_DEPTH")) : -1;
-    const int fc = getenv("BA_B200_ND_CHUNK") ? atoi(getenv("BA_B200_ND_CHUNK")) : -1;
-    nd_make_plan(pl.nd, n / 6, (pl.bw - 5) / 6, 128, fd, fc);
-  }
+  if (pl.banded && n % 6 == 0) nd_make_plan(pl.nd, n / 6, (pl.bw - 5) / 6, 128, force_depth, force_chunk);
   pl.T = (n + 1 + kNB - 1) / kNB;
   pl.first_tile.assign(pl.T, pl.T);
   for (size_t j = 0; j < first_pose.size(); ++j) {
@@ -468,7 +478,7 @@ inline void cholesky_make_plan(CholeskyPlan &pl, int n, const std::vector<int> &
   for (int k = 0; k < pl.T; ++k) pl.max_rows = std::max(pl.max_rows, pl.rows_ptr[k + 1] - pl.rows_ptr[k]);
   // cluster path: every panel's tile jobs fit a few rounds of a <=16-CTA cluster
   pl.cluster_size = 0;
-  if (n > 0 && n <= kClusterMaxN && pl.max_rows <= 12) {
+  if (n > 0 && n <= kClusterMaxN && pl.max_rows <= 12 && chol_mode != 0) {
     const int jobs = pl.max_rows * (pl.max_rows + 1) / 2;
     pl.cluster_size = jobs <= 1 ? 1 : jobs <= 2 ? 2 : jobs <= 4 ? 4 : jobs <= 8 ? 8 : 16;
   }
@@ -481,33 +491,41 @@ inline size_t cholesky_linv_doubles(int n) { return (size_t)((n + kNB - 1) / kNB
 
 // Enqueue factor + solve on `stream`.  Saug: (n+1)^2 doubles, ld = n+1.  x: n doubles.  zbuf: n.
 // linv: ceil(n/64) * 64*64 doubles (inverses of the diagonal blocks).
-// parts: bit 0 diag, 1 trsm, 2 syrk, 3 backward (all by default; subsets are for in-situ timing only)
+// parts: bit 0 diag, 1 trsm, 2 syrk, 3 backward (all by default: the plan's path; a subset runs those parts of the
+// multi-kernel path, for in-situ timing only).  verbose: print the plan and time the single-launch kernels.
 inline void cholesky_solve_enqueue(const CholeskyPlan &pl, double *Saug, double *x, double *zbuf, double *linv,
-                                   const LmState *st, cudaStream_t stream, long long *launches, int parts = 15) {
+                                   const LmState *st, cudaStream_t stream, long long *launches, bool verbose,
+                                   int parts = 15) {
   const int n = pl.n, ld = n + 1, n_rows = n + 1;
-  static const bool verbose = getenv("BA_B200_VERBOSE") != nullptr;
-  if (verbose) fprintf(stderr, "[ba_b200] cholesky n=%d T=%d max_rows=%d cluster_size=%d dense_fraction=%.3f bw=%d banded=%d parts=%d\n", n, pl.T, pl.max_rows, pl.cluster_size, pl.dense_fraction, pl.bw, (int)pl.banded, parts);
-  if (pl.banded && parts == 15) {
-    // BA_B200_BAND_MODE: 6 (default) partitioned, one persistent launch; 5 partitioned, one launch per level;
-    // <= 4 the serial window kernels
-    const int mode = getenv("BA_B200_BAND_MODE") ? atoi(getenv("BA_B200_BAND_MODE")) : 6;
-    if (mode >= 5 && pl.nd.valid && pl.nd_dev.tpw > 0) {
-      if (nd_enqueue(pl.nd, pl.nd_dev, Saug, x, mode, verbose ? 1 : 0, st, stream, launches)) return;
-      const cudaError_t ce = cudaGetLastError();
-      if (verbose) fprintf(stderr, "[ba_b200] partitioned banded launch failed: %s\n", cudaGetErrorString(ce));
+  if (verbose) fprintf(stderr, "[ba_b200] cholesky n=%d T=%d max_rows=%d cluster_size=%d dense_fraction=%.3f bw=%d banded=%d path=%d parts=%d\n", n, pl.T, pl.max_rows, pl.cluster_size, pl.dense_fraction, pl.bw, (int)pl.banded, (int)pl.path, parts);
+  if (parts == 15) {
+    switch (pl.path) {
+      case SolvePath::NdPersistent:
+      case SolvePath::NdLevels: {
+        if (nd_enqueue(pl.nd, pl.nd_dev, Saug, x, pl.path == SolvePath::NdPersistent, verbose ? 1 : 0, st, stream, launches)) return;
+        const cudaError_t ce = cudaGetLastError();
+        if (verbose) fprintf(stderr, "[ba_b200] partitioned banded launch failed: %s\n", cudaGetErrorString(ce));
+      }
+        [[fallthrough]];
+      case SolvePath::Banded:
+        if (cholesky_banded_enqueue(Saug, n, pl.bw, x, linv, verbose ? 1 : 0, st, stream)) {
+          if (launches) *launches += 1;
+          return;
+        }
+        [[fallthrough]];
+      case SolvePath::Cluster:
+        if (pl.cluster_size > 0) {
+          if (cholesky_cluster_enqueue(Saug, n, pl.d_rows_ptr, pl.d_rows, pl.d_first_tile, x, verbose ? 1 : 0, st, stream, pl.cluster_size)) {
+            if (launches) *launches += 1;
+            return;
+          }
+          const cudaError_t ce = cudaGetLastError();  // cluster launch unavailable: fall through to the multi-kernel path
+          if (verbose) fprintf(stderr, "[ba_b200] cluster launch failed: %s\n", cudaGetErrorString(ce));
+        }
+        break;
+      case SolvePath::Dense:
+        break;
     }
-    if (cholesky_banded_enqueue(Saug, n, pl.bw, x, linv, st, stream)) {
-      if (launches) *launches += 1;
-      return;
-    }
-  }
-  if (pl.cluster_size > 0 && parts == 15) {
-    if (cholesky_cluster_enqueue(Saug, n, pl.d_rows_ptr, pl.d_rows, pl.d_first_tile, x, st, stream, pl.cluster_size)) {
-      if (launches) *launches += 1;
-      return;
-    }
-    const cudaError_t ce = cudaGetLastError();  // cluster launch unavailable: fall through to the multi-kernel path
-    if (verbose) fprintf(stderr, "[ba_b200] cluster launch failed: %s\n", cudaGetErrorString(ce));
   }
   static PerDeviceOnce once;
   if (once.first()) cudaFuncSetAttribute(k_chol_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCholDiagSmem);

@@ -522,9 +522,9 @@ inline bool launch_band4(double *Saug, int n, int bw, double *x, double *linv, i
 
 inline bool cholesky_banded_supported(int n, int bw) { return n > 0 && bw + 8 <= kBandMaxW; }
 
-inline bool cholesky_banded_enqueue(double *Saug, int n, int bw, double *x, double *linv, const LmState *st,
+// timing: the kernel records its phase times in g_band_dbg
+inline bool cholesky_banded_enqueue(double *Saug, int n, int bw, double *x, double *linv, int timing, const LmState *st,
                                     cudaStream_t stream) {
-  static const int timing = getenv("BA_B200_VERBOSE") != nullptr;
   // DMMA block steps, window in shared memory (needs W >= bw + 16; cholesky_banded_supported guarantees bw <= 104)
   if (bw + 16 <= 56) return launch_band4<56>(Saug, n, bw, x, linv, timing, st, stream);
   if (bw + 16 <= 88) return launch_band4<88>(Saug, n, bw, x, linv, timing, st, stream);

@@ -461,10 +461,10 @@ k_chol_cluster(double *A, int n, const int *__restrict__ rows_ptr, const int *__
   if (timing && t == 0) { for (int i = 0; i < 6; ++i) g_cl_dbg[i] = tacc[i]; g_cl_dbg[6] = gtime() - tb0; }
 }
 
+// timing: the kernel records its phase times in g_cl_dbg
 inline bool cholesky_cluster_enqueue(double *Saug, int n, const int *d_rows_ptr, const int *d_rows,
-                                     const int *d_first_tile, double *x, const LmState *st, cudaStream_t stream,
-                                     int cluster_size) {
-  static const int timing = getenv("BA_B200_VERBOSE") != nullptr;
+                                     const int *d_first_tile, double *x, int timing, const LmState *st,
+                                     cudaStream_t stream, int cluster_size) {
   static PerDeviceOnce once;
   if (once.first()) {
     cudaFuncSetAttribute(k_chol_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem);

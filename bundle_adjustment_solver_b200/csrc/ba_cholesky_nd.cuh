@@ -824,7 +824,7 @@ inline int nd_tpw_for(int BT) {
 }
 
 template <int TPW, int NC>
-inline bool nd_enqueue_t(const NdPlan &pl, const NdDevice &dv, const double *Saug, double *x, int mode, int timing,
+inline bool nd_enqueue_t(const NdPlan &pl, const NdDevice &dv, const double *Saug, double *x, bool persistent, int timing,
                          const LmState *st, cudaStream_t stream, long long *launches) {
   static PerDeviceOnce once;
   if (once.first()) {
@@ -832,7 +832,7 @@ inline bool nd_enqueue_t(const NdPlan &pl, const NdDevice &dv, const double *Sau
     cudaFuncSetAttribute(k_nd_persistent<TPW, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kNdSmemLimit);
     cudaFuncSetAttribute(k_nd_backward_level, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kNdSmemLimit);
   }
-  if (mode == 6) {
+  if (persistent) {
     cudaMemsetAsync(dv.cta_args.flags, 0, (size_t)(dv.cta_args.abort_idx + 1) * sizeof(int), stream);
     NdArgs a = dv.cta_args;
     a.S = Saug; a.x = x;
@@ -871,22 +871,22 @@ inline bool nd_enqueue_t(const NdPlan &pl, const NdDevice &dv, const double *Sau
   return cudaGetLastError() == cudaSuccess;
 }
 
-// mode 5: one launch per level; mode 6: one persistent launch
-inline bool nd_enqueue(const NdPlan &pl, const NdDevice &dv, const double *Saug, double *x, int mode, int timing,
+// persistent: one cooperative launch over all fronts (the per-level launches if it is refused); else one launch per level
+inline bool nd_enqueue(const NdPlan &pl, const NdDevice &dv, const double *Saug, double *x, bool persistent, int timing,
                        const LmState *st, cudaStream_t stream, long long *launches) {
   if (nd_cons_for(pl.max_BT) == 9) {
     switch (dv.tpw) {
-      case 4: return nd_enqueue_t<4, 9>(pl, dv, Saug, x, mode, timing, st, stream, launches);
-      case 8: return nd_enqueue_t<8, 9>(pl, dv, Saug, x, mode, timing, st, stream, launches);
+      case 4: return nd_enqueue_t<4, 9>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
+      case 8: return nd_enqueue_t<8, 9>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
       default: return false;
     }
   }
   switch (dv.tpw) {
-    case 8: return nd_enqueue_t<8, 11>(pl, dv, Saug, x, mode, timing, st, stream, launches);
-    case 12: return nd_enqueue_t<12, 11>(pl, dv, Saug, x, mode, timing, st, stream, launches);
-    case 14: return nd_enqueue_t<14, 11>(pl, dv, Saug, x, mode, timing, st, stream, launches);
-    case 19: return nd_enqueue_t<19, 11>(pl, dv, Saug, x, mode, timing, st, stream, launches);
-    case 24: return nd_enqueue_t<24, 11>(pl, dv, Saug, x, mode, timing, st, stream, launches);
+    case 8: return nd_enqueue_t<8, 11>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
+    case 12: return nd_enqueue_t<12, 11>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
+    case 14: return nd_enqueue_t<14, 11>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
+    case 19: return nd_enqueue_t<19, 11>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
+    case 24: return nd_enqueue_t<24, 11>(pl, dv, Saug, x, persistent, timing, st, stream, launches);
     default: return false;
   }
 }

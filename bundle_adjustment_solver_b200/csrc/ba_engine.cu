@@ -30,6 +30,8 @@
 // Multi-GPU: landmarks sharded; the band of [S | rhs] is exchanged through peer memory (one-shot pushes + epoch flags,
 // summed in rank order; NCCL all-reduce as the fallback), the five LM scalars by k_exchange_decide.
 // There is no CPU fallback: every entry point that computes requires a CUDA device.
+// The A/B and diagnostic switches (BA_B200_*, DESIGN §4.0) are read from the environment once per solver, by ba_create
+// (read_switches); the reduced solve a plan runs is chosen once, in upload_cholesky_plan (CholeskyPlan::path).
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 #include <nccl.h>
@@ -358,7 +360,7 @@ __device__ __forceinline__ void damp_invert(const double *Craw, double lambda, d
 #include "ba_build_tiles.cuh"
 
 __global__ void __launch_bounds__(128)
-k_schur_pairs_list(int n_list, const int *__restrict__ list /*pair indices p1, or null = identity*/,
+k_schur_pairs_list(int n_list, const int *__restrict__ list /*pair indices p1*/,
                    const int *__restrict__ pair_pose, const int *__restrict__ pair_point,
                    const int *__restrict__ pair_end /*index one past the last pair of this pair's point*/,
                    const double *__restrict__ Bsoa, size_t Pp, const double *__restrict__ ptblk, size_t Mp,
@@ -366,7 +368,7 @@ k_schur_pairs_list(int n_list, const int *__restrict__ list /*pair indices p1, o
   if (st->done) return;
   const int li = blockIdx.x * blockDim.x + threadIdx.x;
   if (li >= n_list) return;
-  const int p1 = list ? list[li] : li;
+  const int p1 = list[li];
   const int pt = pair_point[p1];
   const int j1 = pair_pose[p1];
   double B1[18];
@@ -517,14 +519,6 @@ __device__ __forceinline__ void backsub_points_body(int blk, int M_total, const 
     partials[(size_t)blk * 2 + 1] = acc[1];
   }
 }
-__global__ void __launch_bounds__(kThreads)
-k_backsub_points(int M_total, const int *__restrict__ point_has_pairs, const uint8_t *__restrict__ point_free,
-                 const double *__restrict__ ptblk, size_t Mp, const double *__restrict__ Btx,
-                 double *__restrict__ y /*[M_total][3]*/, Params prm, ParamsW prw,
-                 double *__restrict__ partials /*[grid][2]*/, int method, const LmState *__restrict__ st) {
-  if (st->done) return;
-  backsub_points_body(blockIdx.x, M_total, point_has_pairs, point_free, ptblk, Mp, Btx, y, prm, prw, partials, method, st);
-}
 
 // SolveByGradientDescent, pose side (full_bundle_adjustment_solver_refactor.cpp:1274-1276): x_j = a_j clipped to
 // max_pose_step = 0.001
@@ -589,13 +583,6 @@ __device__ __forceinline__ void update_poses_body(int blk, int N_total, const in
     partials[(size_t)blk * 2 + 1] = acc[1];
   }
 }
-__global__ void __launch_bounds__(kThreads)
-k_update_poses(int N_total, const int *__restrict__ pose_opt, const double *__restrict__ x,
-               const double *__restrict__ A, const double *__restrict__ a, Params prm, ParamsW prw,
-               double *__restrict__ partials /*[grid][2]*/, const LmState *__restrict__ st) {
-  if (st->done) return;
-  update_poses_body(blockIdx.x, N_total, pose_opt, x, A, a, prm, prw, partials, st);
-}
 // Back-substitution of the landmarks and the pose update in ONE launch: the two are independent (both only need x), the
 // pose update is a single latency-bound CTA (9 us on C3) that now runs beside the landmark CTAs
 __global__ void __launch_bounds__(kThreads)
@@ -623,6 +610,9 @@ k_backsub_points_update_poses(int point_blocks, int M_total, const int *__restri
 // ---------------------------------------------------------------------------
 constexpr int kDenseLm = 10;   // landmarks per pass: 30 of the kKH = 32 operand rows
 constexpr int kDenseMaxPoses = 128;   // free poses (a landmark has at most one pair per pose): 6 N + 1 <= 769
+// The by-point Schur products of a reduced system with N free poses go through k_schur_dense_gemm (ba_finalize sends
+// every landmark there when most of them do not fit a window) rather than k_schur_pairs_list
+inline bool dense_schur_fits(int N) { return N <= kDenseMaxPoses; }
 __global__ void __launch_bounds__(256)
 k_schur_dense_gemm(const int2 *__restrict__ groups /*pair range [x, y) of one landmark*/, int n_groups, int split_k,
                    const int *__restrict__ pair_pose, const int *__restrict__ pair_point,
@@ -1299,6 +1289,7 @@ NcclApi g_nccl;
 struct SharedComm {
   ncclComm_t comm = nullptr;
   int rank = 0, n_ranks = 1, device = 0;
+  bool verbose = false;   // BA_B200_VERBOSE of the solver that created the communicator
   PeerExch *local = nullptr;
   PeerExch *peer[kMaxRanks] = {};
   unsigned *d_epoch = nullptr;
@@ -1565,10 +1556,41 @@ struct DevBuf {
   }
 };
 
+// A/B and diagnostic switches (DESIGN §4.0).  read_switches() holds the engine's only getenv calls; ba_create takes
+// one snapshot per solver, so a switch applies to the solvers created after it is set and never changes under a
+// solver that exists.  The defaults are the shipped path.
+struct EngineSwitches {
+  int band_mode = 6;             // BA_B200_BAND_MODE: 6 partitioned, one persistent launch; 5 partitioned, one launch
+                                 // per level; <= 4 the serial window kernel
+  int chol_mode = -1;            // BA_B200_CHOL_MODE: -1 auto, 0 dense multi-kernel, 1 cluster (cholesky_make_plan)
+  int nd_depth = -1, nd_chunk = -1;   // BA_B200_ND_DEPTH / BA_B200_ND_CHUNK: force the partition (tests)
+  bool reduce_stores = true;     // BA_B200_REDUCE_STORES=0: clear of S + k_pose_diag + adding k_tile_reduce instead
+                                 // of the storing reduce on banded plans (the two forms are bit-identical)
+  size_t band_clear_min = (size_t)64 << 20;   // BA_B200_BAND_CLEAR_MIN_MB: dense S above this clears only its band
+  int band_xchg = 1;             // BA_B200_BAND_XCHG: 1 one-shot, 2 two-shot band exchange over peer memory
+  bool no_peer_exchange = false; // BA_B200_NO_PEER_EXCHANGE: NCCL for the scalars and the band (ba_comm_init)
+  bool verbose = false;          // BA_B200_VERBOSE: finalisation laps, the solve plan, in-kernel solve timing
+};
+
+static EngineSwitches read_switches() {
+  EngineSwitches w;
+  if (const char *e = getenv("BA_B200_BAND_MODE")) w.band_mode = atoi(e);
+  if (const char *e = getenv("BA_B200_CHOL_MODE")) w.chol_mode = atoi(e);
+  if (const char *e = getenv("BA_B200_ND_DEPTH")) w.nd_depth = atoi(e);
+  if (const char *e = getenv("BA_B200_ND_CHUNK")) w.nd_chunk = atoi(e);
+  if (const char *e = getenv("BA_B200_REDUCE_STORES")) w.reduce_stores = atoi(e) != 0;
+  if (const char *e = getenv("BA_B200_BAND_CLEAR_MIN_MB")) w.band_clear_min = (size_t)atoi(e) << 20;
+  if (const char *e = getenv("BA_B200_BAND_XCHG")) w.band_xchg = atoi(e) ? atoi(e) : 1;
+  w.no_peer_exchange = getenv("BA_B200_NO_PEER_EXCHANGE") != nullptr;
+  w.verbose = getenv("BA_B200_VERBOSE") != nullptr;
+  return w;
+}
+
 }  // namespace
 
 struct ba_solver {
   int device = 0;
+  EngineSwitches sw;   // read once by ba_create
   std::string err;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -1594,7 +1616,7 @@ struct ba_solver {
   // device problem
   DevBuf<double> d_cams, d_poses[2], d_points[2];
   DevBuf<double2> d_obs_uv, d_uvA;
-  DevBuf<int> d_obs_pose, d_obs_point, d_obs_camflags, d_obs_pair;
+  DevBuf<int> d_obs_pose, d_obs_point, d_obs_camflags;
   DevBuf<int> d_pointA, d_camA, d_poseidA;
   DevBuf<int2> d_pair_obs;
   DevBuf<ChunkA> d_chunksA;
@@ -1624,14 +1646,12 @@ struct ba_solver {
   DevBuf<uint8_t> d_point_fb;
   int n_chunks_fb = 0;
   int n_schur_chunks = 0, n_fallback_pairs = 0;
-  int schur_mode = 1;  // 1 = register-tiled windows + fallback, 0 = direct reds only
   CholeskyPlan chol;
   DevBuf<int> d_chol_rows, d_chol_first, d_chol_rows_ptr;
   DevBuf<NdNode> d_nd_nodes;                       // partitioned banded solve (ba_cholesky_nd.cuh)
   DevBuf<int> d_nd_level_nodes, d_nd_cta_nodes, d_nd_cta_ptr, d_nd_flags, d_nd_helpers;
   DevBuf<double> d_nd_L, d_nd_U;
   DevBuf<double> d_band;   // multi-GPU, banded S: band rows + rhs packed for the all-reduce
-  int chol_mode = -1;  // -1 auto, 0 multi-kernel, 1 cluster
   bool S_clean_outside_band = false;   // Saug was fully cleared since it was allocated / the plan changed
   // blocks
   size_t Mp = 0, Pp = 0;
@@ -1643,7 +1663,6 @@ struct ba_solver {
   DevBuf<double> d_Au[2];           // speculative pose side: undamped A (21) / a (6) sums per free pose and parameter buffer
   DevBuf<double> d_cost_partialsA;  // cost partials of k_cost_linearize_by_pose, one per pose-order chunk
   int n_chunksA_all = 0;            // free-pose chunks (the first n_chunksA) + fixed-pose chunks
-  bool rs_now = false, graph_rs = false;       // storing form of k_tile_reduce allowed (BA_B200_REDUCE_STORES)
   DevBuf<ba_iter_info> d_infos;
   int point_grid = 0, pose_grid = 0;
   LmState *h_state = nullptr;  // pinned
@@ -1699,6 +1718,7 @@ int ba_create(ba_solver **out, int device) {
   if (device < 0 || device >= count) return BA_ERR_INVALID;
   ba_solver *s = new ba_solver();
   s->device = device;
+  s->sw = read_switches();
   *out = s;
   return BA_OK;
 }
@@ -1708,7 +1728,7 @@ static void free_device(ba_solver *s) {
   s->d_cams.release();
   for (int i = 0; i < 2; ++i) { s->d_poses[i].release(); s->d_points[i].release(); }
   s->d_obs_uv.release(); s->d_uvA.release(); s->d_obs_pose.release(); s->d_obs_point.release();
-  s->d_obs_camflags.release(); s->d_obs_pair.release(); s->d_pointA.release(); s->d_camA.release();
+  s->d_obs_camflags.release(); s->d_pointA.release(); s->d_camA.release();
   s->d_poseidA.release(); s->d_pair_obs.release(); s->d_chunksA.release();
   s->d_pose_chunk_ptr.release(); s->d_pose_opt.release(); s->d_pair_pose.release(); s->d_pair_point.release();
   s->d_pair_end.release(); s->d_point_has_pairs.release(); s->d_point_free.release();
@@ -1881,10 +1901,6 @@ static int upload_cholesky_plan(ba_solver *s) {
   s->chol.d_rows = s->d_chol_rows.p;
   s->chol.d_first_tile = s->d_chol_first.p;
   s->chol.d_rows_ptr = s->d_chol_rows_ptr.p;
-  if (const char *e = getenv("BA_B200_CHOL_MODE")) s->chol_mode = atoi(e);
-  // BA_B200_CHOL_MODE: -1 auto (banded > cluster > multi-kernel), 0 multi-kernel, 1 cluster, 2 banded
-  if (s->chol_mode == 0) { s->chol.cluster_size = 0; s->chol.banded = false; }
-  if (s->chol_mode == 1) s->chol.banded = false;
   // partitioned banded solve: node table, level / CTA lists, factor and contribution-block workspaces
   NdPlan &nd = s->chol.nd;
   s->chol.nd_dev = NdDevice();
@@ -1922,6 +1938,14 @@ static int upload_cholesky_plan(ba_solver *s) {
       dv.cta_args.use_helpers = nd.n_helpers > 0;
     }
   }
+  // the reduced solve: BA_B200_BAND_MODE picks between the partition (if it is valid) and the serial window kernel
+  CholeskyPlan &pl = s->chol;
+  if (pl.banded && nd.valid && s->sw.band_mode >= 5)
+    pl.path = s->sw.band_mode == 6 ? SolvePath::NdPersistent : SolvePath::NdLevels;
+  else if (pl.banded)
+    pl.path = SolvePath::Banded;
+  else
+    pl.path = pl.cluster_size > 0 ? SolvePath::Cluster : SolvePath::Dense;
   return BA_OK;
 }
 
@@ -1940,7 +1964,7 @@ static int agree_on_envelope(ba_solver *s) {
   CUDA_TRY(cudaMemcpyAsync(s->h_first_pose.data(), d_fp.p, (size_t)s->N * sizeof(int), cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
   d_fp.release();
-  cholesky_make_plan(s->chol, 6 * s->N, s->h_first_pose);
+  cholesky_make_plan(s->chol, 6 * s->N, s->h_first_pose, s->sw.chol_mode, s->sw.nd_depth, s->sw.nd_chunk);
   if (int rc = upload_cholesky_plan(s)) return rc;
   CUDA_TRY(cudaStreamSynchronize(st));
   // band exchange through peer memory (same count on every rank: the plan is global now)
@@ -1967,7 +1991,7 @@ int ba_finalize(ba_solver *s) {
   CUDA_TRY(cudaSetDevice(s->device));
   if (int rc = ensure_stream(s)) return rc;
   destroy_graph(s);
-  static const bool verbose = getenv("BA_B200_VERBOSE") != nullptr;
+  const bool verbose = s->sw.verbose;
   auto tp0 = std::chrono::high_resolution_clock::now();
   auto lap = [&](const char *what) {
     if (!verbose) return;
@@ -2097,12 +2121,11 @@ int ba_finalize(ba_solver *s) {
       for (int p = grp_start[g]; p < grp_start[g + 1]; ++p) pair_end[p] = grp_start[g + 1];
   });
   lap("point order, pairs");
-  // The point-ordered observation arrays (36 of the ~60 MB this function uploads) are final: a helper thread sends
-  // them while this thread builds the tile / chunk structures.  +1 sentinels so that obs_point[k+1] / obs_pair[k+1]
-  // reads of the kernels stay in bounds (the host code below never reads past n).
+  // The point-ordered observation arrays (most of what this function uploads) are final: a helper thread sends them
+  // while this thread builds the tile / chunk structures.  +1 sentinel so that obs_point[k+1] reads of the kernels
+  // stay in bounds (the host code below never reads past n).
   cudaStream_t st = s->stream;
   o_point.push_back(-1);
-  o_pair.push_back(-2);
   cudaError_t early_err = cudaSuccess;
   std::thread early_upload([&]() {
     cudaSetDevice(s->device);
@@ -2110,7 +2133,6 @@ int ba_finalize(ba_solver *s) {
     cudaError_t e = s->d_obs_uv.upload(uv, st);
     if (e == cudaSuccess) e = s->d_obs_pose.upload(o_pose, st);
     if (e == cudaSuccess) e = s->d_obs_point.upload(o_point, st);
-    if (e == cudaSuccess) e = s->d_obs_pair.upload(o_pair, st);
     if (e == cudaSuccess) e = s->d_pair_obs.upload(pair_obs, st);
     if (e == cudaSuccess) e = s->d_pair_end.upload(pair_end, st);
     early_err = e;
@@ -2136,7 +2158,7 @@ int ba_finalize(ba_solver *s) {
         int prev = -1;
         for (long long q = pt_q0[c.point]; q < pt_q0[c.point + 1]; ++q)
           if (o_pose[q] != prev) { ++c.n_inc; prev = o_pose[q]; }
-        c.ok = (s->schur_mode == 1 && c.jmax - c.jmin + 1 <= kTileW && c.n_inc <= kTileMaxInc) ? 1 : 0;
+        c.ok = (c.jmax - c.jmin + 1 <= kTileW && c.n_inc <= kTileMaxInc) ? 1 : 0;
         all[g] = c;
       }
     });
@@ -2158,7 +2180,7 @@ int ba_finalize(ba_solver *s) {
     // Small reduced system whose landmarks mostly do NOT fit a window (dense co-visibility, test_ba.cpp): the
     // by-point path ends in one dense tensor-core GEMM (k_schur_dense_gemm) that takes the few window landmarks
     // along for free, while a second, nearly empty persistent tile launch would cost its fixed 30 us
-    if (6 * s->N + 1 <= 6 * kDenseMaxPoses + 1 && 2 * (long long)cands.size() < n_grp) {
+    if (dense_schur_fits(s->N) && 2 * (long long)cands.size() < n_grp) {
       for (const Cand &c : cands)
         for (int q = c.p0; q < c.p1; ++q) fallback_pairs.push_back(q);
       cands.clear();
@@ -2283,7 +2305,7 @@ int ba_finalize(ba_solver *s) {
       const int jmin = s->h_pair_pose[grp_start[g]];
       for (int q = grp_start[g]; q < grp_start[g + 1]; ++q) first_pose[s->h_pair_pose[q]] = std::min(first_pose[s->h_pair_pose[q]], jmin);
     }
-    cholesky_make_plan(s->chol, 6 * s->N, first_pose);
+    cholesky_make_plan(s->chol, 6 * s->N, first_pose, s->sw.chol_mode, s->sw.nd_depth, s->sw.nd_chunk);
   }
   s->n_schur_chunks = (int)schur_chunks.size();
   s->n_fallback_pairs = (int)fallback_pairs.size();
@@ -2409,8 +2431,7 @@ int ba_finalize(ba_solver *s) {
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device);
     // measured on B200 (C3: 4 / 8 / 13 observations per thread -> 55 / 47 / 56 us; C4: 4 / 8 / 16 -> 0.46 / 0.41 /
     // 0.39 ms): about three CTAs per slot, between 4 and 16 observations per thread
-    int per_thread = (int)std::min<long long>(16, std::max<long long>(4, nA / ((long long)3 * sms * kThreads)));
-    if (const char *e = getenv("BA_B200_POSE_CHUNK_OBS")) per_thread = std::max(1, atoi(e));   // A/B runs
+    const int per_thread = (int)std::min<long long>(16, std::max<long long>(4, nA / ((long long)3 * sms * kThreads)));
     const long long chunk_cap = (long long)kThreads * per_thread;
     for (int ps = 0; ps < Nt; ++ps) {
       const int j = s->h_pose_opt[ps];
@@ -2627,14 +2648,6 @@ namespace {
 
 struct Phase { enum { Lin = 0, Schur, Solve, Backsub, Update, End, Count }; };
 
-// BA_B200_REDUCE_STORES=0: clear of S + k_pose_diag + adding k_tile_reduce instead of the storing reduce on banded
-// plans (A/B runs; the two forms are bit-identical).  Read by every entry point that builds, so that one process can
-// run both forms; the captured graph is keyed on it.
-static void read_reduce_stores(ba_solver *s) {
-  const char *e = getenv("BA_B200_REDUCE_STORES");
-  s->rs_now = !(e && atoi(e) == 0);
-}
-
 static DecideArgs make_decide_args(ba_solver *s, const ba_options *opt) {
   DecideArgs g;
   g.cost_partials = s->d_cost_partialsA.p; g.n_cost = s->n_chunksA_all;
@@ -2666,6 +2679,13 @@ static int ensure_S_clean(ba_solver *s) {
   return BA_OK;
 }
 
+// Large banded reduced systems (C4: 1.15 GB dense) clear only the band of S per iteration: everything outside it stays
+// zero once ensure_S_clean has cleared it.  A small one is cleared faster by one linear memset.
+static bool clears_band_only(const ba_solver *s) {
+  const size_t ld = (size_t)s->chol.n + 1;
+  return s->chol.banded && ld * ld * sizeof(double) > s->sw.band_clear_min;
+}
+
 // Enqueue the build (K1..K4) on the stream.  ev: optional events at phase boundaries.
 static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
   cudaStream_t st = s->stream;
@@ -2674,18 +2694,15 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
   const LmState *dst = s->d_state.p;
   const int ld = 6 * s->N + 1;
   if (ev) cudaEventRecord(ev[Phase::Lin], st);
-  // BA_B200_BAND_CLEAR_MIN_MB: size of the dense buffer above which only the band is cleared (tests force 0)
-  static const size_t band_clear_min = (size_t)(getenv("BA_B200_BAND_CLEAR_MIN_MB") ? atoi(getenv("BA_B200_BAND_CLEAR_MIN_MB")) : 64) << 20;
   // On a banded plan k_tile_reduce WRITES every band entry and rhs entry of S (damped pose-side sums + windows) and
   // the rows of A / a, so nothing is cleared here and k_pose_diag is not launched (BA_B200_REDUCE_STORES=0: clear +
   // k_pose_diag + adding reduce)
-  const bool reduce_stores = s->rs_now && s->N > 0 && s->n_schur_chunks > 0 && s->chol.banded &&
+  const bool reduce_stores = s->sw.reduce_stores && s->N > 0 && s->n_schur_chunks > 0 && s->chol.banded &&
                              s->S_clean_outside_band && std::max(s->stage_span, s->chol.bw) + 2 <= 2 * 96;
   if (reduce_stores) {
     // nothing to clear
-  } else if (s->chol.banded && s->S_clean_outside_band && (size_t)ld * ld * sizeof(double) > band_clear_min) {
-    // large banded reduced system (C4: 1.15 GB dense; a small one is cleared faster by one linear memset): everything outside the band (and the rhs column) stays zero once cleared -- the
-    // build, the factorisation and the exchange only touch row r's columns r .. r + bw and the last column
+  } else if (clears_band_only(s) && s->S_clean_outside_band) {
+    // the build, the factorisation and the exchange only touch row r's columns r .. r + bw and the last column
     const int n = 6 * s->N;
     const long long total = (long long)n * (s->chol.bw + 2);
     k_clear_band<<<(int)std::min<long long>(148 * 8, (total + 255) / 256), 256, 0, st>>>(s->d_Saug.p, n, ld, s->chol.bw, dst);
@@ -2758,8 +2775,7 @@ static int enqueue_build(ba_solver *s, const ba_options *opt, cudaEvent_t *ev) {
       s->launches++;
     }
   }
-  static const int dense_max = getenv("BA_B200_DENSE_SCHUR_MAX") ? atoi(getenv("BA_B200_DENSE_SCHUR_MAX")) : 6 * kDenseMaxPoses + 1;
-  if (s->n_fallback_pairs > 0 && ld <= dense_max) {
+  if (s->n_fallback_pairs > 0 && dense_schur_fits(s->N)) {
     // small reduced system (dense co-visibility): the products as a tensor-core GEMM over 64 x 64 tiles
     const int nT = (ld + 63) / 64, tile_pairs = nT * (nT + 1) / 2;
     const int split_k = std::max(1, std::min((s->n_fb_groups + kDenseLm - 1) / kDenseLm, (2 * 148 + tile_pairs - 1) / tile_pairs));
@@ -2786,9 +2802,7 @@ static int enqueue_allreduce_S(ba_solver *s) {
     // BA_B200_BAND_XCHG: 1 (default) one-shot pushes, 2 two-shot (reduce-scatter + all-gather).  Measured on 8 B200:
     // C4 (3.5 MB band) 0.507 vs 0.502 ms per iteration, weak C3 (0.7 MB) 0.487 vs 0.507 ms; on 2 B200 the two-shot form
     // is 0.1 ms slower on C4 -- the exchange is bound by its hand-overs, not by NVLink bytes, so fewer hand-overs win
-    static const int xchg_env = getenv("BA_B200_BAND_XCHG") ? atoi(getenv("BA_B200_BAND_XCHG")) : 0;
-    const int xchg = xchg_env ? xchg_env : 1;
-    if (xchg == 1) {
+    if (s->sw.band_xchg == 1) {
       k_band_push1<<<grid, 128, 0, s->stream>>>(s->d_Saug.p, n, (int)ld, s->chol.bw, s->band_peers, s->d_state.p);
       k_band_pull1<<<grid, 128, 0, s->stream>>>(s->d_Saug.p, n, (int)ld, s->chol.bw, s->band_peers, s->d_state.p);
       s->launches += 2;
@@ -2837,7 +2851,7 @@ static int enqueue_solve_backsub(ba_solver *s, const ba_options *opt, cudaEvent_
   if (gd) {
     if (s->N > 0) { k_gd_poses<<<(s->N + 127) / 128, 128, 0, st>>>(s->N, s->d_a.p, s->d_x.p, dst); s->launches++; }
   } else if (n > 0) {
-    cholesky_solve_enqueue(s->chol, s->d_Saug.p, s->d_x.p, s->d_z.p, s->d_linv.p, dst, st, &s->launches);
+    cholesky_solve_enqueue(s->chol, s->d_Saug.p, s->d_x.p, s->d_z.p, s->d_linv.p, dst, st, &s->launches, s->sw.verbose);
   }
   if (ev) cudaEventRecord(ev[Phase::Backsub], st);
   // sum_j B^T x_j of every landmark with pairs: plain stores, except the pieces of a split by-point landmark (reds;
@@ -2972,7 +2986,6 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
   s->launches = 0;
   CUDA_TRY(s->d_infos.alloc(std::max(1, max_it)));
   if (int rc = ensure_S_clean(s)) return rc;
-  read_reduce_stores(s);
   // --- initial cost (:707), the pose-side sums of the initial parameters, and the state
   if (int rc = enqueue_current_cost(s, &opt)) return rc;
   k_init_state<<<1, 1, 0, st>>>(s->d_state.p, s->d_scal.p, (double)opt.initial_lambda);
@@ -3004,7 +3017,7 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
   if (use_graph && max_it > 0) {
     ba_options key = opt;
     key.check_every = 0;
-    if (!s->graph_exec || std::memcmp(&s->graph_opt, &key, sizeof(key)) != 0 || s->graph_rs != s->rs_now) {
+    if (!s->graph_exec || std::memcmp(&s->graph_opt, &key, sizeof(key)) != 0) {
       destroy_graph(s);
       cudaGraph_t graph;
       const long long l0 = s->launches;
@@ -3018,7 +3031,6 @@ int ba_solve(ba_solver *s, const ba_options *opt_in, ba_iter_info *infos, int ca
       CUDA_TRY(cudaGraphInstantiate(&s->graph_exec, graph, 0));
       cudaGraphDestroy(graph);
       s->graph_opt = key;
-      s->graph_rs = s->rs_now;
     }
   }
   std::vector<cudaEvent_t> &evp = s->ev;
@@ -3109,7 +3121,6 @@ int ba_build_only(ba_solver *s, const ba_options *opt_in, double lambda, int do_
     CUDA_TRY(s->d_Bsoa.alloc(std::max<size_t>(1, 18 * s->Pp)));
   }
   if (int rc = ensure_S_clean(s)) return rc;
-  read_reduce_stores(s);
   // the pose-side sums at the accepted parameters (Au[cur]), then the build of an iteration
   DecideArgs g = make_decide_args(s, &opt);
   launch_cost_linearize(s, &opt, 0, /*decide_here*/0, /*ignore_done*/1, g);
@@ -3247,7 +3258,8 @@ int ba_debug_time_solve(ba_solver *s, int parts, int reps, float *ms_per_rep) {
   cudaGraph_t graph;
   cudaGraphExec_t exec;
   CUDA_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
-  cholesky_solve_enqueue(s->chol, s->d_Saug.p, s->d_x.p, s->d_z.p, s->d_linv.p, s->d_state.p, st, nullptr, parts);
+  cholesky_solve_enqueue(s->chol, s->d_Saug.p, s->d_x.p, s->d_z.p, s->d_linv.p, s->d_state.p, st, nullptr, s->sw.verbose,
+                         parts);
   CUDA_TRY(cudaStreamEndCapture(st, &graph));
   CUDA_TRY(cudaGraphInstantiate(&exec, graph, 0));
   cudaEvent_t e0, e1;
@@ -3260,10 +3272,11 @@ int ba_debug_time_solve(ba_solver *s, int parts, int reps, float *ms_per_rep) {
   float ms = 0.f;
   cudaEventElapsedTime(&ms, e0, e1);
   *ms_per_rep = ms / reps;
-  if (getenv("BA_B200_VERBOSE")) {
+  const SolvePath path = s->chol.path;
+  if (s->sw.verbose) {
     unsigned long long dbg[8];
     cudaMemcpyFromSymbol(dbg, g_cl_dbg, sizeof(dbg));
-    if (s->chol.banded && s->chol.nd.valid) {
+    if (path == SolvePath::NdPersistent || path == SolvePath::NdLevels) {
       unsigned long long d3[16];
       cudaMemcpyFromSymbol(d3, g_nd_dbg, 16 * sizeof(unsigned long long));
       const double r = 1.0 / (3.0 + reps);   // accumulated over warm-up + timed replays
@@ -3274,7 +3287,7 @@ int ba_debug_time_solve(ba_solver *s, int parts, int reps, float *ms_per_rep) {
               (double)d3[13] * r, (double)d3[14] * r, (double)d3[11] * r, (double)d3[12] * r, (double)d3[8] * r, (double)d3[15] * r);
       unsigned long long z[16] = {0};
       cudaMemcpyToSymbol(g_nd_dbg, z, sizeof(z));
-    } else if (s->chol.banded) {
+    } else if (path == SolvePath::Banded) {
       unsigned long long d2[16];
       cudaMemcpyFromSymbol(d2, g_band_dbg, 16 * sizeof(unsigned long long));
       fprintf(stderr, "[ba_b200] banded ns: factor %llu backward %llu (n=%d bw=%d) | cycles: producer wait %llu work %llu | consumer0 loads %llu waitL %llu priority %llu bulk %llu endbar %llu\n",
@@ -3307,20 +3320,20 @@ int ba_debug_solve_info(ba_solver *s, char *name, int cap, double *vals) {
   alg += 4.0 * env_entries;
   std::string nm;
   double exec = 0.0, ctas = 1.0, chain = 0.0;
-  static const int band_mode = getenv("BA_B200_BAND_MODE") ? atoi(getenv("BA_B200_BAND_MODE")) : 6;
-  if (pl.banded && pl.nd.valid && pl.nd_dev.tpw > 0 && band_mode >= 5) {
+  const bool persistent = pl.path == SolvePath::NdPersistent;
+  if (persistent || pl.path == SolvePath::NdLevels) {
     for (const NdNode &nd : pl.nd.nodes) {
       const double R = nd.k8 + nd.b8;
       for (int c = 0; c < nd.k8; ++c) exec += (R - c) * (R - c);
     }
     chain = nd_plan_cost(pl.nd);
-    ctas = band_mode == 6 ? pl.nd.n_ctas + pl.nd.n_helpers : pl.nd.n_leaves;
+    ctas = persistent ? pl.nd.n_ctas + pl.nd.n_helpers : pl.nd.n_leaves;
     char buf[256];
     snprintf(buf, sizeof(buf), "%s<%d,%d> (partitioned banded Cholesky: nested dissection depth %d, %d fronts, DMMA panel solves and updates)",
-             band_mode == 6 ? "k_nd_persistent" : "k_nd_forward_level+k_nd_backward_level", pl.nd_dev.tpw, nd_cons_for(pl.nd.max_BT),
+             persistent ? "k_nd_persistent" : "k_nd_forward_level+k_nd_backward_level", pl.nd_dev.tpw, nd_cons_for(pl.nd.max_BT),
              pl.nd.depth, (int)pl.nd.nodes.size());
     nm = buf;
-  } else if (pl.banded) {
+  } else if (pl.path == SolvePath::Banded) {
     const double W = pl.bw + 16.0;
     exec = (double)n * W * W;
     chain = n / 8.0;
@@ -3331,13 +3344,11 @@ int ba_debug_solve_info(ba_solver *s, char *name, int cap, double *vals) {
       exec += (double)kNB * kNB * kNB * (1.0 / 3.0 + m + m * (m + 1) / 2.0);
     }
     chain = n / 8.0;
-    ctas = pl.cluster_size > 0 ? pl.cluster_size : 148;
-    nm = pl.cluster_size > 0 ? "k_chol_cluster (blocked Cholesky in one thread-block-cluster launch)"
+    ctas = pl.path == SolvePath::Cluster ? pl.cluster_size : 148;
+    nm = pl.path == SolvePath::Cluster ? "k_chol_cluster (blocked Cholesky in one thread-block-cluster launch)"
                              : "k_chol_diag+k_chol_trsm+k_syrk_update (blocked dense Cholesky, DMMA TRSM and trailing update)";
   }
-  const size_t ld = (size_t)n + 1;
-  static const size_t band_clear_min = (size_t)(getenv("BA_B200_BAND_CLEAR_MIN_MB") ? atoi(getenv("BA_B200_BAND_CLEAR_MIN_MB")) : 64) << 20;
-  const bool band_clear = pl.banded && ld * ld * sizeof(double) > band_clear_min;   // steady state of the LM loop
+  const bool band_clear = clears_band_only(s);   // steady state of the LM loop
   vals[0] = alg; vals[1] = exec; vals[2] = (double)n * n * n / 3.0 + 2.0 * n * n; vals[3] = pl.bw; vals[4] = ctas;
   vals[5] = chain; vals[6] = band_clear ? 1.0 : 0.0; vals[7] = 8.0 * (env_entries + 2.0 * n);
   if (name && cap > 0) { strncpy(name, nm.c_str(), cap - 1); name[cap - 1] = 0; }
@@ -3444,9 +3455,9 @@ static bool ipc_map_all(SharedComm &sc, cudaStream_t st, void *local, void **map
 
 // peer exchange of the LM scalars: every rank allocates its PeerExch and maps the others'; falls back to the NCCL
 // all-reduce of the scalars when that fails anywhere
-static void setup_peer_exchange(SharedComm &sc, cudaStream_t st) {
+static void setup_peer_exchange(SharedComm &sc, cudaStream_t st, bool no_peer_exchange) {
   sc.peer_ok = false;
-  if (getenv("BA_B200_NO_PEER_EXCHANGE") || sc.n_ranks > kMaxRanks) return;
+  if (no_peer_exchange || sc.n_ranks > kMaxRanks) return;
   bool ok = true;
   if (cudaMalloc(&sc.local, sizeof(PeerExch)) != cudaSuccess) { sc.local = nullptr; ok = false; }
   if (cudaMalloc(&sc.d_epoch, sizeof(unsigned)) != cudaSuccess) { sc.d_epoch = nullptr; ok = false; }
@@ -3460,13 +3471,13 @@ static void setup_peer_exchange(SharedComm &sc, cudaStream_t st) {
   void *mapped[kMaxRanks] = {};
   sc.peer_ok = ipc_map_all(sc, st, ok ? sc.local : nullptr, mapped);
   for (int r = 0; r < sc.n_ranks; ++r) sc.peer[r] = sc.peer_ok ? static_cast<PeerExch *>(mapped[r]) : nullptr;
-  if (getenv("BA_B200_VERBOSE")) fprintf(stderr, "[ba_b200] rank %d/%d: scalar exchange over %s\n", sc.rank, sc.n_ranks, sc.peer_ok ? "peer memory (CUDA IPC)" : "ncclAllReduce");
+  if (sc.verbose) fprintf(stderr, "[ba_b200] rank %d/%d: scalar exchange over %s\n", sc.rank, sc.n_ranks, sc.peer_ok ? "peer memory (CUDA IPC)" : "ncclAllReduce");
 }
 
 // band exchange through peer memory: (re)allocated when a problem needs more than the current capacity.  Collective:
 // every rank calls it at the same point (agree_on_envelope) with the same count (same global plan).
 static void ensure_band_exchange(SharedComm &sc, cudaStream_t st, long long count) {
-  if (!sc.peer_ok || getenv("BA_B200_NO_PEER_BAND") || count <= 0) return;
+  if (!sc.peer_ok || count <= 0) return;
   if (sc.band_ok && count <= sc.band_cap) return;
   if (sc.band_local) sc.retire_band();           // graphs of earlier solvers keep using the old set
   const long long cap = (count + 511) / 512 * 512;
@@ -3497,7 +3508,7 @@ static void ensure_band_exchange(SharedComm &sc, cudaStream_t st, long long coun
   }
   sc.band_cap = sc.band_ok ? cap : 0;
   sc.band_pslot = pslot;
-  if (getenv("BA_B200_VERBOSE")) fprintf(stderr, "[ba_b200] rank %d/%d: band exchange over %s (%lld doubles per slot)\n", sc.rank, sc.n_ranks, sc.band_ok ? "peer memory (CUDA IPC)" : "ncclAllReduce", cap);
+  if (sc.verbose) fprintf(stderr, "[ba_b200] rank %d/%d: band exchange over %s (%lld doubles per slot)\n", sc.rank, sc.n_ranks, sc.band_ok ? "peer memory (CUDA IPC)" : "ncclAllReduce", cap);
 }
 
 static int adopt_comm(ba_solver *s, const std::shared_ptr<SharedComm> &sc, long long global_M, long long global_n_obs) {
@@ -3520,10 +3531,10 @@ int ba_comm_init(ba_solver *s, const void *id128, int rank, int nranks, long lon
   s->comm = nullptr;
   s->shared.reset();                       // re-initialisation: the old communicator goes when its last user does
   auto sc = std::make_shared<SharedComm>();
-  sc->device = s->device; sc->rank = rank; sc->n_ranks = nranks;
+  sc->device = s->device; sc->rank = rank; sc->n_ranks = nranks; sc->verbose = s->sw.verbose;
   ncclResult_t r = g_nccl.CommInitRank(&sc->comm, nranks, id, rank);
   if (r != ncclSuccess) { s->err = "ncclCommInitRank failed"; sc->comm = nullptr; return BA_ERR_NCCL; }
-  setup_peer_exchange(*sc, s->stream);
+  setup_peer_exchange(*sc, s->stream, s->sw.no_peer_exchange);
   {
     std::lock_guard<std::mutex> lk(g_comm_mu);
     g_comm_registry[s->device] = sc;       // the device's communicator for later ba_comm_attach calls

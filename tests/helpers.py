@@ -92,3 +92,13 @@ def launched_kernels(run, names):
             return {k for k in names if any(k in n for n in seen)}
         pause *= 2
     raise AssertionError(f"no profile kept its marker kernel (last pause {pause / 2} s): {sorted(seen)}")
+
+
+def solve_info(e):
+    """(name, vals) of the reduced solve the engine's plan selected (ba_debug_solve_info)."""
+    import ctypes as C
+    from bundle_adjustment_solver_b200.capi import ptr
+    name = C.create_string_buffer(512)
+    vals = np.zeros(8)
+    assert e.L.ba_debug_solve_info(e.h, name, 512, ptr(vals)) == 0
+    return name.value.decode(), vals

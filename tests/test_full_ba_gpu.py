@@ -7,7 +7,8 @@ import numpy as np
 import pytest
 
 from bundle_adjustment_solver_b200 import scenes
-from helpers import BLOCK_TOL, blockwise_rel_err, compare_blocks, load_engine, load_oracle, options_pair
+from helpers import (BLOCK_TOL, blockwise_rel_err, compare_blocks, launched_kernels, load_engine, load_oracle,
+                     options_pair, solve_info)
 
 pytestmark = pytest.mark.gpu
 
@@ -396,6 +397,37 @@ def test_multikernel_and_cluster_reduced_solve_match_numpy(chol_mode, engine_lib
     assert err < 1e-9, (err, n)
 
 
+SOLVE_KERNELS = ("k_nd_persistent", "k_nd_forward_level", "k_chol_banded_smem", "k_chol_cluster", "k_chol_diag")
+
+
+def test_reported_solve_is_the_launched_solve(monkeypatch, engine_lib):
+    """Every solver runs the reduced solve its own switches select, whatever the other solvers of the process use, and
+    ba_debug_solve_info (bench.py's roofline and byte accounting) names that solve: for BA_B200_BAND_MODE 6 / 5 / 4
+    and BA_B200_CHOL_MODE unset / 0 / 1 on one banded trajectory, the reported name starts with the one solve kernel
+    the build launches.  A switch changed after a solver exists does not change that solver's solve."""
+    sc = scenes.scene_trajectory(160, 4800, 6, stereo=True, seed=4, n_fixed=2)
+    _, eo = options_pair()
+    by_band_mode = {6: "k_nd_persistent", 5: "k_nd_forward_level", 4: "k_chol_banded_smem"}
+    for chol_mode in (None, 0, 1):
+        for band_mode in (6, 5, 4):
+            monkeypatch.setenv("BA_B200_BAND_MODE", str(band_mode))
+            if chol_mode is None:
+                monkeypatch.delenv("BA_B200_CHOL_MODE", raising=False)
+            else:
+                monkeypatch.setenv("BA_B200_CHOL_MODE", str(chol_mode))
+            e = load_engine(sc)
+            launched = launched_kernels(lambda: e.build_only(eo, 100.0, do_solve=True), SOLVE_KERNELS)
+            name = solve_info(e)[0]
+            want = {None: by_band_mode[band_mode], 0: "k_chol_diag", 1: "k_chol_cluster"}[chol_mode]
+            assert launched == {want} and name.startswith(want), (band_mode, chol_mode, launched, name)
+    monkeypatch.delenv("BA_B200_CHOL_MODE", raising=False)
+    monkeypatch.setenv("BA_B200_BAND_MODE", "6")
+    e = load_engine(sc)
+    monkeypatch.setenv("BA_B200_BAND_MODE", "4")
+    launched = launched_kernels(lambda: e.build_only(eo, 100.0, do_solve=True), SOLVE_KERNELS)
+    assert launched == {"k_nd_persistent"} and solve_info(e)[0].startswith("k_nd_persistent"), launched
+
+
 def test_dense_reduced_system_dmma_two_level(engine_lib):
     """Loop closures make S dense: n = 2388 > 2048 takes the two-level blocked Cholesky with DMMA TRSM/SYRK
     tiles and the multi-CTA backward sweep."""
@@ -612,36 +644,21 @@ def test_tile_build_is_bit_reproducible(engine_lib):
     assert costs[0] == costs[1]
 
 
-_BAND_CLEAR_WORKER = r'''
-import sys, numpy as np
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + "/tests")
-from bundle_adjustment_solver_b200 import capi, scenes
-from bundle_adjustment_solver_b200 import solver as S
-sc = scenes.scene_trajectory(150, 6000, 8, stereo=True, seed=12, n_fixed=2)
-e = S.load_scene(S.FullBundleAdjustmentSolver(device=0), sc)
-summ = S.Summary()
-e.solve(capi.default_options(max_num_iterations=25, threshold_cost_change=1e-9, threshold_step_size=1e-9), summ)
-print("COSTS", " ".join(repr(i.cost) for i in summ.optimization_info_list))
-print("POSES", repr(float(np.abs(e.get_poses()).sum())))
-'''
-
-
-def test_band_only_clearing_of_the_reduced_system_is_equivalent(tmp_path, engine_lib):
+def test_band_only_clearing_of_the_reduced_system_is_equivalent(monkeypatch, engine_lib):
     """Large banded systems (C4: 1.15 GB dense) clear only the band of S per iteration; forced on a small banded
     problem the LM trajectory must be the one of the full clear (same kernels, same inputs)."""
-    import os, subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "band_clear.py"
-    script.write_text(_BAND_CLEAR_WORKER)
+    from bundle_adjustment_solver_b200 import capi
+    from bundle_adjustment_solver_b200 import solver as S
+    sc = scenes.scene_trajectory(150, 6000, 8, stereo=True, seed=12, n_fixed=2)
     outs = []
     for mb in ("0", "100000"):
-        r = subprocess.run([sys.executable, str(script), root], capture_output=True, text=True, timeout=300,
-                           env=dict(os.environ, BA_B200_BAND_CLEAR_MIN_MB=mb))
-        assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
-        vals = {ln.split()[0]: np.array([float(x) for x in ln.split()[1:]]) for ln in r.stdout.splitlines()
-                if ln.startswith(("COSTS", "POSES"))}
-        outs.append(vals)
-    # the flush of the tile accumulators uses FP64 reds, so two runs differ in the last bits only
+        monkeypatch.setenv("BA_B200_BAND_CLEAR_MIN_MB", mb)
+        e = S.load_scene(S.FullBundleAdjustmentSolver(device=0), sc)
+        summ = S.Summary()
+        e.solve(capi.default_options(max_num_iterations=25, threshold_cost_change=1e-9, threshold_step_size=1e-9), summ)
+        assert solve_info(e)[1][6] == (1.0 if mb == "0" else 0.0)     # band-only clearing reported as set
+        outs.append({"COSTS": np.array([i.cost for i in summ.optimization_info_list]),
+                     "POSES": np.array([float(np.abs(e.get_poses()).sum())])})
     assert len(outs[0]["COSTS"]) == len(outs[1]["COSTS"]) == 25
     np.testing.assert_allclose(outs[0]["COSTS"], outs[1]["COSTS"], rtol=1e-10)
     np.testing.assert_allclose(outs[0]["POSES"], outs[1]["POSES"], rtol=1e-10)

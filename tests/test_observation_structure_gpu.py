@@ -16,22 +16,16 @@ limits.  The scenes here are mutations of them that reach the other branches of 
 Every case asserts the path it was built for (kernel names from torch.profiler, or the reduced solve's name), so a
 change of the classification heuristics fails here instead of silently dropping the coverage."""
 import copy
-import ctypes as C
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 from bundle_adjustment_solver_b200 import scenes
-from bundle_adjustment_solver_b200.capi import ptr
 from bundle_adjustment_solver_b200.solver import Summary
-from helpers import blockwise_rel_err, compare_blocks, launched_kernels, load_engine, load_oracle, options_pair
+from helpers import blockwise_rel_err, compare_blocks, launched_kernels, load_engine, load_oracle, options_pair, solve_info
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TILE, BT_TILE, BT_PAIRS = "k_build_tiles", "k_backsub_tiles", "k_backsub_pairs"
 DENSE, PAIRS_LIST = "k_schur_dense_gemm", "k_schur_pairs_list"
 TILE_ONLY = {TILE, BT_TILE}
@@ -172,13 +166,6 @@ def _launched(run):
     return launched_kernels(run, (TILE, BT_TILE, BT_PAIRS, DENSE, PAIRS_LIST))
 
 
-def _solve_info(e):
-    name = C.create_string_buffer(512)
-    vals = np.zeros(8)
-    assert e.L.ba_debug_solve_info(e.h, name, 512, ptr(vals)) == 0
-    return name.value.decode(), vals
-
-
 def _landmark_step_error(sc, e):
     """max over landmarks with pairs of |y_i - C_i^-1 (b_i - sum_j B_ji^T x_j)| relative to the size of the terms,
     recomputed from the dumped blocks (as test_backsub_tiles_gpu.test_landmark_steps_match_dumped_blocks)."""
@@ -270,7 +257,7 @@ def test_four_camera_rig_matches_oracle(kind, accum, oracle_mod, engine_lib):
     launched, e, _ = _check_blocks(sc, accum)
     if kind == "banded":
         assert launched == TILE_ONLY, launched
-        assert _solve_info(e)[0].startswith("k_nd_persistent")    # banded plan: the storing reduce of the tile flush
+        assert solve_info(e)[0].startswith("k_nd_persistent")    # banded plan: the storing reduce of the tile flush
     else:
         assert {DENSE, BT_PAIRS} <= launched and PAIRS_LIST not in launched, launched
     _check_lm(sc, accum)
@@ -383,7 +370,7 @@ def _f_poses():
     from test_nd_plan_cpu import nd_plan
     sc = _f_base()
     e = load_engine(sc)
-    _, vals = _solve_info(e)
+    _, vals = solve_info(e)
     N, bw = e.sizes()["N"], int(vals[3])
     meta, nodes = nd_plan(N, (bw - 5) // 6)
     assert meta["valid"] and meta["depth"] >= 1, meta
@@ -393,22 +380,6 @@ def _f_poses():
     free = np.setdiff1d(np.arange(len(sc.poses_init)), sc.fixed_poses)
     kinds = {"first": 0, "leaf": mid(leaf), "separator": mid(sep), "last": N - 1}
     return {k: int(free[j]) for k, j in kinds.items()}, (N, bw)
-
-
-_SOLVE_WORKER = r'''
-import sys
-import numpy as np
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + "/tests")
-import test_observation_structure_gpu as t
-from helpers import load_engine, options_pair
-sc = t._drop_pose_observations(t._f_base(), [int(v) for v in sys.argv[3].split(",")])
-e = load_engine(sc)
-e.set_debug(True)
-e.build_only(options_pair()[1], 100.0, do_solve=True)
-n = 6 * e.sizes()["N"]
-name, vals = t._solve_info(e)
-np.savez(sys.argv[2], S=e.dump("S").reshape(n, n), rhs=e.dump("rhs"), x=e.dump("x"), name=name, vals=vals)
-'''
 
 
 def _check_zero_pivot_solve(S, rhs, x, free_idx, tol):
@@ -425,30 +396,27 @@ def _check_zero_pivot_solve(S, rhs, x, free_idx, tol):
 @pytest.mark.parametrize("band_mode,chol_mode,solve_name", [
     (6, None, "k_nd_persistent"), (5, None, "k_nd_forward_level"), (4, None, "k_chol_banded_smem"),
     (None, 0, "k_chol_diag+k_chol_trsm"), (None, 1, "k_chol_cluster")])
-def test_free_poses_without_observations_solve(band_mode, chol_mode, solve_name, tmp_path, engine_lib):
+def test_free_poses_without_observations_solve(band_mode, chol_mode, solve_name, monkeypatch, engine_lib):
     """An unobserved free pose has an exactly zero 6 x 6 block and rhs in S; every reduced solve emulates Eigen LDLT's
     D^+ = 0 there: x is exactly 0 for that pose and the rest solves the system without its rows and columns (1e-9
     relative against numpy).  The poses sit at the first and last free index, inside a leaf's own block and inside a
-    separator of the partitioned solve.  One process per mode: the solver name that ba_debug_solve_info reports reads
-    BA_B200_BAND_MODE once per process."""
+    separator of the partitioned solve.  The switches select the solve of the solver created after they are set."""
     poses, (N, bw) = _f_poses()
-    env = dict(os.environ)
     for k, v in (("BA_B200_BAND_MODE", band_mode), ("BA_B200_CHOL_MODE", chol_mode)):
-        env.pop(k, None)
-        if v is not None:
-            env[k] = str(v)
-    script = tmp_path / "solve.py"
-    script.write_text(_SOLVE_WORKER)
-    out = tmp_path / "out.npz"
-    r = subprocess.run([sys.executable, str(script), ROOT, str(out), ",".join(map(str, poses.values()))],
-                       capture_output=True, text=True, timeout=300, env=env)
-    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
-    d = np.load(out)
-    assert str(d["name"]).startswith(solve_name), str(d["name"])
-    assert int(d["vals"][3]) == bw                                # same band, so the same partition as chosen from
+        if v is None:
+            monkeypatch.delenv(k, raising=False)
+        else:
+            monkeypatch.setenv(k, str(v))
+    e = load_engine(_drop_pose_observations(_f_base(), list(poses.values())))
+    e.set_debug(True)
+    e.build_only(options_pair()[1], 100.0, do_solve=True)
+    n = 6 * e.sizes()["N"]
+    name, vals = solve_info(e)
+    assert name.startswith(solve_name), name
+    assert int(vals[3]) == bw                                     # same band, so the same partition as chosen from
     fixed = _f_base().fixed_poses
     free_idx = [int(np.sum(~np.isin(np.arange(p), fixed))) for p in poses.values()]
-    _check_zero_pivot_solve(d["S"], d["rhs"], d["x"], free_idx, 1e-9)
+    _check_zero_pivot_solve(e.dump("S").reshape(n, n), e.dump("rhs"), e.dump("x"), free_idx, 1e-9)
 
 
 def test_free_poses_without_observations_dense_two_level(engine_lib):
@@ -463,7 +431,7 @@ def test_free_poses_without_observations_dense_two_level(engine_lib):
     e.build_only(options_pair()[1], 100.0, do_solve=True)
     n = 6 * e.sizes()["N"]
     assert n > 2048
-    assert _solve_info(e)[0].startswith("k_chol_diag+k_chol_trsm")
+    assert solve_info(e)[0].startswith("k_chol_diag+k_chol_trsm")
     _check_zero_pivot_solve(e.dump("S").reshape(n, n), e.dump("rhs"), e.dump("x"), idx, 1e-8)
 
 

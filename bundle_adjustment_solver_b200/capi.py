@@ -74,11 +74,14 @@ class PoseOnlyResult(C.Structure):
     ]
 
 
+# row status of ba_observation_residuals (BA_OBS_*)
+OBS_INLIER, OBS_OUTLIER, OBS_BEHIND_CAMERA, OBS_DROPPED = 0, 1, 2, 3
+
 # every symbol include/ba_b200.h declares
 SYMBOLS = [
     "ba_create", "ba_destroy", "ba_reset", "ba_last_error", "ba_set_stream", "ba_set_profile", "ba_set_debug",
     "ba_set_cameras", "ba_set_poses", "ba_set_points", "ba_set_observations", "ba_set_observations_scaled", "ba_finalize",
-    "ba_update_parameters", "ba_solve", "ba_build_only", "ba_cost", "ba_get_poses", "ba_get_points",
+    "ba_update_parameters", "ba_solve", "ba_build_only", "ba_cost", "ba_observation_residuals", "ba_get_poses", "ba_get_points",
     "ba_get_sizes", "ba_debug_dump", "ba_debug_pairs", "ba_debug_time_solve", "ba_debug_nd_plan", "ba_debug_solve_info", "ba_comm_get_unique_id", "ba_comm_init",
     "ba_comm_destroy", "ba_comm_attach", "ba_comm_shutdown", "ba_geometry_batched", "ba_geometry_batched_f", "ba_poseonly_solve_batched", "ba_poseonly_upload", "ba_poseonly_run",
     "ba_poseonly_download", "ba_poseonly_free", "ba_version",
@@ -117,6 +120,7 @@ def lib():
         L.ba_solve.argtypes = [vp, C.POINTER(Options), vp, i, C.POINTER(Result)]
         L.ba_build_only.argtypes = [vp, C.POINTER(Options), C.c_double, i]
         L.ba_cost.argtypes = [vp, C.POINTER(C.c_double)]
+        L.ba_observation_residuals.argtypes = [vp, C.c_double, vp, vp, vp]
         L.ba_get_poses.argtypes = [vp, vp]
         L.ba_get_points.argtypes = [vp, vp]
         L.ba_get_sizes.argtypes = [vp, vp]

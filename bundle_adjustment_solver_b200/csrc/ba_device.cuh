@@ -63,6 +63,13 @@ __device__ __forceinline__ void project(const double *__restrict__ T, const doub
   p.r1 = cam[1] * yinvz + cam[3] - v;
 }
 
+// Depth zc of a projected observation in its camera: the expression project() divides by (kept apart from Proj so
+// that the kernels which inline project() are unchanged).
+__device__ __forceinline__ double camera_depth(const Proj &p, const double *__restrict__ cam) {
+  const double *Rc = cam + 4;
+  return Rc[6] * p.Xb[0] + Rc[7] * p.Xb[1] + Rc[8] * p.Xb[2] + cam[15];
+}
+
 // Huber-style weight by the L1 norm (full...cpp:763-766); thres is the float option promoted.
 __device__ __forceinline__ double huber_weight(double r0, double r1, double thres) {
   const double absrxry = fabs(r0) + fabs(r1);

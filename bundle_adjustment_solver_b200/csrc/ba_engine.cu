@@ -27,6 +27,8 @@
 //   K7 k_cost_linearize_by_pose : trial cost in pose order + the pose-side sums at the trial parameters; the last CTA
 //                             sums the partials in order and takes the rho / accept / lambda / convergence decision
 //                             on the device (:930-1007)
+// Outside the loop, k_obs_residuals (ba_observation_residuals) reports the residual and an inlier / outlier / behind-
+// camera status of every observation row at the accepted parameters, for callers that reject outliers between solves.
 // Multi-GPU: landmarks sharded; the band of [S | rhs] is exchanged through peer memory (one-shot pushes + epoch flags,
 // summed in rank order; NCCL all-reduce as the fallback), the five LM scalars by k_exchange_decide.
 // There is no CPU fallback: every entry point that computes requires a CUDA device.
@@ -956,6 +958,55 @@ __global__ void k_gather_pose_order(long long nA, const int *__restrict__ perm, 
   }
 }
 
+// ba_observation_residuals: residual and status of every observation at the accepted parameters (buffer cur), in one
+// grid-stride pass over the point-ordered arrays; row_of maps a point-order position to its input row, the outputs are
+// indexed by row.  The status counts are summed per block and added with integer atomics (exact, so deterministic).
+// Any output may be null.
+__global__ void __launch_bounds__(kThreads)
+k_obs_residuals(long long n, const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
+                const int *__restrict__ obs_point, const int *__restrict__ obs_camflags, const int *__restrict__ row_of,
+                Params prm, const double *__restrict__ cams, double thres, const LmState *__restrict__ st,
+                double2 *__restrict__ residuals, uint8_t *__restrict__ status, unsigned long long *__restrict__ counts) {
+  __shared__ unsigned wsum[kWarps][3];
+  const double *poses = prm.poses[st->cur];
+  const double *points = prm.points[st->cur];
+  unsigned cnt[3] = {0u, 0u, 0u};
+  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x) {
+    const int cf = obs_camflags[k];
+    const int pt = obs_point[k];
+    const double2 uv = obs_uv[k];
+    double T[12];
+    load_pose(poses + (size_t)obs_pose[k] * 12, T);
+    const double X[3] = {__ldg(points + (size_t)pt * 3), __ldg(points + (size_t)pt * 3 + 1),
+                         __ldg(points + (size_t)pt * 3 + 2)};
+    const double *cam = cams + (cf & kCamMask) * kCamStride;
+    Proj p;
+    project(T, X, cam, uv.x, uv.y, p);
+    int s;
+    if (!(camera_depth(p, cam) > 0.0) || !isfinite(p.r0) || !isfinite(p.r1)) s = BA_OBS_BEHIND_CAMERA;
+    else s = (fabs(p.r0) + fabs(p.r1) > thres) ? BA_OBS_OUTLIER : BA_OBS_INLIER;   // huber_weight's test
+    cnt[0] += s == BA_OBS_INLIER;
+    cnt[1] += s == BA_OBS_OUTLIER;
+    cnt[2] += s == BA_OBS_BEHIND_CAMERA;
+    const int r = row_of[k];
+    if (residuals) residuals[r] = make_double2(p.r0, p.r1);
+    if (status) status[r] = (uint8_t)s;
+  }
+  if (!counts) return;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const unsigned v = __reduce_add_sync(0xffffffffu, cnt[i]);
+    if (lane == 0) wsum[warp][i] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    unsigned long long tot = 0;
+    for (int w = 0; w < kWarps; ++w) tot += wsum[w][threadIdx.x];
+    if (tot) atomicAdd(counts + threadIdx.x, tot);
+  }
+}
+
 // Multi-GPU: ordered sums of the partials, one-shot exchange of the five scalars through the peers' mapped buffers
 // (one remote store per peer + a flag; the sum runs in rank order on every rank, so all ranks take bit-identical
 // decisions) and the trust-region decision, in ONE launch.  Replaces k_reduce_scalars + ncclAllReduce + k_decide.
@@ -1605,6 +1656,14 @@ struct ba_solver {
   std::vector<int> h_obs_cam, h_obs_pose, h_obs_point;
   std::vector<double> h_obs_uv;
   long long n_obs = 0;
+  // rows of the last ba_set_observations call (ba_observation_residuals): how many were passed in, the input row of
+  // every kept observation when some were dropped (empty: the identity), and the kept index of every point-order
+  // position (written by ba_finalize, uploaded on the first ba_observation_residuals after it)
+  long long n_rows = 0;
+  std::vector<int> h_kept_row;
+  hvec<int> h_kept_of_pos;
+  DevBuf<int> d_row_of_pos;
+  bool row_map_uploaded = false;
   int N_total = 0, M_total = 0, N = 0, M = 0;
   long long P = 0;
   bool finalized = false;
@@ -1744,6 +1803,7 @@ static void free_device(ba_solver *s) {
   s->d_point_partials.release(); s->d_pose_partials.release(); s->d_scal.release(); s->d_state.release(); s->d_ticket.release(); s->d_pose_ticket.release();
   s->d_Au[0].release(); s->d_Au[1].release(); s->d_cost_partialsA.release();
   s->d_infos.release();
+  s->d_row_of_pos.release();
 }
 
 void ba_destroy(ba_solver *s) {
@@ -1768,6 +1828,7 @@ int ba_reset(ba_solver *s) {
   s->h_poses.clear(); s->h_points.clear(); s->h_pose_fixed.clear(); s->h_point_fixed.clear();
   s->h_obs_cam.clear(); s->h_obs_pose.clear(); s->h_obs_point.clear(); s->h_obs_uv.clear();
   s->n_obs = 0; s->N_total = s->M_total = s->N = s->M = 0; s->P = 0;
+  s->n_rows = 0; s->h_kept_row.clear(); s->h_kept_of_pos.clear();
   s->finalized = false;
   destroy_graph(s);
   return BA_OK;
@@ -1832,6 +1893,8 @@ int ba_set_observations_scaled(ba_solver *s, long long n_obs, const int *cam_id,
   if (!s || n_obs < 0 || (n_obs > 0 && (!cam_id || !pose || !point || !uv))) return BA_ERR_INVALID;
   if (n_obs > 2000000000LL) { s->err = "too many observations for 32-bit indexing"; return BA_ERR_INVALID; }
   s->h_obs_cam.clear(); s->h_obs_pose.clear(); s->h_obs_point.clear(); s->h_obs_uv.clear();
+  s->n_rows = n_obs;
+  s->h_kept_row.clear();
   // fast path: every row valid (the common case) -> bulk copies and a table look-up of the camera slot
   {
     int max_id = -1, min_id = 0;
@@ -1871,7 +1934,7 @@ int ba_set_observations_scaled(ba_solver *s, long long n_obs, const int *cam_id,
     }
   }
   s->h_obs_cam.reserve(n_obs); s->h_obs_pose.reserve(n_obs); s->h_obs_point.reserve(n_obs);
-  s->h_obs_uv.reserve(2 * n_obs);
+  s->h_obs_uv.reserve(2 * n_obs); s->h_kept_row.reserve(n_obs);
   for (long long k = 0; k < n_obs; ++k) {
     auto it = s->cam_slot.find(cam_id[k]);
     if (it == s->cam_slot.end()) continue;                       // "Invalid camera index." (:160-163)
@@ -1882,6 +1945,7 @@ int ba_set_observations_scaled(ba_solver *s, long long n_obs, const int *cam_id,
     s->h_obs_point.push_back(point[k]);
     s->h_obs_uv.push_back(uv[2 * k] * uv_scale);
     s->h_obs_uv.push_back(uv[2 * k + 1] * uv_scale);
+    s->h_kept_row.push_back((int)k);
   }
   s->n_obs = (long long)s->h_obs_cam.size();
   if (n_kept) *n_kept = s->n_obs;
@@ -2016,6 +2080,9 @@ int ba_finalize(ba_solver *s) {
   // point-ordered observation arrays: written by the scatter pass of the second sort
   hvec<double2> uv(n);
   hvec<int> o_pose(n), o_point(n), o_cf(n), o_pair(n);
+  s->h_kept_of_pos.resize(n);
+  s->d_row_of_pos.release();
+  s->row_map_uploaded = false;
   {
     // both sorts: per-thread histograms over contiguous ranges of the input, bucket offsets per thread, parallel
     // scatter -- stable because every thread's range is contiguous and the ranges are ordered
@@ -2050,6 +2117,7 @@ int ba_finalize(ba_solver *s) {
       const int ps = s->h_obs_pose[k], pt = s->h_obs_point[k];
       const bool pf = s->h_pose_opt[ps] >= 0, qf = s->h_point_opt[pt] >= 0;
       pose_to_point_order[q] = pos;
+      s->h_kept_of_pos[pos] = k;
       uv[pos] = make_double2(s->h_obs_uv[2 * (size_t)k], s->h_obs_uv[2 * (size_t)k + 1]);
       o_pose[pos] = ps; o_point[pos] = pt;
       o_cf[pos] = s->h_obs_cam[k] | (pf ? kFlagPoseFree : 0) | (qf ? kFlagPointFree : 0);
@@ -2967,6 +3035,70 @@ int ba_cost(ba_solver *s, double *cost) {
   CUDA_TRY(cudaMemcpyAsync(s->h_scal, s->d_scal.p, 8 * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
   CUDA_TRY(cudaStreamSynchronize(s->stream));
   *cost = s->h_scal[0];
+  return BA_OK;
+}
+
+int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, uint8_t *status, long long *counts) {
+  if (!s) return BA_ERR_INVALID;
+  if (!(threshold >= 0.0)) { s->err = "ba_observation_residuals: threshold must be >= 0 (NaN is invalid)"; return BA_ERR_INVALID; }
+  if (int rc = ba_finalize(s)) return rc;
+  CUDA_TRY(cudaSetDevice(s->device));
+  if (int rc = ensure_stream(s)) return rc;
+  cudaStream_t st = s->stream;
+  const long long n = s->n_obs, n_rows = s->n_rows;
+  if (!s->row_map_uploaded) {
+    // point-order position -> input row: the kept index, or the input row of the kept row when some were dropped
+    if (s->h_kept_row.empty()) {
+      CUDA_TRY(s->d_row_of_pos.upload(s->h_kept_of_pos, st));
+    } else {
+      hvec<int> row(n);
+      parallel_ranges(n, [&](long long lo_, long long hi_, int) {
+        for (long long q = lo_; q < hi_; ++q) row[q] = s->h_kept_row[s->h_kept_of_pos[q]];
+      });
+      CUDA_TRY(s->d_row_of_pos.upload(row, st));
+      CUDA_TRY(cudaStreamSynchronize(st));   // `row` is freed on return
+    }
+    s->row_map_uploaded = true;
+  }
+  DevBuf<double2> d_res;
+  DevBuf<uint8_t> d_status;
+  DevBuf<unsigned long long> d_counts;
+  struct Release {   // stream-ordered frees on every return path
+    DevBuf<double2> &a; DevBuf<uint8_t> &b; DevBuf<unsigned long long> &c;
+    ~Release() { a.release(); b.release(); c.release(); }
+  } release{d_res, d_status, d_counts};
+  const bool dropped = n_rows > n;
+  if (residuals) {
+    CUDA_TRY(d_res.alloc((size_t)n_rows));
+    if (dropped) CUDA_TRY(cudaMemsetAsync(d_res.p, 0xff, (size_t)n_rows * sizeof(double2), st));   // all-ones: NaN
+  }
+  if (status) {
+    CUDA_TRY(d_status.alloc((size_t)n_rows));
+    if (dropped) CUDA_TRY(cudaMemsetAsync(d_status.p, BA_OBS_DROPPED, (size_t)n_rows, st));
+  }
+  if (counts) {
+    CUDA_TRY(d_counts.alloc(3));
+    CUDA_TRY(cudaMemsetAsync(d_counts.p, 0, 3 * sizeof(unsigned long long), st));
+  }
+  if (n > 0) {
+    const Params prm{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
+    const unsigned grid = (unsigned)std::min<long long>((n + kThreads - 1) / kThreads, 148LL * 8);
+    k_obs_residuals<<<grid, kThreads, 0, st>>>(n, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_point.p, s->d_obs_camflags.p,
+                                               s->d_row_of_pos.p, prm, s->d_cams.p, threshold, s->d_state.p, d_res.p,
+                                               d_status.p, d_counts.p);
+    CUDA_TRY(cudaGetLastError());
+  }
+  unsigned long long h_counts[3] = {0, 0, 0};
+  if (residuals && n_rows > 0)
+    CUDA_TRY(cudaMemcpyAsync(residuals, d_res.p, (size_t)n_rows * sizeof(double2), cudaMemcpyDeviceToHost, st));
+  if (status && n_rows > 0)
+    CUDA_TRY(cudaMemcpyAsync(status, d_status.p, (size_t)n_rows, cudaMemcpyDeviceToHost, st));
+  if (counts) CUDA_TRY(cudaMemcpyAsync(h_counts, d_counts.p, sizeof(h_counts), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  if (counts) {
+    for (int i = 0; i < 3; ++i) counts[i] = (long long)h_counts[i];
+    counts[BA_OBS_DROPPED] = n_rows - n;
+  }
   return BA_OK;
 }
 

@@ -113,6 +113,8 @@ class FullBundleAdjustmentSolver:
         self._obs_chunks = []
         self.is_parameter_finalized = False
         self._uploaded = False
+        self._engine_has_parameters = False
+        self._carried_internal = None   # accepted internal parameters the next upload starts from (remove_observations)
 
     def __del__(self):
         if getattr(self, "h", None):
@@ -236,6 +238,8 @@ class FullBundleAdjustmentSolver:
         _check(L.ba_set_cameras(h, len(ids), ptr(ids), ptr(intr), ptr(cT12)), L, h, "ba_set_cameras")
         if internal_override is not None:
             T12, X = internal_override
+        elif self._carried_internal is not None:
+            T12, X = self._carried_internal
         else:
             T12, X = self.internal_parameters()
         pf = np.ascontiguousarray(self.pose_fixed, dtype=np.uint8)
@@ -256,6 +260,8 @@ class FullBundleAdjustmentSolver:
         self.num_total_observations = kept.value
         _check(L.ba_finalize(h), L, h, "ba_finalize")
         self._uploaded = True
+        self._engine_has_parameters = True
+        self._carried_internal = None
 
     # --- Solve (:630-1044) -------------------------------------------------------------------
     def solve(self, options=None, summary=None):
@@ -348,6 +354,50 @@ class FullBundleAdjustmentSolver:
         c = C.c_double(0)
         _check(self.L.ba_cost(self.h, C.byref(c)), self.L, self.h, "ba_cost")
         return c.value
+
+    # --- per-observation residuals and outlier removal ---------------------------------------------
+    def observation_residuals(self, threshold=np.inf):
+        """Residuals (projection - pixel) of every observation row at the accepted parameters, with a status per row.
+
+        Rows are every observation this mirror sent to the engine, in order: bulk rows the engine dropped are rows
+        (status OBS_DROPPED, NaN residuals); scalar add_observation calls refused here never were.  threshold is in
+        the caller's pixels, on |r_u| + |r_v| as in the Huber weight; a row above it is OBS_OUTLIER, a row behind its
+        camera (or with a non-finite residual) OBS_BEHIND_CAMERA.  Returns (residuals (n, 2) in the caller's pixels,
+        status uint8 (n,), counts (4,) rows per status)."""
+        threshold = float(threshold)
+        self.is_parameter_finalized = True
+        self._upload()
+        n = self._num_rows()
+        res = np.zeros((n, 2))
+        status = np.zeros(n, dtype=np.uint8)
+        counts = np.zeros(4, dtype=np.int64)
+        _check(self.L.ba_observation_residuals(self.h, threshold * self.scaler, ptr(res), ptr(status), ptr(counts)),
+               self.L, self.h, "ba_observation_residuals")
+        return res * self.inverse_scaler, status, counts
+
+    def remove_observations(self, keep):
+        """Keep only the observation rows where `keep` (bool, one per row of observation_residuals) is true.  The next
+        solve uploads the kept rows and starts from the engine's accepted parameters, bit for bit."""
+        self._flush_scalar_obs()
+        keep = np.asarray(keep, dtype=bool)
+        if keep.shape != (self._num_rows(),):
+            raise ValueError(f"keep has shape {keep.shape}, expected ({self._num_rows()},)")
+        if self._engine_has_parameters and self._carried_internal is None:
+            self._carried_internal = self.get_internal()
+        self.is_parameter_finalized = True
+        rows = [np.concatenate([c[k] for c in self._obs_chunks]) for k in range(4)] if self._obs_chunks else None
+        self._obs_chunks = [tuple(np.ascontiguousarray(a[keep]) for a in rows)] if rows is not None else []
+        self._uploaded = False
+
+    def reject_outliers(self, threshold):
+        """Removes every row that is not OBS_INLIER at `threshold` (caller's pixels); returns how many were removed."""
+        _, status, _ = self.observation_residuals(threshold)
+        keep = status == capi.OBS_INLIER
+        self.remove_observations(keep)
+        return int((~keep).sum())
+
+    def _num_rows(self):
+        return sum(len(c[0]) for c in self._obs_chunks) + len(self._obs[0])
 
     def dump(self, name):
         n = self.L.ba_debug_dump(self.h, self.DUMP[name], None)

@@ -135,6 +135,20 @@ int ba_build_only(ba_solver *s, const ba_options *opt, double lambda, int do_sol
 /* EvaluateCurrentCost (:381-433) at the current parameters. */
 int ba_cost(ba_solver *s, double *cost);
 
+/* Per-observation residuals and a status per row, for the solve / reject outliers / solve loop of a front-end. */
+#define BA_OBS_INLIER 0
+#define BA_OBS_OUTLIER 1        /* |r_u| + |r_v| > threshold */
+#define BA_OBS_BEHIND_CAMERA 2  /* depth in the observing camera <= 0, or a non-finite residual; wins over OUTLIER */
+#define BA_OBS_DROPPED 3        /* row rejected by ba_set_observations (unknown camera id, pose or point) */
+/* Residual r = projection - pixel of every row of the last ba_set_observations(_scaled) call, in that call's row order,
+ * at the accepted parameters, in internal units (pixels x scaler_ = 0.01 for the shims).  threshold is in the same
+ * internal units and uses the same L1 norm of the residual as the full-BA Huber weight (full...cpp:763-766); a row
+ * whose norm equals the threshold is an inlier; +inf classifies depth only; NaN or negative is BA_ERR_INVALID.
+ * residuals [2*n_rows], status [n_rows] (BA_OBS_*), counts [4] (rows per BA_OBS_* value): each may be NULL.
+ * Dropped rows get NaN residuals.  Finalizes first, as ba_cost does; does not change the parameters, the LM state or
+ * the next ba_solve.  On a solver joined to a communicator: this rank's rows, no communication. */
+int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, uint8_t *status, long long *counts);
+
 /* ---- results ----------------------------------------------------------- */
 int ba_get_poses(ba_solver *s, double *T_jw);  /* all poses, 12 doubles each, internal units */
 int ba_get_points(ba_solver *s, double *X);    /* all points */

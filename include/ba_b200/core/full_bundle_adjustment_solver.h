@@ -184,15 +184,7 @@ class FullBundleAdjustmentSolver {
     FinalizeParameters();
     GetSolverStatistics();
     CheckPoseAndPointConnectivity();
-    EnsureHandle();
-    Check(ba_set_cameras(handle_, static_cast<int>(camera_ids_.size()), camera_ids_.data(), cam_intr_.data(), cam_T_.data()),
-          "ba_set_cameras");
-    Check(ba_set_poses(handle_, static_cast<int>(pose_ptrs_.size()), T_jw_.data(), pose_fixed_.data()), "ba_set_poses");
-    Check(ba_set_points(handle_, static_cast<int>(point_ptrs_.size()), X_.data(), point_fixed_.data()), "ba_set_points");
-    long long kept = 0;
-    Check(ba_set_observations(handle_, static_cast<long long>(obs_cam_.size()), obs_cam_.data(), obs_pose_.data(),
-                              obs_point_.data(), obs_uv_.data(), &kept), "ba_set_observations");
-    Check(ba_finalize(handle_), "ba_finalize");
+    Upload();
 
     ba_options o{};
     o.solver_type = static_cast<int>(options.solver_type);
@@ -256,6 +248,21 @@ class FullBundleAdjustmentSolver {
     return true;  // always (:666,1043)
   }
 
+  // cameras, the parameters (T_jw_ / X_: the initial values, or the accepted internal values written back by the
+  // last Solve) and the observation rows, then ba_finalize
+  void Upload() {
+    EnsureHandle();
+    Check(ba_set_cameras(handle_, static_cast<int>(camera_ids_.size()), camera_ids_.data(), cam_intr_.data(), cam_T_.data()),
+          "ba_set_cameras");
+    Check(ba_set_poses(handle_, static_cast<int>(pose_ptrs_.size()), T_jw_.data(), pose_fixed_.data()), "ba_set_poses");
+    Check(ba_set_points(handle_, static_cast<int>(point_ptrs_.size()), X_.data(), point_fixed_.data()), "ba_set_points");
+    long long kept = 0;
+    Check(ba_set_observations(handle_, static_cast<long long>(obs_cam_.size()), obs_cam_.data(), obs_pose_.data(),
+                              obs_point_.data(), obs_uv_.data(), &kept), "ba_set_observations");
+    Check(ba_finalize(handle_), "ba_finalize");
+    device_dirty_ = false;
+  }
+
  public:
   std::string GetSolverStatistics() const {  // :208-239 (prints; returns an empty string like the reference)
     std::stringstream ss;
@@ -283,6 +290,43 @@ class FullBundleAdjustmentSolver {
   // extension: device-side result of the last Solve (phase times need ba_set_profile)
   const ba_result &last_result() const { return last_result_; }
   ba_solver *native_handle() { EnsureHandle(); return handle_; }
+
+  // extension: residual (projection - pixel, caller's pixels) and status (BA_OBS_INLIER / _OUTLIER /
+  // _BEHIND_CAMERA, ba_b200.h) of every accepted AddObservation call, in call order, at the parameters of the last
+  // Solve (the initial ones before it).  threshold_px is in the caller's pixels, on |r_u| + |r_v| as the Huber weight
+  // measures it; +inf classifies depth only.  Either output may be null.
+  void GetObservationResiduals(double threshold_px, std::vector<_BA_Pixel> *residuals, std::vector<int> *status) {
+    FinalizeParameters();
+    if (device_dirty_ || !handle_) Upload();
+    const size_t n = obs_cam_.size();
+    std::vector<double> r(residuals ? 2 * n : 0);
+    std::vector<uint8_t> st(status ? n : 0);
+    Check(ba_observation_residuals(handle_, threshold_px * scaler_, residuals ? r.data() : nullptr,
+                                   status ? st.data() : nullptr, nullptr), "ba_observation_residuals");
+    if (residuals) {
+      residuals->resize(n);
+      for (size_t k = 0; k < n; ++k) (*residuals)[k] = _BA_Pixel(r[2 * k] * inverse_scaler_, r[2 * k + 1] * inverse_scaler_);
+    }
+    if (status) status->assign(st.begin(), st.end());
+  }
+
+  // extension: removes every observation that is not BA_OBS_INLIER at threshold_px (caller's pixels) and returns how
+  // many were removed.  The next Solve starts from the accepted parameters of the last one.
+  int RemoveOutlierObservations(double threshold_px) {
+    std::vector<int> status;
+    GetObservationResiduals(threshold_px, nullptr, &status);
+    size_t w = 0;
+    for (size_t k = 0; k < status.size(); ++k) {
+      if (status[k] != BA_OBS_INLIER) continue;
+      obs_cam_[w] = obs_cam_[k]; obs_pose_[w] = obs_pose_[k]; obs_point_[w] = obs_point_[k];
+      obs_uv_[2 * w] = obs_uv_[2 * k]; obs_uv_[2 * w + 1] = obs_uv_[2 * k + 1];
+      ++w;
+    }
+    const int removed = static_cast<int>(status.size() - w);
+    obs_cam_.resize(w); obs_pose_.resize(w); obs_point_.resize(w); obs_uv_.resize(2 * w);
+    if (removed > 0) device_dirty_ = true;
+    return removed;
+  }
   void SetDevice(int device) { device_ = device; }
 
  protected:

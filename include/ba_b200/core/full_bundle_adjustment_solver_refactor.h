@@ -133,6 +133,8 @@ class FullBundleAdjustmentSolverRefactor : private FullBundleAdjustmentSolver {
   using Base::last_result;
   using Base::native_handle;
   using Base::SetDevice;
+  using Base::GetObservationResiduals;
+  using Base::RemoveOutlierObservations;
 };
 
 }  // namespace analytic_solver

@@ -29,6 +29,8 @@
 //                             on the device (:930-1007)
 // Outside the loop, k_obs_residuals (ba_observation_residuals) reports the residual and an inlier / outlier / behind-
 // camera status of every observation row at the accepted parameters, for callers that reject outliers between solves.
+// k_refine_points (ba_refine_points) refines landmarks at fixed poses: every selected landmark runs the LM loop alone
+// (structure-only bundle adjustment), in one launch.
 // Multi-GPU: landmarks sharded; the band of [S | rhs] is exchanged through peer memory (one-shot pushes + epoch flags,
 // summed in rank order; NCCL all-reduce as the fallback), the five LM scalars by k_exchange_decide.
 // There is no CPU fallback: every entry point that computes requires a CUDA device.
@@ -1007,6 +1009,150 @@ k_obs_residuals(long long n, const double2 *__restrict__ obs_uv, const int *__re
   }
 }
 
+// ba_refine_points: one pass over landmark i's observations at X, four lanes of a group taking observations sub,
+// sub + 4, ...: the cost sum ||r||_2 (:381-433) and the undamped C (upper 6, :821) / b (:823) at X.  The partials are
+// combined by an xor butterfly, so every lane of the group holds the same sums, bit for bit.
+struct PointSums {
+  double v[10];   // C upper 6 | b 3 | cost
+};
+__device__ __forceinline__ void point_pass(int a, int e, int sub, unsigned gmask, const double X[3],
+                                           const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
+                                           const int *__restrict__ obs_camflags, const double *poses,
+                                           const double *__restrict__ cams, double thres, PointSums &s) {
+  double *v = s.v;
+#pragma unroll
+  for (int c = 0; c < 10; ++c) v[c] = 0.0;
+  for (int k = a + sub; k < e; k += 4) {
+    const double2 uv = obs_uv[k];
+    double T[12];
+    load_pose(poses + (size_t)obs_pose[k] * 12, T);
+    ObsLin o;
+    linearize_obs(T, X, cams + (obs_camflags[k] & kCamMask) * kCamStride, uv.x, uv.y, thres, o);
+    const double *Rm = o.Rm;
+    const double wr0 = o.w * o.pr.r0, wr1 = o.w * o.pr.r1;
+    v[0] += o.w * (Rm[0] * Rm[0] + Rm[3] * Rm[3]);
+    v[1] += o.w * (Rm[0] * Rm[1] + Rm[3] * Rm[4]);
+    v[2] += o.w * (Rm[0] * Rm[2] + Rm[3] * Rm[5]);
+    v[3] += o.w * (Rm[1] * Rm[1] + Rm[4] * Rm[4]);
+    v[4] += o.w * (Rm[1] * Rm[2] + Rm[4] * Rm[5]);
+    v[5] += o.w * (Rm[2] * Rm[2] + Rm[5] * Rm[5]);
+    v[6] -= Rm[0] * wr0 + Rm[3] * wr1;
+    v[7] -= Rm[1] * wr0 + Rm[4] * wr1;
+    v[8] -= Rm[2] * wr0 + Rm[5] * wr1;
+    v[9] += sqrt(o.pr.r0 * o.pr.r0 + o.pr.r1 * o.pr.r1);
+  }
+#pragma unroll
+  for (int c = 0; c < 10; ++c) {
+    v[c] += __shfl_xor_sync(gmask, v[c], 1);
+    v[c] += __shfl_xor_sync(gmask, v[c], 2);
+  }
+}
+
+// ba_refine_points: structure-only LM, Solve's loop (:707-1008) on every selected free landmark alone with every pose
+// fixed (N_opt = 0: no Schur complement, y = C^-1 b, step = ||y||).  Four adjacent lanes per landmark, one landmark per
+// group, the whole loop in one launch with the iteration state in registers.  The trial-cost pass also forms C / b at
+// the trial point: on accept they are the next linearisation, on reject the kept sums are still in registers (the
+// speculative pose side's idea; bit-identical to re-linearising, same code and order).  The rho / lambda / convergence
+// arithmetic restates decide() per landmark instead of sharing it: decide() works on the device LmState and the
+// OptimizationInfo rows of one global problem, and factoring it would change the code of the kernels that inline it.
+// Reads the points of buffer `cur` and writes the returned point of EVERY landmark (untouched ones included) into both
+// buffers; a group only touches its own landmark.  Status counts: warp and block sums + integer atomics (exact).
+constexpr int kRefineThreads = 128;   // 152 registers, no spills: three CTAs (12 warps) per SM
+__global__ void __launch_bounds__(kRefineThreads)
+k_refine_points(int M_total, const int *__restrict__ pt_start /*[M_total + 1], point-order observation ranges*/,
+                const uint8_t *__restrict__ point_free, const uint8_t *__restrict__ select /*null: all*/,
+                const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
+                const int *__restrict__ obs_camflags, ParamsW prm, const double *__restrict__ cams, double thres,
+                double lambda0, double dec_ratio, double inc_ratio, double inverse_scaler, double thr_step,
+                double thr_cost, int max_iteration, const LmState *__restrict__ st, double *__restrict__ costs,
+                int *__restrict__ iterations, uint8_t *__restrict__ status, unsigned long long *__restrict__ counts) {
+  __shared__ unsigned wsum[kRefineThreads / 32][5];
+  const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+  const int i = gt >> 2, sub = gt & 3;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned gmask = 0xfu << (lane & 28);
+  unsigned cnt[5] = {0u, 0u, 0u, 0u, 0u};
+  if (i < M_total) {
+    const bool cur = st->cur != 0;
+    const double *poses = cur ? prm.poses[1] : prm.poses[0];
+    const double *points = cur ? prm.points[1] : prm.points[0];
+    double X[3] = {points[(size_t)i * 3], points[(size_t)i * 3 + 1], points[(size_t)i * 3 + 2]};
+    const int a = pt_start[i], e = pt_start[i + 1];
+    PointSums acc;
+    point_pass(a, e, sub, gmask, X, obs_uv, obs_pose, obs_camflags, poses, cams, thres, acc);
+    const double cost0 = acc.v[9];
+    double cost = cost0;   // at the returned point
+    int code, iters = 0;
+    if (!point_free[i] || (select && !select[i])) code = BA_POINT_SKIPPED;
+    else if (e == a) code = BA_POINT_UNOBSERVED;
+    else if (!isfinite(cost0)) code = BA_POINT_NONFINITE;
+    else {
+      double lambda = lambda0, prev = cost0;
+      bool converged = false;
+      for (int it = 0; it < max_iteration; ++it) {
+        // damping (:850-852), C^-1 = ldlt().solve(I) (:854), y = C^-1 b (:910-917 without pose terms)
+        const double lp1 = 1.0 + lambda;
+        const double b[3] = {acc.v[6], acc.v[7], acc.v[8]};
+        const double cd[6] = {acc.v[0] * lp1, acc.v[1], acc.v[2], acc.v[3] * lp1, acc.v[4], acc.v[5] * lp1};
+        double inv[9];
+        ldlt3_inverse(cd, inv);
+        double y[3], Xt[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+          y[r] = inv[3 * r] * b[0] + inv[3 * r + 1] * b[1] + inv[3 * r + 2] * b[2];
+          Xt[r] = X[r] + y[r];
+        }
+        // EvaluateCostChangeByQuadraticModel (:435-455) with the damped C
+        double m = b[0] * y[0] + b[1] * y[1] + b[2] * y[2];
+        m += y[0] * (cd[0] * y[0] + cd[1] * y[1] + cd[2] * y[2]) + y[1] * (cd[1] * y[0] + cd[3] * y[1] + cd[4] * y[2]) +
+             y[2] * (cd[2] * y[0] + cd[4] * y[1] + cd[5] * y[2]);
+        const double model = -m;
+        PointSums trial;
+        point_pass(a, e, sub, gmask, Xt, obs_uv, obs_pose, obs_camflags, poses, cams, thres, trial);
+        const double trial_cost = trial.v[9];
+        const double rho = (trial_cost - prev) * inverse_scaler / model;
+        if (rho > 0.25) {   // UPDATE; otherwise RevertToReservedParameters keeps X and its sums
+          X[0] = Xt[0]; X[1] = Xt[1]; X[2] = Xt[2];
+          acc = trial;
+          cost = trial_cost;
+        }
+        if (rho > 0.5) lambda = fmax(1e-10, lambda * dec_ratio);
+        else if (rho <= 0.25) lambda = fmin(100.0, lambda * inc_ratio);
+        const double step = sqrt(y[0] * y[0] + y[1] * y[1] + y[2] * y[2]);   // N_opt + M_opt = 1
+        converged = (step < thr_step) || (fabs(trial_cost - prev) < thr_cost);
+        if (it >= max_iteration - 1) converged = false;
+        prev = trial_cost;   // unconditionally (:1005)
+        iters = it + 1;
+        if (converged) break;
+      }
+      code = converged ? BA_POINT_CONVERGED : BA_POINT_MAX_ITERATIONS;
+    }
+    if (sub < 3) {   // lane sub writes coordinate sub of both buffers
+      const double xs = sub == 0 ? X[0] : (sub == 1 ? X[1] : X[2]);
+      prm.points[0][(size_t)i * 3 + sub] = xs;
+      prm.points[1][(size_t)i * 3 + sub] = xs;
+    } else {
+      if (costs) { costs[2 * (size_t)i] = cost0; costs[2 * (size_t)i + 1] = cost; }
+      if (iterations) iterations[i] = iters;
+      if (status) status[i] = (uint8_t)code;
+#pragma unroll
+      for (int c = 0; c < 5; ++c) cnt[c] = code == c;
+    }
+  }
+  if (!counts) return;
+#pragma unroll
+  for (int c = 0; c < 5; ++c) {
+    const unsigned v = __reduce_add_sync(0xffffffffu, cnt[c]);
+    if (lane == 0) wsum[warp][c] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < 5) {
+    unsigned long long tot = 0;
+    for (int w = 0; w < kRefineThreads / 32; ++w) tot += wsum[w][threadIdx.x];
+    if (tot) atomicAdd(counts + threadIdx.x, tot);
+  }
+}
+
 // Multi-GPU: ordered sums of the partials, one-shot exchange of the five scalars through the peers' mapped buffers
 // (one remote store per peer + a flag; the sum runs in rank order on every rank, so all ranks take bit-identical
 // decisions) and the trust-region decision, in ONE launch.  Replaces k_reduce_scalars + ncclAllReduce + k_decide.
@@ -1664,6 +1810,11 @@ struct ba_solver {
   hvec<int> h_kept_of_pos;
   DevBuf<int> d_row_of_pos;
   bool row_map_uploaded = false;
+  // observation range of every landmark in the point-ordered arrays, M_total + 1 starts (ba_refine_points): written by
+  // ba_finalize, uploaded on the first ba_refine_points after it
+  std::vector<int> h_point_obs_start;
+  DevBuf<int> d_point_obs_start;
+  bool point_start_uploaded = false;
   int N_total = 0, M_total = 0, N = 0, M = 0;
   long long P = 0;
   bool finalized = false;
@@ -1804,6 +1955,7 @@ static void free_device(ba_solver *s) {
   s->d_Au[0].release(); s->d_Au[1].release(); s->d_cost_partialsA.release();
   s->d_infos.release();
   s->d_row_of_pos.release();
+  s->d_point_obs_start.release();
 }
 
 void ba_destroy(ba_solver *s) {
@@ -1828,7 +1980,7 @@ int ba_reset(ba_solver *s) {
   s->h_poses.clear(); s->h_points.clear(); s->h_pose_fixed.clear(); s->h_point_fixed.clear();
   s->h_obs_cam.clear(); s->h_obs_pose.clear(); s->h_obs_point.clear(); s->h_obs_uv.clear();
   s->n_obs = 0; s->N_total = s->M_total = s->N = s->M = 0; s->P = 0;
-  s->n_rows = 0; s->h_kept_row.clear(); s->h_kept_of_pos.clear();
+  s->n_rows = 0; s->h_kept_row.clear(); s->h_kept_of_pos.clear(); s->h_point_obs_start.clear();
   s->finalized = false;
   destroy_graph(s);
   return BA_OK;
@@ -2083,6 +2235,8 @@ int ba_finalize(ba_solver *s) {
   s->h_kept_of_pos.resize(n);
   s->d_row_of_pos.release();
   s->row_map_uploaded = false;
+  s->d_point_obs_start.release();
+  s->point_start_uploaded = false;
   {
     // both sorts: per-thread histograms over contiguous ranges of the input, bucket offsets per thread, parallel
     // scatter -- stable because every thread's range is contiguous and the ranges are ordered
@@ -2208,6 +2362,7 @@ int ba_finalize(ba_solver *s) {
   struct Joiner { std::thread &t; ~Joiner() { if (t.joinable()) t.join(); } } early_joiner{early_upload};
   // --- observation range of every landmark in point order
   if ((long long)pt_q0.size() != (long long)Mt + 1) pt_q0.assign((size_t)Mt + 1, 0);   // (no observations at all)
+  s->h_point_obs_start.assign(pt_q0.begin(), pt_q0.end());
   // --- tile chunks: runs of consecutive landmarks whose free poses fit one window of kTileW poses
   std::vector<SchurChunk> schur_chunks;
   std::vector<int> tpt_point, tpt_inc_start, fallback_pairs;
@@ -3099,6 +3254,80 @@ int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, 
     for (int i = 0; i < 3; ++i) counts[i] = (long long)h_counts[i];
     counts[BA_OBS_DROPPED] = n_rows - n;
   }
+  return BA_OK;
+}
+
+int ba_refine_points(ba_solver *s, const ba_options *opt_in, const uint8_t *select, double *costs, int *iterations,
+                     uint8_t *status, long long *counts) {
+  if (!s || !opt_in) return BA_ERR_INVALID;
+  if (opt_in->method != BA_METHOD_LEVENBERG_MARQUARDT) { s->err = "ba_refine_points: only BA_METHOD_LEVENBERG_MARQUARDT"; return BA_ERR_INVALID; }
+  if (opt_in->max_num_iterations < 1) { s->err = "ba_refine_points: max_num_iterations must be >= 1"; return BA_ERR_INVALID; }
+  if (s->comm) { s->err = "ba_refine_points: not available on a solver joined to a communicator"; return BA_ERR_STATE; }
+  if (int rc = ba_finalize(s)) return rc;
+  CUDA_TRY(cudaSetDevice(s->device));
+  if (int rc = ensure_stream(s)) return rc;
+  cudaStream_t st = s->stream;
+  const int Mt = s->M_total;
+  if (!s->point_start_uploaded) {
+    CUDA_TRY(s->d_point_obs_start.upload(s->h_point_obs_start, st));
+    s->point_start_uploaded = true;
+  }
+  // the buffer of the accepted parameters; the kernel reads its points, the poses are copied into the other buffer
+  CUDA_TRY(cudaMemcpyAsync(s->h_state, s->d_state.p, sizeof(LmState), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  const int cur = s->h_state->cur & 1;
+  DevBuf<uint8_t> d_select, d_status;
+  DevBuf<double> d_costs;
+  DevBuf<int> d_iters;
+  DevBuf<unsigned long long> d_counts;
+  struct Release {   // stream-ordered frees on every return path
+    DevBuf<uint8_t> &a, &b; DevBuf<double> &c; DevBuf<int> &d; DevBuf<unsigned long long> &e;
+    ~Release() { a.release(); b.release(); c.release(); d.release(); e.release(); }
+  } release{d_select, d_status, d_costs, d_iters, d_counts};
+  if (select && Mt > 0) {
+    CUDA_TRY(d_select.alloc((size_t)Mt));
+    CUDA_TRY(cudaMemcpyAsync(d_select.p, select, (size_t)Mt, cudaMemcpyHostToDevice, st));
+  }
+  if (status) CUDA_TRY(d_status.alloc((size_t)Mt));
+  if (costs) CUDA_TRY(d_costs.alloc(2 * (size_t)Mt));
+  if (iterations) CUDA_TRY(d_iters.alloc((size_t)Mt));
+  if (counts) {
+    CUDA_TRY(d_counts.alloc(5));
+    CUDA_TRY(cudaMemsetAsync(d_counts.p, 0, 5 * sizeof(unsigned long long), st));
+  }
+  if (Mt > 0) {
+    const double inverse_scaler = opt_in->inverse_scaler == 0.0 ? 100.0 : opt_in->inverse_scaler;
+    const ParamsW prw{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
+    const unsigned grid = (unsigned)(((long long)Mt * 4 + kRefineThreads - 1) / kRefineThreads);
+    k_refine_points<<<grid, kRefineThreads, 0, st>>>(
+        Mt, s->d_point_obs_start.p, s->d_point_free.p, d_select.p, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_camflags.p,
+        prw, s->d_cams.p, (double)opt_in->threshold_huber_loss, (double)opt_in->initial_lambda,
+        (double)opt_in->decrease_ratio_lambda, (double)opt_in->increase_ratio_lambda, inverse_scaler,
+        (double)opt_in->threshold_step_size, (double)opt_in->threshold_cost_change, opt_in->max_num_iterations,
+        s->d_state.p, d_costs.p, d_iters.p, d_status.p, d_counts.p);
+    CUDA_TRY(cudaGetLastError());
+  }
+  // the state ba_update_parameters(s, NULL, refined points) leaves: both buffers hold the accepted poses and the
+  // refined points, the LM state is cleared (cur = 0), and the host copy of the points follows
+  if (cur == 1 && s->N_total > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->d_poses[0].p, s->d_poses[1].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  else if (s->N_total > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->d_poses[1].p, s->d_poses[0].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  CUDA_TRY(cudaMemsetAsync(s->d_state.p, 0, sizeof(LmState), st));
+  s->h_points.resize((size_t)Mt * 3);
+  if (Mt > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->h_points.data(), s->d_points[0].p, (size_t)Mt * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
+  unsigned long long h_counts[5] = {0, 0, 0, 0, 0};
+  if (costs && Mt > 0) CUDA_TRY(cudaMemcpyAsync(costs, d_costs.p, 2 * (size_t)Mt * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (iterations && Mt > 0) CUDA_TRY(cudaMemcpyAsync(iterations, d_iters.p, (size_t)Mt * sizeof(int), cudaMemcpyDeviceToHost, st));
+  if (status && Mt > 0) CUDA_TRY(cudaMemcpyAsync(status, d_status.p, (size_t)Mt, cudaMemcpyDeviceToHost, st));
+  if (counts) CUDA_TRY(cudaMemcpyAsync(h_counts, d_counts.p, sizeof(h_counts), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  {
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { s->err = std::string("kernel failure: ") + cudaGetErrorString(e); return BA_ERR_CUDA; }
+  }
+  if (counts) for (int i = 0; i < 5; ++i) counts[i] = (long long)h_counts[i];
   return BA_OK;
 }
 

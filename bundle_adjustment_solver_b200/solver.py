@@ -399,6 +399,36 @@ class FullBundleAdjustmentSolver:
     def _num_rows(self):
         return sum(len(c[0]) for c in self._obs_chunks) + len(self._obs[0])
 
+    # --- structure-only bundle adjustment -----------------------------------------------------------
+    def refine_points(self, options=None, select=None):
+        """Refines landmarks at fixed poses: every selected free landmark runs the LM loop of solve() alone, over all
+        of its observations, with its own lambda and convergence verdict (ba_refine_points).  select: bool per
+        landmark, or None for every free landmark.  Only options.method = LM is accepted.  Writes the refined landmarks
+        into self.points (caller's units); the next solve starts from them.  Returns (status uint8 (M,) of
+        capi.POINT_*, iterations int32 (M,), costs (M, 2): the cost of each landmark's observations at entry and at the
+        returned point, in the engine's units as in the iteration table)."""
+        options = options or default_options()
+        if options.inverse_scaler == 0.0:
+            options.inverse_scaler = self.inverse_scaler
+        self.is_parameter_finalized = True
+        self._upload()
+        m = len(np.asarray(self.points).reshape(-1, 3))
+        sel = None
+        if select is not None:
+            sel = np.ascontiguousarray(np.asarray(select, dtype=bool).astype(np.uint8))
+            if sel.shape != (m,):
+                raise ValueError(f"select has shape {sel.shape}, expected ({m},)")
+        status = np.zeros(m, dtype=np.uint8)
+        iterations = np.zeros(m, dtype=np.int32)
+        costs = np.zeros((m, 2))
+        _check(self.L.ba_refine_points(self.h, C.byref(options), ptr(sel), ptr(costs), ptr(iterations), ptr(status), None),
+               self.L, self.h, "ba_refine_points")
+        X = np.zeros((m, 3))
+        _check(self.L.ba_get_points(self.h, ptr(X)), self.L, self.h, "ba_get_points")
+        refined = status <= capi.POINT_MAX_ITERATIONS
+        self.points[refined] = X[refined] * self.inverse_scaler
+        return status, iterations, costs
+
     def dump(self, name):
         n = self.L.ba_debug_dump(self.h, self.DUMP[name], None)
         if n < 0:

@@ -149,6 +149,26 @@ int ba_cost(ba_solver *s, double *cost);
  * the next ba_solve.  On a solver joined to a communicator: this rank's rows, no communication. */
 int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, uint8_t *status, long long *counts);
 
+/* Structure-only bundle adjustment: refines landmarks while every pose stays where it is. */
+#define BA_POINT_CONVERGED 0       /* the loop ended on the step / cost-change test */
+#define BA_POINT_MAX_ITERATIONS 1  /* max_num_iterations reached without converging */
+#define BA_POINT_SKIPPED 2         /* fixed, or not selected: untouched */
+#define BA_POINT_UNOBSERVED 3      /* selected and free, but no observation: untouched */
+#define BA_POINT_NONFINITE 4       /* cost at the start is not finite: untouched, no iteration */
+/* Every selected free landmark i runs Solve's LM loop (:707-1008) on the problem made of landmark i alone, every pose
+ * fixed, and all of i's observations (those from poses that are fixed in the registered problem included): its own
+ * lambda (from initial_lambda), iteration count and convergence verdict, step = ||y||.  opt->method must be
+ * BA_METHOD_LEVENBERG_MARQUARDT and max_num_iterations >= 1 (else BA_ERR_INVALID); check_every, use_graph and
+ * b_accumulate are ignored.  select [M_total] (order of ba_set_points), or NULL for every free landmark.
+ * costs [2*M_total]: the cost sum ||r||_2 of each landmark's observations at entry and at the returned point, for
+ * every landmark (skipped ones included; 0 without observations), internal units as ba_iter_info.cost.
+ * iterations [M_total], status [M_total] (BA_POINT_*), counts [5] (landmarks per BA_POINT_* value): each may be NULL.
+ * Finalizes first, as ba_cost does.  Afterwards the poses are unchanged and the solver is in the state
+ * ba_update_parameters(s, NULL, refined points) leaves: the next ba_solve, ba_cost or ba_observation_residuals
+ * behaves as on a solver given these parameters.  BA_ERR_STATE on a solver joined to a communicator. */
+int ba_refine_points(ba_solver *s, const ba_options *opt, const uint8_t *select, double *costs, int *iterations,
+                     uint8_t *status, long long *counts);
+
 /* ---- results ----------------------------------------------------------- */
 int ba_get_poses(ba_solver *s, double *T_jw);  /* all poses, 12 doubles each, internal units */
 int ba_get_points(ba_solver *s, double *X);    /* all points */

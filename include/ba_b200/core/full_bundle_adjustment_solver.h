@@ -186,21 +186,7 @@ class FullBundleAdjustmentSolver {
     CheckPoseAndPointConnectivity();
     Upload();
 
-    ba_options o{};
-    o.solver_type = static_cast<int>(options.solver_type);
-    o.threshold_step_size = options.convergence_handle.threshold_step_size;
-    o.threshold_cost_change = options.convergence_handle.threshold_cost_change;
-    o.threshold_huber_loss = options.outlier_handle.threshold_huber_loss;
-    o.threshold_outlier_rejection = options.outlier_handle.threshold_outlier_rejection;
-    o.max_num_iterations = options.iteration_handle.max_num_iterations;
-    o.initial_lambda = options.trust_region_handle.initial_lambda;
-    o.decrease_ratio_lambda = options.trust_region_handle.decrease_ratio_lambda;
-    o.increase_ratio_lambda = options.trust_region_handle.increase_ratio_lambda;
-    o.b_accumulate = options.accumulate_offdiagonal_blocks ? 1 : 0;
-    o.inverse_scaler = inverse_scaler_;
-    o.check_every = 0;
-    o.use_graph = 1;
-    o.method = method;
+    const ba_options o = EngineOptions(options, method);
     const int cap = o.max_num_iterations > 0 ? o.max_num_iterations : 1;
     std::vector<ba_iter_info> infos(cap);
     ba_result result{};
@@ -246,6 +232,26 @@ class FullBundleAdjustmentSolver {
     }
     last_result_ = result;
     return true;  // always (:666,1043)
+  }
+
+  // Options -> ba_options of the engine
+  ba_options EngineOptions(const Options &options, int method) const {
+    ba_options o{};
+    o.solver_type = static_cast<int>(options.solver_type);
+    o.threshold_step_size = options.convergence_handle.threshold_step_size;
+    o.threshold_cost_change = options.convergence_handle.threshold_cost_change;
+    o.threshold_huber_loss = options.outlier_handle.threshold_huber_loss;
+    o.threshold_outlier_rejection = options.outlier_handle.threshold_outlier_rejection;
+    o.max_num_iterations = options.iteration_handle.max_num_iterations;
+    o.initial_lambda = options.trust_region_handle.initial_lambda;
+    o.decrease_ratio_lambda = options.trust_region_handle.decrease_ratio_lambda;
+    o.increase_ratio_lambda = options.trust_region_handle.increase_ratio_lambda;
+    o.b_accumulate = options.accumulate_offdiagonal_blocks ? 1 : 0;
+    o.inverse_scaler = inverse_scaler_;
+    o.check_every = 0;
+    o.use_graph = 1;
+    o.method = method;
+    return o;
   }
 
   // cameras, the parameters (T_jw_ / X_: the initial values, or the accepted internal values written back by the
@@ -326,6 +332,31 @@ class FullBundleAdjustmentSolver {
     obs_cam_.resize(w); obs_pose_.resize(w); obs_point_.resize(w); obs_uv_.resize(2 * w);
     if (removed > 0) device_dirty_ = true;
     return removed;
+  }
+
+  // extension: structure-only bundle adjustment.  Every free landmark runs Solve's LM loop alone, over all of its
+  // observations, with every pose where it is (its own lambda and convergence verdict; ba_refine_points).  Starts from
+  // the parameters of the last Solve (the initial ones before it); the refined landmarks are written through the
+  // caller's _BA_Point pointers, and the next Solve starts from them.  status (optional): a BA_POINT_* value per
+  // AddPoint call.  Returns the number of landmarks refined (BA_POINT_CONVERGED or BA_POINT_MAX_ITERATIONS).
+  int RefinePoints(Options options, std::vector<int> *status = nullptr) {
+    FinalizeParameters();
+    if (device_dirty_ || !handle_) Upload();
+    const ba_options o = EngineOptions(options, BA_METHOD_LEVENBERG_MARQUARDT);
+    const size_t m = point_ptrs_.size();
+    std::vector<uint8_t> st(m);
+    Check(ba_refine_points(handle_, &o, nullptr, nullptr, nullptr, st.data(), nullptr), "ba_refine_points");
+    std::vector<double> X(m * 3);
+    Check(ba_get_points(handle_, X.data()), "ba_get_points");
+    X_ = X;
+    int refined = 0;
+    for (size_t i = 0; i < m; ++i) {
+      if (st[i] != BA_POINT_CONVERGED && st[i] != BA_POINT_MAX_ITERATIONS) continue;
+      *point_ptrs_[i] = _BA_Point(X[i * 3] * inverse_scaler_, X[i * 3 + 1] * inverse_scaler_, X[i * 3 + 2] * inverse_scaler_);
+      ++refined;
+    }
+    if (status) status->assign(st.begin(), st.end());
+    return refined;
   }
   void SetDevice(int device) { device_ = device; }
 

@@ -135,6 +135,7 @@ class FullBundleAdjustmentSolverRefactor : private FullBundleAdjustmentSolver {
   using Base::SetDevice;
   using Base::GetObservationResiduals;
   using Base::RemoveOutlierObservations;
+  using Base::RefinePoints;
 };
 
 }  // namespace analytic_solver

@@ -78,12 +78,15 @@ class PoseOnlyResult(C.Structure):
 OBS_INLIER, OBS_OUTLIER, OBS_BEHIND_CAMERA, OBS_DROPPED = 0, 1, 2, 3
 # landmark status of ba_refine_points (BA_POINT_*)
 POINT_CONVERGED, POINT_MAX_ITERATIONS, POINT_SKIPPED, POINT_UNOBSERVED, POINT_NONFINITE = 0, 1, 2, 3, 4
+# landmark status of ba_triangulate_points (BA_TRI_*)
+(TRI_TRIANGULATED, TRI_SKIPPED, TRI_TOO_FEW_OBSERVATIONS, TRI_LOW_PARALLAX, TRI_BEHIND_CAMERA,
+ TRI_LARGE_RESIDUAL) = 0, 1, 2, 3, 4, 5
 
 # every symbol include/ba_b200.h declares
 SYMBOLS = [
     "ba_create", "ba_destroy", "ba_reset", "ba_last_error", "ba_set_stream", "ba_set_profile", "ba_set_debug",
     "ba_set_cameras", "ba_set_poses", "ba_set_points", "ba_set_observations", "ba_set_observations_scaled", "ba_finalize",
-    "ba_update_parameters", "ba_solve", "ba_build_only", "ba_cost", "ba_observation_residuals", "ba_refine_points", "ba_get_poses", "ba_get_points",
+    "ba_update_parameters", "ba_solve", "ba_build_only", "ba_cost", "ba_observation_residuals", "ba_refine_points", "ba_triangulate_points", "ba_get_poses", "ba_get_points",
     "ba_get_sizes", "ba_debug_dump", "ba_debug_pairs", "ba_debug_time_solve", "ba_debug_nd_plan", "ba_debug_solve_info", "ba_comm_get_unique_id", "ba_comm_init",
     "ba_comm_destroy", "ba_comm_attach", "ba_comm_shutdown", "ba_geometry_batched", "ba_geometry_batched_f", "ba_poseonly_solve_batched", "ba_poseonly_upload", "ba_poseonly_run",
     "ba_poseonly_download", "ba_poseonly_free", "ba_version",
@@ -124,6 +127,7 @@ def lib():
         L.ba_cost.argtypes = [vp, C.POINTER(C.c_double)]
         L.ba_observation_residuals.argtypes = [vp, C.c_double, vp, vp, vp]
         L.ba_refine_points.argtypes = [vp, C.POINTER(Options), vp, vp, vp, vp, vp]
+        L.ba_triangulate_points.argtypes = [vp, vp, C.c_double, C.c_double, vp, vp]
         L.ba_get_poses.argtypes = [vp, vp]
         L.ba_get_points.argtypes = [vp, vp]
         L.ba_get_sizes.argtypes = [vp, vp]

@@ -70,6 +70,29 @@ __device__ __forceinline__ double camera_depth(const Proj &p, const double *__re
   return Rc[6] * p.Xb[0] + Rc[7] * p.Xb[1] + Rc[8] * p.Xb[2] + cam[15];
 }
 
+// Viewing ray of one observation in the world frame (ba_triangulate_points): the observing camera is R_k = R_c R_jw,
+// t_k = R_c t_jw + t_c (the transform project() applies); its centre is c = -R_k^T t_k and the unit ray through the
+// pixel is d = R_k^T m / ||m||, m = ((u - cx) / fx, (v - cy) / fy, 1).
+__device__ __forceinline__ void obs_ray(const double *__restrict__ T, const double *__restrict__ cam, double u,
+                                        double v, double *c, double *d) {
+  const double *Rc = cam + 4;
+  double Rk[9], tk[3];
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+#pragma unroll
+    for (int col = 0; col < 3; ++col)
+      Rk[r * 3 + col] = Rc[r * 3] * T[col] + Rc[r * 3 + 1] * T[3 + col] + Rc[r * 3 + 2] * T[6 + col];
+    tk[r] = Rc[r * 3] * T[9] + Rc[r * 3 + 1] * T[10] + Rc[r * 3 + 2] * T[11] + cam[13 + r];
+  }
+  const double m0 = (u - cam[2]) / cam[0], m1 = (v - cam[3]) / cam[1];
+  const double norm = sqrt(m0 * m0 + m1 * m1 + 1.0);
+#pragma unroll
+  for (int col = 0; col < 3; ++col) {
+    c[col] = -(Rk[col] * tk[0] + Rk[3 + col] * tk[1] + Rk[6 + col] * tk[2]);
+    d[col] = (Rk[col] * m0 + Rk[3 + col] * m1 + Rk[6 + col]) / norm;
+  }
+}
+
 // Huber-style weight by the L1 norm (full...cpp:763-766); thres is the float option promoted.
 __device__ __forceinline__ double huber_weight(double r0, double r1, double thres) {
   const double absrxry = fabs(r0) + fabs(r1);

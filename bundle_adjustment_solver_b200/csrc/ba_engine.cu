@@ -30,7 +30,8 @@
 // Outside the loop, k_obs_residuals (ba_observation_residuals) reports the residual and an inlier / outlier / behind-
 // camera status of every observation row at the accepted parameters, for callers that reject outliers between solves.
 // k_refine_points (ba_refine_points) refines landmarks at fixed poses: every selected landmark runs the LM loop alone
-// (structure-only bundle adjustment), in one launch.
+// (structure-only bundle adjustment), in one launch.  k_triangulate_points (ba_triangulate_points) places landmarks at
+// the midpoint of their viewing rays, with parallax, depth and residual checks, in one launch.
 // Multi-GPU: landmarks sharded; the band of [S | rhs] is exchanged through peer memory (one-shot pushes + epoch flags,
 // summed in rank order; NCCL all-reduce as the fallback), the five LM scalars by k_exchange_decide.
 // There is no CPU fallback: every entry point that computes requires a CUDA device.
@@ -1153,6 +1154,132 @@ k_refine_points(int M_total, const int *__restrict__ pt_start /*[M_total + 1], p
   }
 }
 
+// ba_triangulate_points: every selected free landmark with two or more observations is placed at the multi-view
+// midpoint of its viewing rays at the accepted poses, X = c_f + A^-1 g with A = sum_k (I - d_k d_k^T) and
+// g = sum_k (I - d_k d_k^T)(c_k - c_f), f the landmark's first observation in point order (obs_ray: centre c_k and unit
+// ray d_k of observation k).  The skeleton of k_refine_points: four adjacent lanes per landmark, lane `sub` taking
+// observations sub, sub + 4, ... of its range; every lane forms c_f / d_f itself.  Pass 1 sums A (6) and g (3) and takes
+// the minimum of d_f . d_k; the partials are combined by an xor butterfly (sum / min), so every lane holds the same
+// values and takes the same decision, bit for bit.  Parallax is tested before the solve (min d_f . d_k > cos_min:
+// BA_TRI_LOW_PARALLAX), A^-1 is ldlt3_inverse's (a non-finite X is BA_TRI_LOW_PARALLAX too).  Pass 2 projects X with
+// project() and ORs two flags across the group: depth <= 0 or a non-finite residual in some observing camera
+// (BA_TRI_BEHIND_CAMERA; k_obs_residuals' BEHIND_CAMERA test) and |r_u| + |r_v| > max_res (BA_TRI_LARGE_RESIDUAL;
+// its OUTLIER test).  Reads the points of buffer `cur` and writes every landmark into both buffers: X where the status is
+// BA_TRI_TRIANGULATED, the accepted value otherwise.  Status counts: warp and block sums + integer atomics (exact).
+constexpr int kTriangulateThreads = 128;
+__global__ void __launch_bounds__(kTriangulateThreads)
+k_triangulate_points(int M_total, const int *__restrict__ pt_start /*[M_total + 1], point-order observation ranges*/,
+                     const uint8_t *__restrict__ point_free, const uint8_t *__restrict__ select /*null: all*/,
+                     const double2 *__restrict__ obs_uv, const int *__restrict__ obs_pose,
+                     const int *__restrict__ obs_camflags, ParamsW prm, const double *__restrict__ cams,
+                     double cos_min, double max_res, const LmState *__restrict__ st, uint8_t *__restrict__ status,
+                     unsigned long long *__restrict__ counts) {
+  constexpr int kStates = 6;
+  __shared__ unsigned wsum[kTriangulateThreads / 32][kStates];
+  const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+  const int i = gt >> 2, sub = gt & 3;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned gmask = 0xfu << (lane & 28);
+  unsigned cnt[kStates] = {0u, 0u, 0u, 0u, 0u, 0u};
+  if (i < M_total) {
+    const bool cur = st->cur != 0;
+    const double *poses = cur ? prm.poses[1] : prm.poses[0];
+    const double *points = cur ? prm.points[1] : prm.points[0];
+    double X[3] = {points[(size_t)i * 3], points[(size_t)i * 3 + 1], points[(size_t)i * 3 + 2]};
+    const int a = pt_start[i], e = pt_start[i + 1];
+    int code;
+    if (!point_free[i] || (select && !select[i])) code = BA_TRI_SKIPPED;
+    else if (e - a < 2) code = BA_TRI_TOO_FEW_OBSERVATIONS;
+    else {
+      double T[12], cf[3], df[3];
+      {
+        const double2 uv = obs_uv[a];
+        load_pose(poses + (size_t)obs_pose[a] * 12, T);
+        obs_ray(T, cams + (obs_camflags[a] & kCamMask) * kCamStride, uv.x, uv.y, cf, df);
+      }
+      // pass 1: A (upper 6), g (3), min d_f . d_k
+      double v[9];
+#pragma unroll
+      for (int c = 0; c < 9; ++c) v[c] = 0.0;
+      double min_dot = __longlong_as_double(0x7ff0000000000000LL);   // +inf
+      for (int k = a + sub; k < e; k += 4) {
+        const double2 uv = obs_uv[k];
+        load_pose(poses + (size_t)obs_pose[k] * 12, T);
+        double c[3], d[3];
+        obs_ray(T, cams + (obs_camflags[k] & kCamMask) * kCamStride, uv.x, uv.y, c, d);
+        min_dot = fmin(min_dot, df[0] * d[0] + df[1] * d[1] + df[2] * d[2]);
+        const double w0 = c[0] - cf[0], w1 = c[1] - cf[1], w2 = c[2] - cf[2];
+        const double dw = d[0] * w0 + d[1] * w1 + d[2] * w2;
+        v[0] += 1.0 - d[0] * d[0];
+        v[1] -= d[0] * d[1];
+        v[2] -= d[0] * d[2];
+        v[3] += 1.0 - d[1] * d[1];
+        v[4] -= d[1] * d[2];
+        v[5] += 1.0 - d[2] * d[2];
+        v[6] += w0 - d[0] * dw;
+        v[7] += w1 - d[1] * dw;
+        v[8] += w2 - d[2] * dw;
+      }
+#pragma unroll
+      for (int c = 0; c < 9; ++c) {
+        v[c] += __shfl_xor_sync(gmask, v[c], 1);
+        v[c] += __shfl_xor_sync(gmask, v[c], 2);
+      }
+      min_dot = fmin(min_dot, __shfl_xor_sync(gmask, min_dot, 1));
+      min_dot = fmin(min_dot, __shfl_xor_sync(gmask, min_dot, 2));
+      if (min_dot > cos_min) code = BA_TRI_LOW_PARALLAX;
+      else {
+        double inv[9], Xt[3];
+        ldlt3_inverse(v, inv);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) Xt[r] = cf[r] + (inv[3 * r] * v[6] + inv[3 * r + 1] * v[7] + inv[3 * r + 2] * v[8]);
+        if (!(isfinite(Xt[0]) && isfinite(Xt[1]) && isfinite(Xt[2]))) code = BA_TRI_LOW_PARALLAX;
+        else {
+          // pass 2: depth and residual of every observation at Xt (bit 0: behind the camera, bit 1: large residual)
+          unsigned flags = 0u;
+          for (int k = a + sub; k < e; k += 4) {
+            const double2 uv = obs_uv[k];
+            load_pose(poses + (size_t)obs_pose[k] * 12, T);
+            const double *cam = cams + (obs_camflags[k] & kCamMask) * kCamStride;
+            Proj p;
+            project(T, Xt, cam, uv.x, uv.y, p);
+            if (!(camera_depth(p, cam) > 0.0) || !isfinite(p.r0) || !isfinite(p.r1)) flags |= 1u;
+            if (fabs(p.r0) + fabs(p.r1) > max_res) flags |= 2u;
+          }
+          flags = __reduce_or_sync(gmask, flags);
+          if (flags & 1u) code = BA_TRI_BEHIND_CAMERA;
+          else if (flags & 2u) code = BA_TRI_LARGE_RESIDUAL;
+          else {
+            code = BA_TRI_TRIANGULATED;
+            X[0] = Xt[0]; X[1] = Xt[1]; X[2] = Xt[2];
+          }
+        }
+      }
+    }
+    if (sub < 3) {   // lane sub writes coordinate sub of both buffers
+      const double xs = sub == 0 ? X[0] : (sub == 1 ? X[1] : X[2]);
+      prm.points[0][(size_t)i * 3 + sub] = xs;
+      prm.points[1][(size_t)i * 3 + sub] = xs;
+    } else {
+      if (status) status[i] = (uint8_t)code;
+#pragma unroll
+      for (int c = 0; c < kStates; ++c) cnt[c] = code == c;
+    }
+  }
+  if (!counts) return;
+#pragma unroll
+  for (int c = 0; c < kStates; ++c) {
+    const unsigned v = __reduce_add_sync(0xffffffffu, cnt[c]);
+    if (lane == 0) wsum[warp][c] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < kStates) {
+    unsigned long long tot = 0;
+    for (int w = 0; w < kTriangulateThreads / 32; ++w) tot += wsum[w][threadIdx.x];
+    if (tot) atomicAdd(counts + threadIdx.x, tot);
+  }
+}
+
 // Multi-GPU: ordered sums of the partials, one-shot exchange of the five scalars through the peers' mapped buffers
 // (one remote store per peer + a flag; the sum runs in rank order on every rank, so all ranks take bit-identical
 // decisions) and the trust-region decision, in ONE launch.  Replaces k_reduce_scalars + ncclAllReduce + k_decide.
@@ -1810,8 +1937,8 @@ struct ba_solver {
   hvec<int> h_kept_of_pos;
   DevBuf<int> d_row_of_pos;
   bool row_map_uploaded = false;
-  // observation range of every landmark in the point-ordered arrays, M_total + 1 starts (ba_refine_points): written by
-  // ba_finalize, uploaded on the first ba_refine_points after it
+  // observation range of every landmark in the point-ordered arrays, M_total + 1 starts (ba_refine_points,
+  // ba_triangulate_points): written by ba_finalize, uploaded on the first call of either after it
   std::vector<int> h_point_obs_start;
   DevBuf<int> d_point_obs_start;
   bool point_start_uploaded = false;
@@ -3257,6 +3384,24 @@ int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, 
   return BA_OK;
 }
 
+// The host tail of the entry points that move landmarks at fixed poses (ba_refine_points, ba_triangulate_points), once
+// their kernel has written the new points into BOTH buffers: the state ba_update_parameters(s, NULL, new points)
+// leaves.  Both buffers hold the accepted poses (buffer `cur` copied into the other), the LM state is cleared (cur = 0),
+// and the host copy of the points follows (enqueued; the caller synchronises the stream).
+static int settle_point_update(ba_solver *s, int cur) {
+  cudaStream_t st = s->stream;
+  const int Mt = s->M_total;
+  if (cur == 1 && s->N_total > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->d_poses[0].p, s->d_poses[1].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  else if (s->N_total > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->d_poses[1].p, s->d_poses[0].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  CUDA_TRY(cudaMemsetAsync(s->d_state.p, 0, sizeof(LmState), st));
+  s->h_points.resize((size_t)Mt * 3);
+  if (Mt > 0)
+    CUDA_TRY(cudaMemcpyAsync(s->h_points.data(), s->d_points[0].p, (size_t)Mt * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
+  return BA_OK;
+}
+
 int ba_refine_points(ba_solver *s, const ba_options *opt_in, const uint8_t *select, double *costs, int *iterations,
                      uint8_t *status, long long *counts) {
   if (!s || !opt_in) return BA_ERR_INVALID;
@@ -3307,16 +3452,7 @@ int ba_refine_points(ba_solver *s, const ba_options *opt_in, const uint8_t *sele
         s->d_state.p, d_costs.p, d_iters.p, d_status.p, d_counts.p);
     CUDA_TRY(cudaGetLastError());
   }
-  // the state ba_update_parameters(s, NULL, refined points) leaves: both buffers hold the accepted poses and the
-  // refined points, the LM state is cleared (cur = 0), and the host copy of the points follows
-  if (cur == 1 && s->N_total > 0)
-    CUDA_TRY(cudaMemcpyAsync(s->d_poses[0].p, s->d_poses[1].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  else if (s->N_total > 0)
-    CUDA_TRY(cudaMemcpyAsync(s->d_poses[1].p, s->d_poses[0].p, (size_t)s->N_total * 12 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  CUDA_TRY(cudaMemsetAsync(s->d_state.p, 0, sizeof(LmState), st));
-  s->h_points.resize((size_t)Mt * 3);
-  if (Mt > 0)
-    CUDA_TRY(cudaMemcpyAsync(s->h_points.data(), s->d_points[0].p, (size_t)Mt * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (int rc = settle_point_update(s, cur)) return rc;
   unsigned long long h_counts[5] = {0, 0, 0, 0, 0};
   if (costs && Mt > 0) CUDA_TRY(cudaMemcpyAsync(costs, d_costs.p, 2 * (size_t)Mt * sizeof(double), cudaMemcpyDeviceToHost, st));
   if (iterations && Mt > 0) CUDA_TRY(cudaMemcpyAsync(iterations, d_iters.p, (size_t)Mt * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -3328,6 +3464,65 @@ int ba_refine_points(ba_solver *s, const ba_options *opt_in, const uint8_t *sele
     if (e != cudaSuccess) { s->err = std::string("kernel failure: ") + cudaGetErrorString(e); return BA_ERR_CUDA; }
   }
   if (counts) for (int i = 0; i < 5; ++i) counts[i] = (long long)h_counts[i];
+  return BA_OK;
+}
+
+int ba_triangulate_points(ba_solver *s, const uint8_t *select, double min_parallax, double max_residual,
+                          uint8_t *status, long long *counts) {
+  if (!s) return BA_ERR_INVALID;
+  if (!(min_parallax > 0.0 && min_parallax <= 3.14159265358979323846)) {
+    s->err = "ba_triangulate_points: min_parallax must be in (0, pi] radians";
+    return BA_ERR_INVALID;
+  }
+  if (!(max_residual >= 0.0)) { s->err = "ba_triangulate_points: max_residual must be >= 0 (NaN is invalid)"; return BA_ERR_INVALID; }
+  if (s->comm) { s->err = "ba_triangulate_points: not available on a solver joined to a communicator"; return BA_ERR_STATE; }
+  if (int rc = ba_finalize(s)) return rc;
+  CUDA_TRY(cudaSetDevice(s->device));
+  if (int rc = ensure_stream(s)) return rc;
+  cudaStream_t st = s->stream;
+  const int Mt = s->M_total;
+  if (!s->point_start_uploaded) {
+    CUDA_TRY(s->d_point_obs_start.upload(s->h_point_obs_start, st));
+    s->point_start_uploaded = true;
+  }
+  // the buffer of the accepted parameters; the kernel reads its points, the poses are copied into the other buffer
+  CUDA_TRY(cudaMemcpyAsync(s->h_state, s->d_state.p, sizeof(LmState), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  const int cur = s->h_state->cur & 1;
+  DevBuf<uint8_t> d_select, d_status;
+  DevBuf<unsigned long long> d_counts;
+  struct Release {   // stream-ordered frees on every return path
+    DevBuf<uint8_t> &a, &b; DevBuf<unsigned long long> &c;
+    ~Release() { a.release(); b.release(); c.release(); }
+  } release{d_select, d_status, d_counts};
+  if (select && Mt > 0) {
+    CUDA_TRY(d_select.alloc((size_t)Mt));
+    CUDA_TRY(cudaMemcpyAsync(d_select.p, select, (size_t)Mt, cudaMemcpyHostToDevice, st));
+  }
+  if (status) CUDA_TRY(d_status.alloc((size_t)Mt));
+  if (counts) {
+    CUDA_TRY(d_counts.alloc(6));
+    CUDA_TRY(cudaMemsetAsync(d_counts.p, 0, 6 * sizeof(unsigned long long), st));
+  }
+  if (Mt > 0) {
+    const double cos_min = std::cos(min_parallax);   // once, in double precision
+    const ParamsW prw{{s->d_poses[0].p, s->d_poses[1].p}, {s->d_points[0].p, s->d_points[1].p}};
+    const unsigned grid = (unsigned)(((long long)Mt * 4 + kTriangulateThreads - 1) / kTriangulateThreads);
+    k_triangulate_points<<<grid, kTriangulateThreads, 0, st>>>(
+        Mt, s->d_point_obs_start.p, s->d_point_free.p, d_select.p, s->d_obs_uv.p, s->d_obs_pose.p, s->d_obs_camflags.p,
+        prw, s->d_cams.p, cos_min, max_residual, s->d_state.p, d_status.p, d_counts.p);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (int rc = settle_point_update(s, cur)) return rc;
+  unsigned long long h_counts[6] = {0, 0, 0, 0, 0, 0};
+  if (status && Mt > 0) CUDA_TRY(cudaMemcpyAsync(status, d_status.p, (size_t)Mt, cudaMemcpyDeviceToHost, st));
+  if (counts) CUDA_TRY(cudaMemcpyAsync(h_counts, d_counts.p, sizeof(h_counts), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  {
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { s->err = std::string("kernel failure: ") + cudaGetErrorString(e); return BA_ERR_CUDA; }
+  }
+  if (counts) for (int i = 0; i < 6; ++i) counts[i] = (long long)h_counts[i];
   return BA_OK;
 }
 

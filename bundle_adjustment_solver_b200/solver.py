@@ -9,6 +9,7 @@ Parameters are identified by the integer handle the Add* call returns (the refer
 object address).  All arithmetic runs on the GPU; this file only converts units and copies buffers.
 """
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -428,6 +429,34 @@ class FullBundleAdjustmentSolver:
         refined = status <= capi.POINT_MAX_ITERATIONS
         self.points[refined] = X[refined] * self.inverse_scaler
         return status, iterations, costs
+
+    # --- triangulation ---------------------------------------------------------------------------------
+    def triangulate_points(self, select=None, min_parallax_deg=1.0, max_residual_px=np.inf):
+        """Places landmarks at the midpoint of their viewing rays from the accepted poses (ba_triangulate_points), e.g.
+        new landmarks registered without a position (NaN).  select: bool per landmark, or None for every free landmark.
+        A landmark is triangulated when it has two or more observations, some ray of which is at least
+        min_parallax_deg (degrees) away from its first ray, and the point lies in front of every observing camera with
+        |r_u| + |r_v| <= max_residual_px (caller's pixels; inf disables the test) on every observation.  Writes the
+        triangulated landmarks into self.points (caller's units); every other landmark keeps its value; the next solve
+        starts from them.  Returns (status uint8 (M,) of capi.TRI_*, counts int64 (6,) landmarks per status)."""
+        self.is_parameter_finalized = True
+        self._upload()
+        m = len(np.asarray(self.points).reshape(-1, 3))
+        sel = None
+        if select is not None:
+            sel = np.ascontiguousarray(np.asarray(select, dtype=bool).astype(np.uint8))
+            if sel.shape != (m,):
+                raise ValueError(f"select has shape {sel.shape}, expected ({m},)")
+        status = np.zeros(m, dtype=np.uint8)
+        counts = np.zeros(6, dtype=np.int64)
+        _check(self.L.ba_triangulate_points(self.h, ptr(sel), math.radians(min_parallax_deg),
+                                            float(max_residual_px) * self.scaler, ptr(status), ptr(counts)),
+               self.L, self.h, "ba_triangulate_points")
+        X = np.zeros((m, 3))
+        _check(self.L.ba_get_points(self.h, ptr(X)), self.L, self.h, "ba_get_points")
+        done = status == capi.TRI_TRIANGULATED
+        self.points[done] = X[done] * self.inverse_scaler
+        return status, counts
 
     def dump(self, name):
         n = self.L.ba_debug_dump(self.h, self.DUMP[name], None)

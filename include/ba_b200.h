@@ -169,6 +169,35 @@ int ba_observation_residuals(ba_solver *s, double threshold, double *residuals, 
 int ba_refine_points(ba_solver *s, const ba_options *opt, const uint8_t *select, double *costs, int *iterations,
                      uint8_t *status, long long *counts);
 
+/* Triangulation: places landmarks from the accepted poses and their observations, e.g. new landmarks before a solve. */
+#define BA_TRI_TRIANGULATED 0
+#define BA_TRI_SKIPPED 1              /* fixed, or not selected: untouched */
+#define BA_TRI_TOO_FEW_OBSERVATIONS 2 /* fewer than two observations */
+#define BA_TRI_LOW_PARALLAX 3         /* rays too close to parallel, or the solve is not finite */
+#define BA_TRI_BEHIND_CAMERA 4        /* depth <= 0 in some observing camera */
+#define BA_TRI_LARGE_RESIDUAL 5       /* some observation's |r_u| + |r_v| > max_residual */
+/* Landmark i, over all of its observations k in point order (lowest pose index first, then insertion order; those
+ * from fixed poses included): the observing camera is R_k = R_c R_jw, t_k = R_c t_jw + t_c, its centre
+ * c_k = -R_k^T t_k and the unit ray d_k = R_k^T m_k / ||m_k||, m_k = ((u - cx) / fx, (v - cy) / fy, 1); f is the first
+ * observation.  The status rules, first match wins:
+ *   1. fixed or not selected: BA_TRI_SKIPPED;  2. fewer than two observations: BA_TRI_TOO_FEW_OBSERVATIONS;
+ *   3. min_k d_f . d_k > cos(min_parallax): BA_TRI_LOW_PARALLAX;
+ *   4. X = c_f + A^-1 g, A = sum_k (I - d_k d_k^T), g = sum_k (I - d_k d_k^T)(c_k - c_f) (the multi-view midpoint;
+ *      A^-1 by the pivoted LDL^T of the landmark side); X not finite: BA_TRI_LOW_PARALLAX;
+ *   5. some observation has depth <= 0 at X, or a non-finite residual: BA_TRI_BEHIND_CAMERA;
+ *   6. some observation has |r_u| + |r_v| > max_residual at X: BA_TRI_LARGE_RESIDUAL;
+ *   7. otherwise BA_TRI_TRIANGULATED.
+ * Rules 5 and 6 are the BA_OBS_BEHIND_CAMERA and BA_OBS_OUTLIER tests of ba_observation_residuals, so after the call
+ * every observation of a triangulated landmark is BA_OBS_INLIER at threshold max_residual.
+ * select [M_total] (order of ba_set_points), or NULL for every free landmark.  min_parallax in radians, in (0, pi];
+ * max_residual in internal units (pixels x scaler_), >= 0, +inf disables rule 6; anything else (NaN included) is
+ * BA_ERR_INVALID.  status [M_total] (BA_TRI_*), counts [6] (landmarks per BA_TRI_* value): each may be NULL.
+ * Only BA_TRI_TRIANGULATED landmarks are written; every other landmark keeps its accepted value bit for bit (NaN
+ * included).  Finalizes first, as ba_cost does.  Afterwards the poses are unchanged and the solver is in the state
+ * ba_update_parameters(s, NULL, X) leaves.  BA_ERR_STATE on a solver joined to a communicator. */
+int ba_triangulate_points(ba_solver *s, const uint8_t *select, double min_parallax, double max_residual,
+                          uint8_t *status, long long *counts);
+
 /* ---- results ----------------------------------------------------------- */
 int ba_get_poses(ba_solver *s, double *T_jw);  /* all poses, 12 doubles each, internal units */
 int ba_get_points(ba_solver *s, double *X);    /* all points */

@@ -358,6 +358,44 @@ class FullBundleAdjustmentSolver {
     if (status) status->assign(st.begin(), st.end());
     return refined;
   }
+
+  // extension: triangulation (ba_triangulate_points).  Every selected free landmark with two or more observations is
+  // placed at the midpoint of its viewing rays from the poses of the last Solve (the initial ones before it), e.g. a new
+  // landmark added without a position.  It is written only if some ray is at least min_parallax_deg (degrees) away
+  // from its first ray and the point lies in front of every observing camera with |r_u| + |r_v| <= max_residual_px
+  // (caller's pixels; +inf disables the test) on every observation.  Triangulated landmarks are written through the
+  // caller's _BA_Point pointers, and the next Solve or RefinePoints starts from them.  select: the landmarks to try, or
+  // null for every free landmark (an unknown pointer throws std::runtime_error); status (optional): a BA_TRI_* value
+  // per AddPoint call.  Returns the number of landmarks triangulated.
+  int TriangulatePoints(double min_parallax_deg, double max_residual_px, const std::vector<_BA_Point *> *select = nullptr,
+                        std::vector<int> *status = nullptr) {
+    const size_t m = point_ptrs_.size();
+    std::vector<uint8_t> sel;
+    if (select) {
+      sel.assign(m, 0);
+      for (_BA_Point *p : *select) {
+        auto it = point_index_.find(p);
+        if (it == point_index_.end()) throw std::runtime_error("There is no pointer in the BA point pool.");
+        sel[it->second] = 1;
+      }
+    }
+    FinalizeParameters();
+    if (device_dirty_ || !handle_) Upload();
+    std::vector<uint8_t> st(m);
+    Check(ba_triangulate_points(handle_, select ? sel.data() : nullptr, min_parallax_deg * (3.14159265358979323846 / 180.0),
+                                max_residual_px * scaler_, st.data(), nullptr), "ba_triangulate_points");
+    std::vector<double> X(m * 3);
+    Check(ba_get_points(handle_, X.data()), "ba_get_points");
+    X_ = X;
+    int triangulated = 0;
+    for (size_t i = 0; i < m; ++i) {
+      if (st[i] != BA_TRI_TRIANGULATED) continue;
+      *point_ptrs_[i] = _BA_Point(X[i * 3] * inverse_scaler_, X[i * 3 + 1] * inverse_scaler_, X[i * 3 + 2] * inverse_scaler_);
+      ++triangulated;
+    }
+    if (status) status->assign(st.begin(), st.end());
+    return triangulated;
+  }
   void SetDevice(int device) { device_ = device; }
 
  protected:

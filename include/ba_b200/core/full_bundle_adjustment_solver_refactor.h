@@ -136,6 +136,7 @@ class FullBundleAdjustmentSolverRefactor : private FullBundleAdjustmentSolver {
   using Base::GetObservationResiduals;
   using Base::RemoveOutlierObservations;
   using Base::RefinePoints;
+  using Base::TriangulatePoints;
 };
 
 }  // namespace analytic_solver
